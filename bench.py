@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- images/s of the embedding-to-distance hot path (patchify -> alpha -> X -> dist).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload config2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload config2] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic input: hooked backbone feature maps resident
@@ -19,7 +19,9 @@ Workloads = BASELINE.json's configs (the default, config2, is the one the metric
 At N > 1: unsupervised / supervised workloads shard the query images over the ranks (operand all-gather over NCCL,
 X rows gathered back; strong scaling of the same workload); config4pc assigns whole categories to ranks (LPT, no
 collective).  During warm-up rank 0 also runs the whole workload alone and compares -> `parity_ok`.
-`--impl reference` times the oracle port of the reference's torch CPU path on the host cores."""
+`--impl reference` times the oracle port of the reference's torch CPU path on the host cores.
+`--dump-outputs DIR` writes what the last timed step returned on rank 0 (alpha, X, Dmat, w, ...) as DIR/<name>.npy; the
+synthetic inputs depend only on the arguments, so two builds can be compared output for output."""
 from __future__ import annotations
 
 import argparse
@@ -101,6 +103,44 @@ def load_peaks():
         return dict(hbm_gbs=p["hbm_gbs"], bf16_burst=p["bf16_tflops"], bf16_sustained=p.get("bf16_tflops_sustained", p["bf16_tflops"]),
                     source="measured")
     return dict(hbm_gbs=6650.0, bf16_burst=1590.0, bf16_sustained=1400.0, source="fallback")
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+NPY_HEADER_BYTES = 1024          # allowance per file for the .npy header (np.save writes 128 bytes for these shapes)
+
+
+def dump_outputs(out, directory, limit_bytes=DUMP_LIMIT_BYTES):
+    """Writes the tensors of one step's result `out` ({name: tensor or list of tensors}) as <directory>/<name>.npy, a list
+    as <name>_<i>.npy.  float64 stays float64, every other dtype is stored as float32.  The files hold at most
+    `limit_bytes` in all: the smallest arrays are written whole, and an array larger than its share of what is left is
+    replaced by a 1-D sample of its flattened elements at sorted indices drawn from np.random.default_rng(0), so the
+    sample depends only on the array's shape and is the same for every build.  Returns {file name: (shape, sampled)}."""
+    import numpy as np
+    import torch
+
+    items = []
+    for name in sorted(out):
+        v = out[name]
+        items += [("%s_%d" % (name, i), t) for i, t in enumerate(v)] if isinstance(v, (list, tuple)) else [(name, v)]
+    items = [(n, t, 8 if t.dtype == torch.float64 else 4) for n, t in items]
+    items.sort(key=lambda it: (it[1].numel() * it[2], it[0]))
+    os.makedirs(directory, exist_ok=True)
+    left = limit_bytes - NPY_HEADER_BYTES * len(items)
+    written = {}
+    for k, (name, t, size) in enumerate(items):
+        share = left // (len(items) - k)
+        x = t.detach().reshape(-1)
+        sampled = x.numel() * size > share
+        if sampled:
+            idx = np.unique(np.random.default_rng(0).integers(0, x.numel(), size=max(1, share // size)))
+            x = x[torch.from_numpy(idx).to(x.device)]
+        arr = x.to("cpu", torch.float64 if size == 8 else torch.float32).numpy()
+        if not sampled:
+            arr = arr.reshape(tuple(t.shape))
+        np.save(os.path.join(directory, name + ".npy"), arr)
+        left -= arr.nbytes
+        written[name + ".npy"] = (tuple(t.shape), sampled)
+    return written
 
 
 class ClockSampler:
@@ -310,7 +350,13 @@ def main(argv=None):
     ap.add_argument("--z-free", action="store_true", help="(default now; kept for old command lines)")
     ap.add_argument("--no-symmetry", action="store_true", help="force the all-pairs distance kernel (every image pair multiplied twice)")
     ap.add_argument("--cuda-profiler", action="store_true", help="cudaProfilerStart/Stop around the timed steps (ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, float32 / float64, at most 64 MB")
     args = ap.parse_args(argv)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl ours)")
     wl = WORKLOADS[args.workload]
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
@@ -430,6 +476,8 @@ def main(argv=None):
         torch.cuda.profiler.stop()
     clocks = sampler.stop(t_begin, t_end) if rank == 0 else None
     launches = ops.launches() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)       # before the untimed legs below run the path again
     elapsed_ms = ev0.elapsed_time(ev1)
     marks = pipeline.PROFILE
     pipeline.PROFILE = None

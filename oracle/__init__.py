@@ -10,8 +10,8 @@ Parity status
 -------------
 * stages 1-3 (Z, w, alpha, X): the reference has NO golden vectors or
   known-answer tests for this path (SURVEY.md section 8c).  The restatement is
-  pinned by executing the reference's own Python code (imported from
-  /root/reference by `oracle/ref_import.py`, build container only) on seeded
+  pinned by executing the reference's own Python code (imported from the
+  checkout AC_REFERENCE_DIR names by `oracle/ref_import.py`) on seeded
   synthetic inputs; `oracle/make_golden.py` stores those reference outputs as
   fixtures in `tests/golden/` and `tests/test_oracle_golden.py` re-checks the
   restatement against them on every run.

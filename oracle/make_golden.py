@@ -1,9 +1,9 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (build container only).
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference.
 
-    python -m oracle.make_golden
+    AC_REFERENCE_DIR=<checkout of Anomaly-Clustering> python -m oracle.make_golden
 
 TEST INFRASTRUCTURE.  Each fixture holds seeded synthetic inputs together with the
-outputs of the reference's own code (imported from /root/reference by oracle/ref_import.py):
+outputs of the reference's own code (imported from AC_REFERENCE_DIR by oracle/ref_import.py):
 
   embed_*.npz        AnomalyClusteringCore._embed (models/patchcore/patchcore.py:355-431)
   alpha_*.npz        Matrix_Alpha_Unsupervised / _Supervised (models/patchcore/utils.py:240-277)
@@ -14,9 +14,17 @@ outputs of the reference's own code (imported from /root/reference by oracle/ref
                      categories an isometric low-rank copy of X (all pairwise distances kept to
                      ~1e-12), the anomaly labels from info_<cat>.pickle and the NMI/ARI/F1 the
                      reference published in *_tau_result.csv (TAU=2 block).
+  fuzz_golden.npz    _embed on the 24 seeded random geometries of fuzz_cases() and on single_case()
+                     (shape, float64 sum and sum of squares of Z, Z at a fixed sample of positions)
+                     and Matrix_Alpha_* on their seeded alpha cases; `source` says what produced it.
 
 The restatement (oracle/restated.py, oracle/cluster.py) is asserted equal to the reference
 here as well, so a fixture is only written when the oracle already agrees with it.
+
+    python -m oracle.make_golden fuzz
+
+writes fuzz_golden.npz alone: from the reference when AC_REFERENCE_DIR is set (after the same
+agreement check), otherwise from the restatement, recorded as such in `source`.
 """
 from __future__ import annotations
 
@@ -154,7 +162,7 @@ def _load_pickle(path):
 
 
 def make_shipped():
-    base = os.path.join(ref_import.REFERENCE_ROOT, "Anomaly-Clustering", "outputs", "mvtec_ad")
+    base = os.path.join(ref_import.OUTPUTS, "mvtec_ad")
     out = {}
     cases = [("unsupervised", c) for c in ("bottle", "cable", "tile")] + [
         ("supervised", c) for c in ("cable", "hazelnut", "leather")
@@ -198,14 +206,101 @@ def make_shipped():
     np.savez_compressed(os.path.join(GOLD, "shipped_cluster_golden.npz"), **out)
 
 
+def fuzz_cases():
+    """The seeded random geometries of the live fuzz test: 24 embed cases (CNN pyramids with 1-3 layers of different
+    grids, ViT token layers, patch size 1/3/5, stride 1/2, pooling up and down, aggregator windows that straddle layers)
+    as (k, s, feats, Dp, D), then 8 alpha cases as (Z, Z_train, tau).  One random stream feeds both lists, in this order."""
+    rng = np.random.default_rng(2023)
+    gen = torch.Generator().manual_seed(2023)
+    embed = []
+    for case in range(24):
+        k = int(rng.choice([1, 3, 3, 3, 5]))
+        s = int(rng.choice([1, 1, 1, 2]))
+        B = int(rng.integers(1, 3))
+        if case % 3 == 0:      # ViT tokens: all layers share the grid
+            g = int(rng.integers(4, 9))
+            feats = [torch.randn(B, 1 + g * g, int(rng.integers(8, 40)), generator=gen) for _ in range(int(rng.integers(1, 4)))]
+        else:                  # CNN pyramid: grid halves per layer
+            g = int(rng.choice([8, 12, 16]))
+            L = int(rng.integers(1, 4))
+            feats = [torch.randn(B, int(rng.integers(6, 30)), max(g >> l, k), max(g >> l, k), generator=gen) for l in range(L)]
+        Dp, D = int(rng.integers(5, 70)), int(rng.integers(5, 90))
+        embed.append((k, s, feats, Dp, D))
+    alpha = []
+    for case in range(8):
+        N, P, Dd = int(rng.integers(2, 6)), int(rng.integers(4, 30)), int(rng.integers(8, 40))
+        Z = torch.randn(N, P, Dd, generator=gen) * float(rng.uniform(0.5, 3.0))
+        Zt = torch.randn(int(rng.integers(1, 5)), P, Dd, generator=gen)
+        tau = float(rng.choice([0.0, 0.3, 1.0, 2.5, 20.0]))
+        alpha.append((Z, Zt, tau))
+    return embed, alpha
+
+
+def single_case():
+    """The seeded inputs of the single live check: two ViT token layers [1, 65, 48] (patch 3, stride 1, 128 -> 256) and a
+    [4, 30, 32] Z for unsupervised alpha at tau = 1."""
+    gen = torch.Generator().manual_seed(11)
+    feats = [torch.randn(1, 1 + 64, 48, generator=gen), torch.randn(1, 1 + 64, 48, generator=gen)]
+    return feats, torch.randn(4, 30, 32, generator=gen)
+
+
+FUZZ_SAMPLE = 512       # Z elements stored per embed case, at np.unique(default_rng(seed).integers(0, Z.numel(), FUZZ_SAMPLE))
+
+
+def fuzz_sample_index(seed, numel):
+    return np.unique(np.random.default_rng(seed).integers(0, numel, FUZZ_SAMPLE))
+
+
+def _store_embed(out, key, seed, z, feats):
+    z64 = z.double()
+    out[key + "_shape"] = np.array(z.shape)
+    out[key + "_sums"] = np.array([z64.sum().item(), (z64 * z64).sum().item()])
+    out[key + "_sample"] = z.reshape(-1).numpy()[fuzz_sample_index(seed, z.numel())]
+    out[key + "_input_sums"] = np.array([f.double().sum().item() for f in feats])
+
+
+def make_fuzz():
+    live = ref_import.available()
+    embed, alpha = fuzz_cases()
+    feats1, Z1 = single_case()
+    out = {"source": np.array("reference" if live else "restatement")}
+    for i, (k, s, feats, Dp, D) in enumerate(embed + [(3, 1, feats1, 128, 256)]):
+        z = restated.embed(feats, k, s, Dp, D)
+        if live:
+            zr = ref_import.reference_embed(feats, k, s, Dp, D)
+            assert zr.shape == z.shape and (zr - z).abs().max().item() <= 5e-6, (i, k, s, Dp, D)
+            z = zr
+        _store_embed(out, "embed%d" % i if i < len(embed) else "single", i, z, feats)
+    for i, (Z, Zt, tau) in enumerate(alpha):
+        au, asup = restated.matrix_alpha_unsupervised(tau, Z), restated.matrix_alpha_supervised(tau, Z, Zt)
+        if live:
+            ru, rs = ref_import.reference_alpha_unsupervised(tau, Z), ref_import.reference_alpha_supervised(tau, Z, Zt)
+            assert (ru - au).abs().max().item() <= 1e-6 and (rs - asup).abs().max().item() <= 1e-6, (i, tau)
+            au, asup = ru, rs
+        out["alpha%d_unsup" % i] = au.numpy()
+        out["alpha%d_sup" % i] = asup.numpy()
+        out["alpha%d_input_sums" % i] = np.array([Z.double().sum().item(), Zt.double().sum().item(), tau])
+    a1 = restated.matrix_alpha_unsupervised(1.0, Z1)
+    if live:
+        r1 = ref_import.reference_alpha_unsupervised(1.0, Z1)
+        assert (r1 - a1).abs().max().item() <= 1e-6
+        a1 = r1
+    out["single_alpha_unsup"] = a1.numpy()
+    np.savez_compressed(os.path.join(GOLD, "fuzz_golden.npz"), **out)
+    print("fuzz_golden from the", out["source"], "->", os.path.getsize(os.path.join(GOLD, "fuzz_golden.npz")), "bytes")
+
+
 def main():
-    assert ref_import.available(), "needs /root/reference (build container)"
+    if sys.argv[1:] == ["fuzz"]:
+        return make_fuzz()
+    assert ref_import.available() and ref_import.outputs_available(), "set AC_REFERENCE_DIR to a checkout of Anomaly-Clustering"
     os.makedirs(GOLD, exist_ok=True)
     torch.set_num_threads(8)
     make_embed()
     make_alpha()
     make_patchify()
     make_shipped()
+    make_fuzz()
 
 
 if __name__ == "__main__":

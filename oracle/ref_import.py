@@ -1,9 +1,11 @@
-"""Import the UNMODIFIED reference modules from /root/reference (build container only).
+"""Import the UNMODIFIED reference modules from a checkout of the original project.
 
-TEST INFRASTRUCTURE.  /root/reference does not exist on the GPU box, so nothing
-that runs there (`-m gpu` tests, smoke(), bench.py) may call this module; it is
-used by `oracle/make_golden.py` (fixture generation) and by the CPU-side tests
-that are skipped when the reference tree is absent.
+TEST INFRASTRUCTURE.  The original project (KevinWangHP/Anomaly-Clustering, with
+its shipped `outputs/`) is not part of this repository: AC_REFERENCE_DIR names a
+checkout of it.  Nothing the suite needs may call this module unconditionally
+(`-m gpu` tests, smoke(), bench.py never do); it is used by
+`oracle/make_golden.py` (fixture generation) and by the CPU-side tests that are
+skipped when AC_REFERENCE_DIR is not set.
 
 The reference imports faiss / timm / matplotlib / munkres at module top level
 (Anomaly-Clustering/models/patchcore/common.py:7, backbones.py:1, utils.py:7);
@@ -16,12 +18,17 @@ import sys
 import types
 from unittest import mock
 
-REFERENCE_ROOT = "/root/reference"
-_MODELS = os.path.join(REFERENCE_ROOT, "Anomaly-Clustering", "models")
+REFERENCE_DIR = os.environ.get("AC_REFERENCE_DIR", "")
+_MODELS = os.path.join(REFERENCE_DIR, "models")
+OUTPUTS = os.path.join(REFERENCE_DIR, "outputs")
 
 
 def available() -> bool:
-    return os.path.isdir(_MODELS)
+    return bool(REFERENCE_DIR) and os.path.isdir(_MODELS)
+
+
+def outputs_available() -> bool:
+    return bool(REFERENCE_DIR) and os.path.isdir(OUTPUTS)
 
 
 _cached = None
@@ -33,7 +40,7 @@ def load():
     if _cached is not None:
         return _cached
     if not available():
-        raise RuntimeError("reference tree not present at %s" % REFERENCE_ROOT)
+        raise RuntimeError("set AC_REFERENCE_DIR to a checkout of the original Anomaly-Clustering project (got %r)" % REFERENCE_DIR)
     for name in ("faiss", "timm", "matplotlib", "matplotlib.pyplot", "munkres"):
         if name not in sys.modules:
             sys.modules[name] = mock.MagicMock()

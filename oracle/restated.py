@@ -1,7 +1,7 @@
 """CPU restatement of the reference's embedding-to-distance path.  TEST INFRASTRUCTURE ONLY.
 
-Every function cites the reference lines it follows (paths relative to
-/root/reference/Anomaly-Clustering).  Written from the algorithm's closed form
+Every function cites the reference lines it follows (paths relative to the
+root of the Anomaly-Clustering project).  Written from the algorithm's closed form
 (SURVEY.md section 8c), vectorised so that it finishes in seconds at test sizes.
 Pinned against the reference's own code by tests/golden (see oracle/__init__.py).
 

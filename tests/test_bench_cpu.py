@@ -62,6 +62,46 @@ def test_clock_sampler_without_nvidia_smi(tmp_path, monkeypatch):
     assert s.stop(0.0, 1.0)["reasons"] == ["nvidia-smi unavailable"]
 
 
+def test_dump_outputs_dtypes_names_and_size_cap(tmp_path):
+    import numpy as np
+    import torch
+
+    gen = torch.Generator().manual_seed(0)
+    out = {"alpha": torch.rand(2, 3, 50, dtype=torch.float64, generator=gen), "X": torch.rand(2, 3, 64, generator=gen).half(),
+           "Dmat": [torch.rand(1, 3, 3, generator=gen), torch.rand(1, 4, 4, generator=gen)], "w": torch.rand(3, 50, generator=gen)}
+    got = bench.dump_outputs(out, str(tmp_path / "full"))
+    assert sorted(got) == ["Dmat_0.npy", "Dmat_1.npy", "X.npy", "alpha.npy", "w.npy"] and not any(s for _, s in got.values())
+    a, X, d1 = (np.load(str(tmp_path / "full" / n)) for n in ("alpha.npy", "X.npy", "Dmat_1.npy"))
+    assert a.dtype == np.float64 and np.array_equal(a, out["alpha"].numpy())
+    assert X.dtype == np.float32 and np.array_equal(X, out["X"].float().numpy())
+    assert d1.dtype == np.float32 and np.array_equal(d1, out["Dmat"][1].numpy())
+    # over the cap: the small arrays stay whole, the large ones become fixed samples, the files stay under the cap
+    big = {"X": torch.rand(400, 1000, generator=gen), "Dmat": torch.rand(300, 300, dtype=torch.float64, generator=gen),
+           "w": torch.rand(10, 10, generator=gen)}
+    limit = 1 << 20
+    for run in ("s1", "s2"):
+        got = bench.dump_outputs(big, str(tmp_path / run), limit_bytes=limit)
+        assert got == {"w.npy": ((10, 10), False), "X.npy": ((400, 1000), True), "Dmat.npy": ((300, 300), True)}
+        assert sum(os.path.getsize(str(tmp_path / run / n)) for n in got) <= limit
+    for n in got:
+        assert np.array_equal(np.load(str(tmp_path / "s1" / n)), np.load(str(tmp_path / "s2" / n)))
+    # the documented rule: smallest first, each array gets what is left over the arrays still to write, and a sampled
+    # array holds the elements at np.unique(default_rng(0).integers(0, numel, size=share // itemsize))
+    left = limit - 3 * bench.NPY_HEADER_BYTES - 10 * 10 * 4
+    for name, itemsize, n_after in (("Dmat", 8, 2), ("X", 4, 1)):
+        src = big[name].numpy().ravel()
+        idx = np.unique(np.random.default_rng(0).integers(0, src.size, size=(left // n_after) // itemsize))
+        xs = np.load(str(tmp_path / "s1" / (name + ".npy")))
+        assert xs.dtype == src.dtype and np.array_equal(xs, src[idx]), name
+        left -= xs.nbytes
+
+
+def test_bench_refuses_zero_steps():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=120,
+                       cwd=ROOT)
+    assert r.returncode == 2 and "--steps must be at least 1" in r.stderr
+
+
 @pytest.mark.timeout(900)
 def test_reference_arm_prints_the_contract_line():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "tiny", "--steps", "2",

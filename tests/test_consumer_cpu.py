@@ -7,6 +7,7 @@ import pytest
 import torch
 
 from anomaly_clustering_b200 import cluster, io
+from oracle import ref_import
 
 
 def test_metrics_from_distance_matrix_match_published_csv(golden_dir):
@@ -41,10 +42,10 @@ def test_pickle_roundtrip_matches_reference_layout(tmp_path):
     assert np.array_equal(Xl, X)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/Anomaly-Clustering/outputs"), reason="reference artefacts absent")
+@pytest.mark.skipif(not ref_import.outputs_available(), reason="AC_REFERENCE_DIR (a checkout of the original project) not set")
 def test_reads_the_reference_shipped_pickle():
-    p = ("/root/reference/Anomaly-Clustering/outputs/mvtec_ad/dino_vitbase8/unsupervised/"
-         "blocks.10_blocks.11_2048_4096_2.0_1.0/matrix_alpha_X_bottle_unsupervised.pickle")
+    p = os.path.join(ref_import.OUTPUTS, "mvtec_ad", "dino_vitbase8", "unsupervised", "blocks.10_blocks.11_2048_4096_2.0_1.0",
+                     "matrix_alpha_X_bottle_unsupervised.pickle")
     a, X = io.load_matrix_alpha_X(p)
     assert a.shape == (83, 1, 784) and X.shape == (83, 4096)
 
@@ -59,6 +60,28 @@ def test_result_csv_roundtrip_is_byte_identical(golden_dir, tmp_path):
     out = io.write_result_csv(str(tmp_path / "x.csv"), mode, blocks)
     # the shipped copy went through git's end-of-line normalisation (LF); csv.writer emits CRLF like the reference's does
     assert open(out, "rb").read().replace(b"\r\n", b"\n") == open(src, "rb").read()
+
+
+# MVTec AD test-set sizes without the 'combined' images, which test.py drops before clustering (cable, pill, zipper and wood
+# have 11, 17, 16 and 11 of them)
+MVTEC_SIZES = dict(bottle=83, cable=139, capsule=132, hazelnut=110, metal_nut=115, pill=150, screw=160, toothbrush=42, transistor=100,
+                   zipper=135, carpet=117, grid=78, leather=124, tile=117, wood=68)
+
+
+def test_aggregate_rows_match_the_shipped_csv(golden_dir):
+    """The MVTec(object) / MVTec(texture) rows of every tau block of the shipped CSV head are size_weighted_mean of the
+    category rows, weighted by the images left after dropping 'combined' ones."""
+    g = np.load(os.path.join(golden_dir, "shipped_cluster_golden.npz"), allow_pickle=False)
+    for key in (str(k) for k in g["cases"]):     # the sizes agree with the stored labels of the reference's info pickles
+        assert MVTEC_SIZES[key.split("_", 1)[1]] == sum(str(a) != "combined" for a in g[key + "_anomaly"]), key
+    _, blocks = io.read_result_csv(os.path.join(golden_dir, "shipped_tau_result_head.csv"))
+    for tau, rows in blocks:
+        d = {r[0]: r[1:] for r in rows}
+        for c, n in MVTEC_SIZES.items():           # F1-micro is a count of correct images over n
+            assert abs(d[c][2] * n - round(d[c][2] * n)) < 1e-9, (tau, c)
+        for title, group in (("MVTec(object)", io.OBJECT), ("MVTec(texture)", io.TEXTURE)):
+            got = [cluster.size_weighted_mean([d[c][m] for c in group], [MVTEC_SIZES[c] for c in group]) for m in range(3)]
+            assert np.allclose(got, d[title], rtol=0, atol=1e-12), (tau, title, got, d[title])
 
 
 def test_info_pickle_layout(tmp_path):
@@ -109,23 +132,31 @@ def test_evaluate_runs_on_synthetic_outputs(tmp_path):
     assert mode == "unsupervised" and back[0][0] == "1" and [r[0] for r in back[0][1]] == [r[0] for r in rows]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/Anomaly-Clustering/outputs"), reason="reference artefacts absent")
 @pytest.mark.parametrize("mode", ["unsupervised", "supervised"])
-def test_evaluate_runs_reproduces_the_shipped_csv_block(mode, tmp_path):
-    """The shipped (alpha, X) pickles (15 supervised, 13 unsupervised) + info pickles at tau=2 -> exactly the TAU=2 block of the shipped CSV,
-    category rows and both aggregate rows."""
-    root = "/root/reference/Anomaly-Clustering/outputs"
+def test_evaluate_runs_reproduces_the_shipped_csv_block(mode, golden_dir, tmp_path):
+    """The reference's shipped results of the categories kept in tests/golden/shipped_cluster_golden.npz (X as an isometric
+    copy, the anomaly labels of info_<category>.pickle), written back in the reference's on-disk layout at tau=2 -> the
+    category rows of the TAU=2 block of the shipped CSV, and both aggregate rows as the means of those rows weighted as the
+    shipped aggregate rows are (test_aggregate_rows_match_the_shipped_csv)."""
+    g = np.load(os.path.join(golden_dir, "shipped_cluster_golden.npz"), allow_pickle=False)
     layers = ["blocks.10", "blocks.11"]
+    root = str(tmp_path)
+    mode_dir = os.path.join(root, "mvtec_ad", "dino_vitbase8", mode)
+    want = {}
+    for key in (str(k) for k in g["cases"] if str(k).startswith(mode + "_")):
+        cat, names = key[len(mode) + 1:], [str(a) for a in g[key + "_anomaly"]]
+        X = g[key + "_Xlow"]
+        io.save_matrix_alpha_X(mode_dir, layers, 2048, 4096, 2, 1, cat, mode, torch.full((len(X), 784), 1 / 784), X)
+        io.save_info(root, "mvtec_ad", cat, io.make_info(cat, names))
+        want[cat] = g[key + "_csv"]
+    for title, group in (("MVTec(object)", io.OBJECT), ("MVTec(texture)", io.TEXTURE)):
+        cats = [c for c in group if c in want]
+        want[title] = sum(want[c] * MVTEC_SIZES[c] for c in cats) / sum(MVTEC_SIZES[c] for c in cats)
     blocks = cluster.evaluate_runs(root, "mvtec_ad", "dino_vitbase8", mode, layers, 2048, 4096, [2], dmat_fn=_cpu_dmat,
                                    write_csv=False)
-    _, shipped = io.read_result_csv(io.result_csv_path(os.path.join(root, "mvtec_ad", "dino_vitbase8", mode), layers, 2048, 4096))
-    want = {r[0]: r[1:] for r in dict(shipped)["2"]}
     got = {r[0]: r[1:] for r in blocks[0][1]}
-    assert len(got) >= 13
-    complete = all(c in got for c in io.OBJECT + io.TEXTURE)     # the shipped unsupervised run lacks pill and screw
+    assert len(got) == 5 and sorted(got) == sorted(want)
     for name, vals in got.items():
-        if name.startswith("MVTec(") and not (complete or name == "MVTec(texture)"):
-            continue                                             # an aggregate over fewer categories than the CSV's
         assert np.allclose(vals, want[name], atol=1e-9), (name, vals, want[name])
 
 

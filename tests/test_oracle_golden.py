@@ -7,7 +7,7 @@ import pytest
 import torch
 
 from oracle import cluster as ocluster
-from oracle import restated
+from oracle import make_golden, ref_import, restated
 
 EMBED_CASES = ["embed_vit_small", "embed_wrn_small", "embed_ragged", "embed_k5s2", "embed_single"]
 
@@ -86,51 +86,58 @@ def test_pairwise_matches_scipy():
     assert np.allclose(D, ref, atol=1e-12)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/Anomaly-Clustering"), reason="reference tree absent")
-def test_oracle_against_live_reference():
-    """Build container only: run the imported reference on fresh seeded inputs."""
-    from oracle import ref_import
+def _check_embed(g, key, seed, z, feats, tol):
+    assert np.allclose(g[key + "_input_sums"], [f.double().sum().item() for f in feats], rtol=1e-12, atol=1e-9), \
+        (key, "the seeded inputs changed: the fixture no longer describes these inputs")
+    assert tuple(z.shape) == tuple(g[key + "_shape"]), key
+    n, zmax = z.numel(), float(z.abs().max())
+    z64 = z.double()
+    assert abs(z64.sum().item() - g[key + "_sums"][0]) <= tol * n, key
+    assert abs((z64 * z64).sum().item() - g[key + "_sums"][1]) <= tol * n * (2 * zmax + tol), key
+    idx = make_golden.fuzz_sample_index(seed, n)
+    assert np.abs(z.reshape(-1).numpy()[idx] - g[key + "_sample"]).max() <= tol, key
 
-    gen = torch.Generator().manual_seed(11)
-    feats = [torch.randn(1, 1 + 64, 48, generator=gen), torch.randn(1, 1 + 64, 48, generator=gen)]
+
+def test_oracle_matches_stored_fuzz_outputs(golden_dir):
+    """The restatement on the seeded inputs of the two live-reference tests below against tests/golden/fuzz_golden.npz,
+    at the same tolerances: Z of every embed geometry (shape, float64 sum and sum of squares, a fixed sample of elements)
+    and alpha of every alpha case in both modes."""
+    g = load(golden_dir, "fuzz_golden")
+    embed, alpha = make_golden.fuzz_cases()
+    for i, (k, s, feats, Dp, D) in enumerate(embed):
+        _check_embed(g, "embed%d" % i, i, restated.embed(feats, k, s, Dp, D), feats, 5e-6)
+    feats1, Z1 = make_golden.single_case()
+    _check_embed(g, "single", len(embed), restated.embed(feats1, 3, 1, 128, 256), feats1, 2e-6)
+    for i, (Z, Zt, tau) in enumerate(alpha):
+        assert np.allclose(g["alpha%d_input_sums" % i], [Z.double().sum().item(), Zt.double().sum().item(), tau], rtol=1e-12, atol=1e-9), i
+        assert np.abs(restated.matrix_alpha_unsupervised(tau, Z).numpy() - g["alpha%d_unsup" % i]).max() <= 1e-6, (i, tau)
+        assert np.abs(restated.matrix_alpha_supervised(tau, Z, Zt).numpy() - g["alpha%d_sup" % i]).max() <= 1e-6, (i, tau)
+    assert np.abs(restated.matrix_alpha_unsupervised(1.0, Z1).numpy() - g["single_alpha_unsup"]).max() <= 1e-6
+
+
+@pytest.mark.skipif(not ref_import.available(), reason="AC_REFERENCE_DIR (a checkout of the original project) not set")
+def test_oracle_against_live_reference():
+    """Runs the imported reference on the seeded inputs of make_golden.single_case()."""
+    feats, Z = make_golden.single_case()
     zr = ref_import.reference_embed(feats, 3, 1, 128, 256)
     zo = restated.embed(feats, 3, 1, 128, 256)
     assert (zr - zo).abs().max().item() <= 2e-6
-    Z = torch.randn(4, 30, 32, generator=gen)
     ar = ref_import.reference_alpha_unsupervised(1.0, Z)
     ao = restated.matrix_alpha_unsupervised(1.0, Z)
     assert (ar - ao).abs().max().item() <= 1e-6
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/Anomaly-Clustering"), reason="reference tree absent")
+@pytest.mark.skipif(not ref_import.available(), reason="AC_REFERENCE_DIR (a checkout of the original project) not set")
 def test_oracle_fuzz_against_live_reference():
-    """Build container only: 24 seeded random geometries (CNN pyramids with 1-3 layers of different grids, ViT
+    """The 24 seeded random geometries of make_golden.fuzz_cases() (CNN pyramids with 1-3 layers of different grids, ViT
     token layers, patch size 1/3/5, stride 1/2, pooling up and down, aggregator windows that straddle layers)
     through the imported reference's _embed, and random-tau alpha in both modes, against the restatement."""
-    from oracle import ref_import
-
-    rng = np.random.default_rng(2023)
-    gen = torch.Generator().manual_seed(2023)
-    for case in range(24):
-        k = int(rng.choice([1, 3, 3, 3, 5]))
-        s = int(rng.choice([1, 1, 1, 2]))
-        B = int(rng.integers(1, 3))
-        if case % 3 == 0:      # ViT tokens: all layers share the grid
-            g = int(rng.integers(4, 9))
-            feats = [torch.randn(B, 1 + g * g, int(rng.integers(8, 40)), generator=gen) for _ in range(int(rng.integers(1, 4)))]
-        else:                  # CNN pyramid: grid halves per layer
-            g = int(rng.choice([8, 12, 16]))
-            L = int(rng.integers(1, 4))
-            feats = [torch.randn(B, int(rng.integers(6, 30)), max(g >> l, k), max(g >> l, k), generator=gen) for l in range(L)]
-        Dp, D = int(rng.integers(5, 70)), int(rng.integers(5, 90))
+    embed, alpha = make_golden.fuzz_cases()
+    for case, (k, s, feats, Dp, D) in enumerate(embed):
         zr = ref_import.reference_embed(feats, k, s, Dp, D)
         zo = restated.embed(feats, k, s, Dp, D)
         assert zr.shape == zo.shape, (case, zr.shape, zo.shape)
         assert (zr - zo).abs().max().item() <= 5e-6, (case, k, s, [tuple(f.shape) for f in feats], Dp, D)
-    for case in range(8):
-        N, P, Dd = int(rng.integers(2, 6)), int(rng.integers(4, 30)), int(rng.integers(8, 40))
-        Z = torch.randn(N, P, Dd, generator=gen) * float(rng.uniform(0.5, 3.0))
-        Zt = torch.randn(int(rng.integers(1, 5)), P, Dd, generator=gen)
-        tau = float(rng.choice([0.0, 0.3, 1.0, 2.5, 20.0]))
+    for Z, Zt, tau in alpha:
         assert (ref_import.reference_alpha_unsupervised(tau, Z) - restated.matrix_alpha_unsupervised(tau, Z)).abs().max().item() <= 1e-6
         assert (ref_import.reference_alpha_supervised(tau, Z, Zt) - restated.matrix_alpha_supervised(tau, Z, Zt)).abs().max().item() <= 1e-6
