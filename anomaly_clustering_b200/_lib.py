@@ -147,9 +147,6 @@ def load() -> ctypes.CDLL:
     lib.ac_debug_launches.argtypes = []
     lib.ac_debug_set.restype = c_int
     lib.ac_debug_set.argtypes = [c_int, c_int]
-    # tuning overrides (debug knobs of csrc/mindist_tc.cu): AC_TC_DYNAMIC=1 -> dynamic unit scheduler
-    if os.environ.get("AC_TC_DYNAMIC") in ("0", "1"):
-        lib.ac_debug_set(4, int(os.environ["AC_TC_DYNAMIC"]))
     _lib = lib
     return lib
 

@@ -737,9 +737,6 @@ struct FusedParams {
   long long n_items;       // (B + LA) * S
   const float* zero_row;   // >= 4 KB of zeros (lean kernel: stands in for taps outside the map)
   unsigned long long* murs;  // [B][L] (mean, 1/std) packed as two floats, all-ones until the last statistics warp of the image wrote it (lean kernel)
-  int pd;                  // lean kernel: items the L2 prefetch of the statistics rows runs ahead of the claims (0 = off)
-  int cs;                  // lean kernel: operand rows stored with the streaming (evict-first) policy
-  int l2pol;               // lean kernel: L2 policy of the map loads: 0 normal, 1 evict_last
 };
 
 __device__ __forceinline__ int ld_acquire_gpu(const int* p) {
@@ -1251,10 +1248,7 @@ __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const _
   // L2 policies of the map loads: the maps must survive in L2 from their statistics read to their last embed read while
   // 1.3x their volume of operand rows streams out through the same cache
   uint64_t pol_keep = 0;
-  if (producer) {
-    if (fp.l2pol == 0) asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol_keep));
-    else asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol_keep));
-  }
+  if (producer) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol_keep));
   for (;;) {
     long long item;
     if (producer) {
@@ -1297,24 +1291,15 @@ __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const _
       // select per row.
       const bool hasA = (bA >= 0) && p.layernorm, hasB = (bE >= 0);
       const uint32_t ring_u = e_smem_u32(ring);
-      if (fp.pd > 0 && p.layernorm) {
-        // statistics rows of the item claimed fp.pd - 1 claims from now (1 = the item just claimed, whose first copies wait
-        // behind the ring slots of the previous item): DRAM -> L2 ahead of time, so that the statistics slots at the head of
-        // the item's in-order ring are L2 hits like its embed slots
-        const long long it2 = item + (fp.pd - 1);
-        const int q2 = (int)(it2 / fp.S);
-        if (q2 < p.B) {
-          const int sg2 = (int)(it2 - (long long)q2 * fp.S);
-          const int y2 = sg2 / p.nxseg, xs2 = sg2 - y2 * p.nxseg;
-          const int xa2 = xs2 * p.xseg_len, np2 = min(p.w0, xa2 + p.xseg_len) - xa2;
-          for (int l = 0; l < p.L; ++l) {
-            const LayerDev& ly = p.layers[l];
-            if (ly.sw == NCH)      // the tokens of a row are contiguous
-              e_prefetch_l2(ly.ptr + (long long)q2 * ly.sb + (long long)y2 * ly.sh + (long long)xa2 * ly.sw, (uint32_t)np2 * kRowBytes);
-          }
-        }
-      }
       if (hasA) {
+        // statistics rows of the item just claimed (its first copies wait behind the ring slots of the previous item):
+        // DRAM -> L2 ahead of time, so that the statistics slots at the head of the item's in-order ring are L2 hits like
+        // its embed slots
+        for (int l = 0; l < p.L; ++l) {
+          const LayerDev& ly = p.layers[l];
+          if (ly.sw == NCH)      // the tokens of a row are contiguous
+            e_prefetch_l2(ly.ptr + (long long)bA * ly.sb + (long long)yA * ly.sh + (long long)xaA * ly.sw, (uint32_t)nposA * kRowBytes);
+        }
         for (int l = 0; l < p.L; ++l) {
           const LayerDev& ly = p.layers[l];
           const long long sw = ly.sw;
@@ -1539,9 +1524,8 @@ __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const _
                   nv2.x = e_sq_acc(__low2half(h[i]), nv2.x);
                   nv2.y = e_sq_acc(__high2half(h[i]), nv2.y);
                 }
-                uint4* dst4 = reinterpret_cast<uint4*>(ph_ + half_ * (FT * NOUT) + o);
-                if (fp.cs) __stcs(dst4, *reinterpret_cast<const uint4*>(h));
-                else *dst4 = *reinterpret_cast<const uint4*>(h);
+                // streaming (evict-first) store: the operand rows must not push the maps out of L2
+                __stcs(reinterpret_cast<uint4*>(ph_ + half_ * (FT * NOUT) + o), *reinterpret_cast<const uint4*>(h));
               }
               if constexpr (NOUT == 4) {
                 __align__(8) __half2 h[2];
@@ -2051,8 +2035,8 @@ static int launch_periodic(EmbedParams p, const Periodic& pr, int l, int num_sms
 }
 
 // ---- single-pass fused form: eligibility and launch
-static int g_fused_la = 2;        // debug knob (ac_debug_set key 7): images the statistics run ahead of the embedding
-static int g_fused_cps = 3;       // debug knob (key 8): persistent CTAs per SM
+static constexpr int kLookAhead = 2;   // images the statistics run ahead of the embedding
+static constexpr int kCtasPerSm = 3;   // persistent CTAs per SM (the lean kernel: at most its MINB)
 
 static bool fused_eligible(const Plan& plan, const EmbedParams& p, const Periodic* pr, int L) {
   if (g_embed_variant != 0 || !plan.fused || p.k != 3 || p.s != 1) return false;
@@ -2068,7 +2052,7 @@ static bool fused_eligible(const Plan& plan, const EmbedParams& p, const Periodi
 
 static constexpr size_t kZeroRowBytes = 12288;  // lean kernel: zeros that stand in for taps outside the map (one ring slot: 3 tokens x <= 768 channels)
 
-static constexpr int kMinSeg = 4;   // shortest x segment the segment-length knob allows (sizes the statistics slots)
+static constexpr int kMinSeg = 4;   // the workspace sizes the lean kernel's statistics slots for x segments this short
 
 // workspace of the fused kernels: [mean / rstd per (image, layer)] [statistics partials] [done[B], claim counter] [zero row]
 static size_t fused_murs_bytes(int L, int B) { return ((size_t)B * L * sizeof(unsigned long long) + 255) & ~(size_t)255; }
@@ -2083,11 +2067,7 @@ static size_t fused_ws_bytes(int L, int B, int h0, int w0) {
   return fused_murs_bytes(L, B) + fused_stats_bytes(L, B, h0, w0) + fused_ctr_bytes(B) + kZeroRowBytes;
 }
 
-static int g_fused_lean = 1;      // debug knob (ac_debug_set key 9): 0 = always the general fused kernel
-static int g_fused_pd = 1;        // debug knob (key 10): lean kernel, L2 prefetch of the statistics rows: 0 = off, n = of the item n - 1 claims ahead
-static int g_fused_cs = 1;        // debug knob (key 11): lean kernel, operand rows stored with the streaming policy
-static int g_fused_l2pol = 1;     // debug knob (key 12): lean kernel, L2 policy of the map loads (0 normal, 1 evict_last)
-static int g_fused_seg = kMaxSeg; // debug knob (key 13): lean kernel, longest x segment of an item (kMinSeg .. kMaxSeg)
+static int g_fused_lean = 1;      // test hook (ac_debug_set key 9): 0 = always the general fused kernel
 
 static int launch_fused(EmbedParams p, const Periodic& pr, float* n2, void* ws, int num_sms, cudaStream_t st) {
   FusedParams fp;
@@ -2096,14 +2076,13 @@ static int launch_fused(EmbedParams p, const Periodic& pr, float* n2, void* ws, 
   const bool lean_out = g_fused_lean && p.Zhi && !p.Zlo && p.op_dtype == AC_DT_F16 && n2 && pr.R == 1 && pr.A == 27 &&
                         (p.ldz % 8 == 0) && (pr.ncols % 8 == 0) && (reinterpret_cast<uintptr_t>(p.Zhi) % 16 == 0) &&
                         (!p.Z || reinterpret_cast<uintptr_t>(p.Z) % 16 == 0) && p.h0 == p.w0;   // slices: row runs / column runs
-  const int seg_max = lean_out ? g_fused_seg : kMaxSeg;
-  p.nxseg = ceil_div(p.w0, seg_max);
+  p.nxseg = ceil_div(p.w0, kMaxSeg);
   p.xseg_len = ceil_div(p.w0, p.nxseg);
   p.nxseg = ceil_div(p.w0, p.xseg_len);
   p.b0 = 0;
   fp.n2 = n2;
   fp.S = p.h0 * p.nxseg;
-  fp.LA = std::max(1, std::min(g_fused_la, p.B));
+  fp.LA = std::max(1, std::min(kLookAhead, p.B));
   fp.nperiods = pr.nperiods;
   fp.gx = ceil_div(pr.nperiods, kFT * kPP);
   fp.t_stride = pr.ncols;
@@ -2114,9 +2093,6 @@ static int launch_fused(EmbedParams p, const Periodic& pr, float* n2, void* ws, 
   fp.done = (int*)((char*)ws + murs_b + stats_b);
   fp.counter = (unsigned int*)(fp.done + p.B);
   fp.zero_row = (const float*)((char*)fp.done + ctr_b);
-  fp.pd = g_fused_pd;
-  fp.cs = g_fused_cs;
-  fp.l2pol = g_fused_l2pol;
   fp.e = p;
   // one launch: mean / rstd and the lean kernel's statistics slots = all-ones ("unset", see kUnset); done[B], the claim counter
   // and the zero row = 0
@@ -2128,7 +2104,7 @@ static int launch_fused(EmbedParams p, const Periodic& pr, float* n2, void* ws, 
 #define XLK(b, ft, wz, ring, minb)                                                                                    \
   {                                                                                                                   \
     const size_t smem = ((size_t)ring * 3 * ft * kPP * 3 + (size_t)kMaxSeg * ft) * sizeof(float);                     \
-    const int grid_l = (int)std::min<long long>(fp.n_items, (long long)num_sms * std::min(g_fused_cps, minb));        \
+    const int grid_l = (int)std::min<long long>(fp.n_items, (long long)num_sms * std::min(kCtasPerSm, minb));         \
     auto kern = embed_fused_fast_kernel<27, b, 1, ft, wz, ring, minb>;                                                \
     AC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                      \
     kern<<<grid_l, ft + 32, smem, st>>>(fp);                                                                          \
@@ -2142,7 +2118,7 @@ static int launch_fused(EmbedParams p, const Periodic& pr, float* n2, void* ws, 
   XL(8, 128) XL(4, 128) XL(16, 64)
 #undef XL
 #undef XLK
-  const int grid = (int)std::min<long long>(fp.n_items, (long long)num_sms * g_fused_cps);
+  const int grid = (int)std::min<long long>(fp.n_items, (long long)num_sms * kCtasPerSm);
 #define X(a, b, r)                                                                                                   \
   if (pr.A == a && pr.B == b && pr.R == r) {                                                                         \
     auto kern = embed_fused_kernel<a, b, r>;                                                                         \
@@ -2395,19 +2371,12 @@ extern "C" int ac_embed(const ac_layer_t* layers, int L, int B, int patchsize, i
   return ac_embed_ex(layers, L, B, patchsize, stride, Dp, D, layernorm, eps, Z, Zhi, Zlo, op_dtype, nullptr, ws, ws_bytes, stream);
 }
 
-extern "C" int ac_debug_set_embed(int value) {
-  if (value < 0 || value > 3) return AC_ERR_INVALID;   // 3 = per-layer launches (TMA kernel where it applies), never the fused form
-  g_embed_variant = value;
-  return AC_OK;
-}
-extern "C" int ac_debug_set_fused(int key, int value) {
+// test hook (not part of the public header): forces the embedding paths the library otherwise picks from the input.
+//   key 2 = kernel variant: 0 auto, 1 LDG periodic, 2 generic tap kernel, 3 per-layer launches (TMA kernel where it applies)
+//   key 9 = lean fused kernel: 1 when eligible, 0 always the general fused kernel
+extern "C" int ac_debug_set(int key, int value) {
+  if (key == 2 && value >= 0 && value <= 3) { g_embed_variant = value; return AC_OK; }
   if (key == 9 && (value == 0 || value == 1)) { g_fused_lean = value; return AC_OK; }
-  if (key == 7 && value >= 1 && value <= 64) { g_fused_la = value; return AC_OK; }
-  if (key == 8 && value >= 1 && value <= 3) { g_fused_cps = value; return AC_OK; }
-  if (key == 10 && value >= 0 && value <= 4096) { g_fused_pd = value; return AC_OK; }
-  if (key == 11 && (value == 0 || value == 1)) { g_fused_cs = value; return AC_OK; }
-  if (key == 12 && value >= 0 && value <= 1) { g_fused_l2pol = value; return AC_OK; }
-  if (key == 13 && value >= kMinSeg && value <= kMaxSeg) { g_fused_seg = value; return AC_OK; }
   return AC_ERR_INVALID;
 }
 

@@ -5,17 +5,17 @@
 //
 //   dmin[j, r] = sqrt(max(0, |q_r|^2 + min_{c in image j} (|b_c|^2 - 2 q_r . b_c)))
 //
-// Structure (one persistent CTA -- or CTA pair with cta_group::2 -- per SM):
+// Structure (one persistent CTA pair per two SMs, cta_group::2 MMAs):
 //   warp 0      TMA producer: 128B-swizzled K-major operand tiles -> kStages-deep smem ring; in the leader CTA it
 //               also CLAIMS the work units (global atomic counter) and publishes them to the other roles through
-//               a small smem queue (dynamic scheduling; the peer CTA's copy is written with st.shared::cluster)
+//               a small smem queue (the peer CTA's copy is written with st.shared::cluster)
 //   warp 1      MMA issuer:   tcgen05.mma kind::f16, fp32 accumulators in TMEM (2 x 256 columns,
 //               double buffered so the epilogue of tile i overlaps the MMAs of tile i+1)
 //   warps 2-5   epilogue: tcgen05.ld 32 lanes x 32 columns, d2 = bn2[c] - 2*acc, running row-min in
 //               registers across the tiles of one bank image (each thread owns one query row, so
 //               the row-min needs no shuffles), one coalesced store per (row, bank image).
 //   The [Mq, Nb*P] distance matrix never exists in memory.
-// Work unit = (block of 128*kCtaGroup query rows, bank image).  A bank image is cut into nt tiles
+// Work unit = (block of 2*kTileM = 256 query rows, one kTileM half per CTA of the pair, bank image).  A bank image is cut into nt tiles
 // of <= 256 rows whose widths are multiples of 16 (P=784 -> 208+208+208+160), so no tile straddles
 // two images; excess columns of the last tile are masked with +inf norms.
 // Units are rasterised so that concurrently resident units share A blocks and bank images in L2.
@@ -35,8 +35,11 @@ namespace ac {
 static constexpr int kTcThreads = 192;
 static constexpr int kBlockK = 64;         // elements per K block = one 128-byte swizzle row (2-byte operands)
 static constexpr int kUmmaK = 16;
-static constexpr int kTileM = 128;         // rows per CTA
+static constexpr int kTileM = 128;         // rows per CTA; a CTA pair multiplies 2 * kTileM query rows
 static constexpr int kMaxN = 256;
+static constexpr int kBRows = kMaxN / 2;   // bank rows staged per CTA per stage (each CTA holds half of the N tile)
+static constexpr int kStages = 6;
+static constexpr int kGM = 16;             // query blocks per raster group: 16 x 2 MB of A + the streaming bank images stay L2-resident (tuned on B200)
 static constexpr int kTmemCols = 512;
 static constexpr long long kWatchdogCycles = 20000000000LL;  // ~10 s
 
@@ -54,19 +57,17 @@ struct __align__(64) TcParams {
   int nkb;                   // K blocks per segment
   int nseg;                  // 1 or 3
   int nt, wmain, wlast;      // tiles per bank image, widths (multiples of 16)
-  int n_mblocks, GM;
+  int n_mblocks;
   uint32_t idesc_main, idesc_last;
   // symmetric (self-bank) mode: every unordered image pair is multiplied once
   int sym;                   // 0 = every (query block, bank image) unit; 1 = only pairs owned by the query image
   int q_img0;                // global image index of query row 0 (query slice of a sharded run)
   int KU;                    // units per query block in sym mode
-  int l2_hint;               // 1: operand loads carry an L2 evict_last policy
   unsigned int* colmin;      // [nq_img, nb_img*P] squared distances (fp32 bits), atomicMin target
   const int2* units;         // sym mode: explicit (query block, bank image) list in raster order (device-built)
   const long long* n_units;  // sym mode: length of that list (device memory)
   int win_begin, win_count;  // sym mode: only bank images in the circular window [win_begin, win_begin + win_count)
-  int dynamic;               // 1: units are claimed from a global counter (work stealing) instead of round-robin
-  unsigned long long* counter;
+  unsigned long long* counter;   // next unclaimed unit (work stealing)
   // arg-min tracking (kArg kernels; the exact re-evaluation of ac_refine_min_dist needs WHICH bank row won)
   // per-category banks in one launch (the reference runs one make_category_data per category, examples/main.py:353):
   // groups[2*j], groups[2*j+1] = first image and image count of the category of bank image j; pairs exist only inside
@@ -189,91 +190,38 @@ __device__ __forceinline__ bool elect_one() {
   return pred != 0;
 }
 
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-
-// same as tma_load_2d with an L2 eviction-priority hint: the operand working set (A group + a few bank
-// images) must stay L2-resident against unrelated traffic (e.g. a concurrent H2D copy streaming through L2)
-template <int G>
-__device__ __forceinline__ void tma_load_2d_hint(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, uint64_t pol) {
-  if (G == 1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(dst),
-        "l"(map), "r"(bar), "r"(c0), "r"(c1), "l"(pol)
-        : "memory");
-  } else {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(dst),
-        "l"(map), "r"(bar), "r"(c0), "r"(c1), "l"(pol)
-        : "memory");
-  }
-}
-
-template <int G>
+// data lands in this CTA's shared memory, completion bytes are signalled on the LEADER CTA's barrier
 __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1) {
-  if (G == 1) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(dst),
-                 "l"(map), "r"(bar), "r"(c0), "r"(c1)
-                 : "memory");
-  } else {
-    // data lands in this CTA's shared memory, completion bytes are signalled on the LEADER CTA's barrier
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(dst),
-        "l"(map), "r"(bar), "r"(c0), "r"(c1)
-        : "memory");
-  }
+  asm volatile(
+      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(dst),
+      "l"(map), "r"(bar), "r"(c0), "r"(c1)
+      : "memory");
 }
 
-template <int G>
 __device__ __forceinline__ void tmem_alloc(uint32_t dst_smem, uint32_t ncols) {
-  if (G == 1)
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(ncols) : "memory");
-  else
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(ncols) : "memory");
+  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(ncols) : "memory");
 }
-template <int G>
 __device__ __forceinline__ void tmem_relinquish() {
-  if (G == 1)
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  else
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
 }
-template <int G>
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-  if (G == 1)
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-  else
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
 
-template <int G>
 __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  if (G == 1)
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-  else
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
+  asm volatile(
+      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
 }
 
-// tcgen05.commit: the mbarrier receives one arrival once all previously issued MMAs have completed
-template <int G>
+// tcgen05.commit: the mbarrier receives one arrival once all previously issued MMAs have completed;
+// multicast to the same barrier offset in both CTAs of the pair
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
-  if (G == 1)
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-  else  // same barrier offset in both CTAs of the pair
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"((uint16_t)3)
-                 : "memory");
+  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
+               "h"((uint16_t)3)
+               : "memory");
 }
 
 #define AC_TMEM_LD16(taddr, v)                                                                                          \
@@ -347,7 +295,6 @@ __device__ __forceinline__ void wait_bank_ready(const TcParams& p, int img) {
   } while (v == 0);
 }
 
-template <int G>
 __device__ __forceinline__ bool decode_unit(const TcParams& p, long long u, int& mb, int& img) {
   if (p.sym) {
     // compact host-built list (only units that carry work), so all CTA pairs stay in lock-step on the
@@ -358,21 +305,20 @@ __device__ __forceinline__ bool decode_unit(const TcParams& p, long long u, int&
     return true;
   }
   const int per_mb = p.nb_img;
-  const long long per_group = (long long)p.GM * per_mb;
+  const long long per_group = (long long)kGM * per_mb;
   const int mg = (int)(u / per_group);
   const long long rem = u - (long long)mg * per_group;
-  const int gm_cur = min(p.GM, p.n_mblocks - mg * p.GM);
+  const int gm_cur = min(kGM, p.n_mblocks - mg * kGM);
   const int k = (int)(rem / gm_cur);
-  mb = mg * p.GM + (int)(rem - (long long)k * gm_cur);
+  mb = mg * kGM + (int)(rem - (long long)k * gm_cur);
   img = k + p.img_rot;
   if (img >= p.nb_img) img -= p.nb_img;
   return true;
 }
 
 // ------------------------------------------------------------------------------------------------
-template <int G, int kStages, bool kArg>
+template <bool kArg>
 __global__ void __launch_bounds__(kTcThreads, 1) mindist_tc_kernel(const __grid_constant__ TcParams p) {
-  constexpr int kBRows = kMaxN / G;                         // bank rows staged per CTA per stage
   constexpr uint32_t kABytes = kTileM * kBlockK * 2;        // 16 KB
   constexpr uint32_t kBBytes = kBRows * kBlockK * 2;
   constexpr uint32_t kStageBytes = kABytes + kBBytes;
@@ -386,17 +332,15 @@ __global__ void __launch_bounds__(kTcThreads, 1) mindist_tc_kernel(const __grid_
   uint64_t* empty_bar = s_bar + kStages;      // [kStages]
   uint64_t* tfull_bar = s_bar + 2 * kStages;  // [2]
   uint64_t* tempty_bar = tfull_bar + 2;       // [2]
-  constexpr int kQD = 4;                                   // depth of the dynamic-scheduler unit queue
+  constexpr int kQD = 4;                                   // depth of the unit queue
   uint64_t* qfull_bar = tempty_bar + 2;                    // [kQD]
   uint64_t* qempty_bar = qfull_bar + kQD;                  // [kQD] (the leader CTA's copy collects both CTAs' readers)
   long long* s_qunit = reinterpret_cast<long long*>(qempty_bar + kQD);   // [kQD]
   uint32_t* s_tmem = reinterpret_cast<uint32_t*>(s_qunit + kQD);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = (G == 2) ? cluster_ctarank() : 0u;
+  const uint32_t rank = cluster_ctarank();
   const bool leader = (rank == 0);
-  const long long worker = (G == 2) ? (blockIdx.x >> 1) : blockIdx.x;
-  const long long nworkers = (G == 2) ? (gridDim.x >> 1) : gridDim.x;
   const long long total_units = p.sym ? __ldg(p.n_units) : p.total_units;
 
   if (warp == 0 && lane == 0) {
@@ -406,31 +350,30 @@ __global__ void __launch_bounds__(kTcThreads, 1) mindist_tc_kernel(const __grid_
     }
     for (int b = 0; b < 2; ++b) {
       mbar_init(smem_u32(&tfull_bar[b]), 1);
-      mbar_init(smem_u32(&tempty_bar[b]), 4 * G);  // one arrival per epilogue warp of every CTA in the group
+      mbar_init(smem_u32(&tempty_bar[b]), 4 * 2);  // one arrival per epilogue warp of both CTAs of the pair
     }
     for (int i = 0; i < kQD; ++i) {
       mbar_init(smem_u32(&qfull_bar[i]), 1);
-      mbar_init(smem_u32(&qempty_bar[i]), 5 * G);  // readers: MMA warp (or the peer's producer) + 4 epilogue warps per CTA
+      mbar_init(smem_u32(&qempty_bar[i]), 5 * 2);  // readers: MMA warp (or the peer's producer) + 4 epilogue warps per CTA
     }
     fence_barrier_init();
   }
   if (warp == 2) {
-    tmem_alloc<G>(smem_u32(s_tmem), kTmemCols);
-    tmem_relinquish<G>();
+    tmem_alloc(smem_u32(s_tmem), kTmemCols);
+    tmem_relinquish();
   }
   tc_fence_before();
-  if (G == 2) cluster_sync_all(); else __syncthreads();
+  cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *s_tmem;
 
-  // ---- unit sequence.  static: u = worker, worker + nworkers, ...   dynamic: the leader's producer claims units
-  // from a global counter and publishes them through a kQD-deep smem queue to every other role of the group.
-  const uint32_t qempty_leader0 = (G == 2) ? mapa_rank(smem_u32(&qempty_bar[0]), 0) : smem_u32(&qempty_bar[0]);
+  // ---- unit sequence: the leader's producer claims units from a global counter and publishes them through a kQD-deep
+  // smem queue to every other role of the pair.
+  const uint32_t qempty_leader0 = mapa_rank(smem_u32(&qempty_bar[0]), 0);
   auto queue_read = [&](uint32_t& qs, uint32_t& qph) -> long long {   // one lane per reader warp
     mbar_wait_cluster(smem_u32(&qfull_bar[qs]), qph, p.err, 5);
     const long long u = *reinterpret_cast<volatile long long*>(&s_qunit[qs]);
-    if (G == 2) mbar_arrive_cluster(qempty_leader0 + qs * 8);
-    else asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(qempty_leader0 + qs * 8) : "memory");
+    mbar_arrive_cluster(qempty_leader0 + qs * 8);
     if (++qs == kQD) { qs = 0; qph ^= 1; }
     return u;
   };
@@ -439,59 +382,47 @@ __global__ void __launch_bounds__(kTcThreads, 1) mindist_tc_kernel(const __grid_
     // ================================================================ TMA producer
     if (elect_one()) {
       uint32_t stage = 0, phase = 0;
-      const uint64_t pol = l2_policy_evict_last();
-      const uint32_t full0 = (G == 2) ? mapa_rank(smem_u32(&full_bar[0]), 0) : smem_u32(&full_bar[0]);
+      const uint32_t full0 = mapa_rank(smem_u32(&full_bar[0]), 0);
       uint32_t qs = 0, qph = 0;
-      long long u_static = worker;
       for (;;) {
         long long u;
-        if (!p.dynamic) {
-          u = (u_static < total_units) ? u_static : -1;
-          u_static += nworkers;
-        } else if (leader) {
+        if (leader) {
           mbar_wait_cluster(smem_u32(&qempty_bar[qs]), qph ^ 1, p.err, 6);   // slot free in both CTAs
           const unsigned long long c = atomicAdd(p.counter, 1ull);
           u = (c < (unsigned long long)total_units) ? (long long)c : -1;
           s_qunit[qs] = u;
           asm volatile("mbarrier.arrive.release.cta.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&qfull_bar[qs])) : "memory");
-          if (G == 2) {
-            st_cluster_s64(mapa_rank(smem_u32(&s_qunit[qs]), 1), u);
-            mbar_arrive_cluster(mapa_rank(smem_u32(&qfull_bar[qs]), 1));
-          }
+          st_cluster_s64(mapa_rank(smem_u32(&s_qunit[qs]), 1), u);
+          mbar_arrive_cluster(mapa_rank(smem_u32(&qfull_bar[qs]), 1));
           if (++qs == kQD) { qs = 0; qph ^= 1; }
         } else {
           u = queue_read(qs, qph);
         }
         if (u < 0) break;
         int mb, img;
-        if (!decode_unit<G>(p, u, mb, img)) continue;
+        if (!decode_unit(p, u, mb, img)) continue;
         if (p.bank_ready) {
           // the shard that holds this bank image may still be travelling (copy-engine pull on another stream): wait for its flag,
           // then order the flag read before the TMA (async proxy) reads of the landed rows
           wait_bank_ready(p, img);
           asm volatile("fence.proxy.async;" ::: "memory");
         }
-        const int arow = mb * (kTileM * G) + (int)rank * kTileM;
+        const int arow = mb * (kTileM * 2) + (int)rank * kTileM;
         for (int t = 0; t < p.nt; ++t) {
           const bool last = (t == p.nt - 1);
           const int width = last ? p.wlast : p.wmain;
-          const int brow = img * p.P + t * p.wmain + (int)rank * (width / G);
-          const uint32_t bbytes = (uint32_t)(width / G) * kBlockK * 2;
+          const int brow = img * p.P + t * p.wmain + (int)rank * (width / 2);
+          const uint32_t bbytes = (uint32_t)(width / 2) * kBlockK * 2;
           for (int seg = 0; seg < p.nseg; ++seg) {
             const CUtensorMap* ma = &p.mapA[seg == 1 ? 1 : 0];
             const CUtensorMap* mbp = last ? &p.mapBlast[seg == 2 ? 1 : 0] : &p.mapBmain[seg == 2 ? 1 : 0];
             for (int kb = 0; kb < p.nkb; ++kb) {
               mbar_wait(smem_u32(&empty_bar[stage]), phase ^ 1, p.err, 1);
-              if (leader) mbar_expect_tx(smem_u32(&full_bar[stage]), (kABytes + bbytes) * G);
+              if (leader) mbar_expect_tx(smem_u32(&full_bar[stage]), (kABytes + bbytes) * 2);
               const uint32_t fb = full0 + stage * 8;
               uint8_t* sa = smem + stage * kStageBytes;
-              if (p.l2_hint) {
-                tma_load_2d_hint<G>(smem_u32(sa), ma, fb, kb * kBlockK, arow, pol);
-                tma_load_2d_hint<G>(smem_u32(sa + kABytes), mbp, fb, kb * kBlockK, brow, pol);
-              } else {
-                tma_load_2d<G>(smem_u32(sa), ma, fb, kb * kBlockK, arow);
-                tma_load_2d<G>(smem_u32(sa + kABytes), mbp, fb, kb * kBlockK, brow);
-              }
+              tma_load_2d(smem_u32(sa), ma, fb, kb * kBlockK, arow);
+              tma_load_2d(smem_u32(sa + kABytes), mbp, fb, kb * kBlockK, brow);
               if (++stage == kStages) { stage = 0; phase ^= 1; }
             }
           }
@@ -504,18 +435,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) mindist_tc_kernel(const __grid_
       uint32_t stage = 0, phase = 0;
       uint32_t tile_ctr = 0;
       uint32_t qs = 0, qph = 0;
-      long long u_static = worker;
       for (;;) {
-        long long u;
-        if (!p.dynamic) {
-          u = (u_static < total_units) ? u_static : -1;
-          u_static += nworkers;
-        } else {
-          u = queue_read(qs, qph);
-        }
+        const long long u = queue_read(qs, qph);
         if (u < 0) break;
         int mb_, img_;
-        if (!decode_unit<G>(p, u, mb_, img_)) continue;
+        if (!decode_unit(p, u, mb_, img_)) continue;
         for (int t = 0; t < p.nt; ++t, ++tile_ctr) {
           const uint32_t buf = tile_ctr & 1, tphase = (tile_ctr >> 1) & 1;
           const uint32_t idesc = (t == p.nt - 1) ? p.idesc_last : p.idesc_main;
@@ -532,12 +456,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) mindist_tc_kernel(const __grid_
 #pragma unroll
             for (int k = 0; k < kBlockK / kUmmaK; ++k) {
               // advance 32 bytes (16 elements) along K inside the 128-byte swizzle row
-              umma_f16<G>(d_tmem, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (kb | k) != 0 ? 1u : 0u);
+              umma_f16(d_tmem, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (kb | k) != 0 ? 1u : 0u);
             }
-            umma_commit<G>(smem_u32(&empty_bar[stage]));     // frees the smem slot once these MMAs retire
+            umma_commit(smem_u32(&empty_bar[stage]));     // frees the smem slot once these MMAs retire
             if (++stage == kStages) { stage = 0; phase ^= 1; }
           }
-          umma_commit<G>(smem_u32(&tfull_bar[buf]));         // accumulator complete -> epilogue
+          umma_commit(smem_u32(&tfull_bar[buf]));         // accumulator complete -> epilogue
         }
       }
     }
@@ -546,30 +470,23 @@ __global__ void __launch_bounds__(kTcThreads, 1) mindist_tc_kernel(const __grid_
     const int q = warp & 3;                       // TMEM lane quarter this warp may access
     const int et = q * 32 + lane;                 // row inside the CTA tile == TMEM lane
     const int eidx = threadIdx.x - 64;            // 0..127
-    const uint32_t tempty0 = (G == 2) ? mapa_rank(smem_u32(&tempty_bar[0]), 0) : smem_u32(&tempty_bar[0]);
+    const uint32_t tempty0 = mapa_rank(smem_u32(&tempty_bar[0]), 0);
     uint32_t tile_ctr = 0;
     uint32_t qs = 0, qph = 0;
-    long long u_static = worker;
     for (;;) {
-      long long u;
-      if (!p.dynamic) {
-        u = (u_static < total_units) ? u_static : -1;
-        u_static += nworkers;
-      } else {
-        long long uu = 0;
-        if (lane == 0) uu = queue_read(qs, qph);
-        else if (++qs == kQD) { qs = 0; qph ^= 1; }      // keep every lane's queue cursor in step
-        u = __shfl_sync(0xffffffffu, uu, 0);
-      }
+      long long uu = 0;
+      if (lane == 0) uu = queue_read(qs, qph);
+      else if (++qs == kQD) { qs = 0; qph ^= 1; }      // keep every lane's queue cursor in step
+      const long long u = __shfl_sync(0xffffffffu, uu, 0);
       if (u < 0) break;
       int mb, img;
-      if (!decode_unit<G>(p, u, mb, img)) continue;
+      if (!decode_unit(p, u, mb, img)) continue;
       if (p.bank_ready) {
         // the norms of this bank image are read below, ahead of the accumulator: they travel with the rows, wait for the flag too
         if (lane == 0) wait_bank_ready(p, img);
         __syncwarp();
       }
-      const long long row = (long long)mb * (kTileM * G) + rank * kTileM + et;
+      const long long row = (long long)mb * (kTileM * 2) + rank * kTileM + et;
       const bool rvalid = row < p.Mq;
       // sym mode: this row contributes (row-min and column-min) only if its image owns the pair
       const int irow = p.q_img0 + (int)((rvalid ? row : p.Mq - 1) / p.P);
@@ -686,10 +603,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) mindist_tc_kernel(const __grid_
         }
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) {
-          if (G == 2) mbar_arrive_cluster(tempty0 + buf * 8);
-          else asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tempty0 + buf * 8) : "memory");
-        }
+        if (lane == 0) mbar_arrive_cluster(tempty0 + buf * 8);
       }
       if (act) {
         const float d2 = fmaxf(best + qn, 0.f);
@@ -701,8 +615,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) mindist_tc_kernel(const __grid_
 
   // ---------------------------------------------------------------- teardown
   tc_fence_before();
-  if (G == 2) cluster_sync_all(); else __syncthreads();
-  if (warp == 2) tmem_dealloc<G>(tmem_base, kTmemCols);
+  cluster_sync_all();
+  if (warp == 2) tmem_dealloc(tmem_base, kTmemCols);
 }
 
 
@@ -718,11 +632,11 @@ static constexpr int kUnitWarps = kUnitBlocks * 8;
 // The image range of every query block is tabulated in shared memory first, so the row loop carries no 64-bit division.
 // COUNT: returns the number of units of the run; otherwise emits them in raster order from position pos.
 template <bool COUNT>
-__device__ __forceinline__ long long walk_units(const TcParams& p, int G, int2* units, long long pos) {
+__device__ __forceinline__ long long walk_units(const TcParams& p, int2* units, long long pos) {
   __shared__ int s_i0[kUnitTab], s_i1[kUnitTab];
   const int tid = threadIdx.x, lane = tid & 31;
   const int gw = blockIdx.x * (blockDim.x >> 5) + (tid >> 5), nw = gridDim.x * (blockDim.x >> 5);
-  const long long rows_per_mb = (long long)kTileM * G;
+  const long long rows_per_mb = (long long)kTileM * 2;
   const bool tab = p.n_mblocks <= kUnitTab;
   auto mb_range = [&](int mb, int& i0, int& i1) {
     const long long r0 = (long long)mb * rows_per_mb, r1 = min(p.Mq, r0 + rows_per_mb) - 1;
@@ -743,9 +657,9 @@ __device__ __forceinline__ long long walk_units(const TcParams& p, int G, int2* 
       if (pair_owned_grouped(p.groups, i, img, p.nb_img)) return true;
     return false;
   };
-  const int n_groups = (p.n_mblocks + p.GM - 1) / p.GM;
+  const int n_groups = (p.n_mblocks + kGM - 1) / kGM;
   const long long rows = (long long)n_groups * p.KU;
-  // raster row = (group of GM query blocks, candidate bank image); the candidates of a group are walked circularly
+  // raster row = (group of kGM query blocks, candidate bank image); the candidates of a group are walked circularly
   // from the first image after the group's first query image (ownership looks forward in that order).
   // A contiguous slice of rows per warp keeps the raster order.
   const long long per = (rows + nw - 1) / nw;
@@ -754,14 +668,14 @@ __device__ __forceinline__ long long walk_units(const TcParams& p, int G, int2* 
   if (ra < rb) {
     int mg = (int)(ra / p.KU), k = (int)(ra - (long long)mg * p.KU);
     for (long long r = ra; r < rb; ++r) {
-      const int gm_cur = min(p.GM, p.n_mblocks - mg * p.GM);
+      const int gm_cur = min(kGM, p.n_mblocks - mg * kGM);
       int ig, i1_;
-      if (tab) ig = s_i0[mg * p.GM]; else mb_range(mg * p.GM, ig, i1_);
+      if (tab) ig = s_i0[mg * kGM]; else mb_range(mg * kGM, ig, i1_);
       int img = ig + 1 + k;                       // < 2 * nb_img
       if (img >= p.nb_img) img -= p.nb_img;
       if (img >= p.nb_img) img -= p.nb_img;
       for (int m0 = 0; m0 < gm_cur; m0 += 32) {
-        const int mi = m0 + lane, mb = mg * p.GM + mi;
+        const int mi = m0 + lane, mb = mg * kGM + mi;
         const bool act = (mi < gm_cur) && has_work(mb, img);
         const unsigned mask = __ballot_sync(0xffffffffu, act);
         if (COUNT) {
@@ -780,16 +694,16 @@ __device__ __forceinline__ long long walk_units(const TcParams& p, int G, int2* 
 // Two small multi-CTA launches instead of one CTA (which needed 46 us -- 3 % of an 8-GPU config-2 step -- whichever way its
 // single SM was used): every warp counts the units of its run of raster rows, then every warp sums the counts of the runs
 // before its own (fixed order) and emits.
-__global__ void __launch_bounds__(256) count_units_kernel(TcParams p, int G, long long* warp_cnt, int* err_flag) {
+__global__ void __launch_bounds__(256) count_units_kernel(TcParams p, long long* warp_cnt, int* err_flag) {
   if (blockIdx.x == 0 && threadIdx.x == 0 && err_flag) {
     *err_flag = 0;
-    *reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(err_flag) + 128) = 0ull;   // dynamic-scheduler counter
+    *reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(err_flag) + 128) = 0ull;   // unit claim counter
   }
-  const long long cnt = walk_units<true>(p, G, nullptr, 0);
+  const long long cnt = walk_units<true>(p, nullptr, 0);
   if ((threadIdx.x & 31) == 0) warp_cnt[blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)] = cnt;
 }
 
-__global__ void __launch_bounds__(256) emit_units_kernel(TcParams p, int G, const long long* __restrict__ warp_cnt, int2* units,
+__global__ void __launch_bounds__(256) emit_units_kernel(TcParams p, const long long* __restrict__ warp_cnt, int2* units,
                                                          long long* n_units) {
   const int lane = threadIdx.x & 31;
   const int gw = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), nw = gridDim.x * (blockDim.x >> 5);
@@ -805,7 +719,7 @@ __global__ void __launch_bounds__(256) emit_units_kernel(TcParams p, int G, cons
     all += __shfl_xor_sync(0xffffffffu, all, off);
   }
   if (gw == 0 && lane == 0) *n_units = all;
-  walk_units<false>(p, G, units, before);
+  walk_units<false>(p, units, before);
 }
 
 // grid-stride fill (SM-side replacement of cudaMemsetAsync: keeps the launch sequence off the copy engines)
@@ -871,28 +785,21 @@ static int* watchdog_flag() {
   return g_wd_dev;   // null when the allocation failed: the kernels then only trap
 }
 
-static int g_tc_cta_group = 2;   // test hook (ac_debug_set): 1 = single-CTA MMAs, 2 = CTA pairs
-static int g_tc_dynamic = 1;  // knob 4: dynamic unit scheduler (work stealing); measured 7 % faster than static round-robin
-static int g_tc_l2hint = 0;  // debug knob 3: L2 evict_last policy on operand loads (measured: no gain, off)
-static int g_tc_gm = 16;  // query blocks per raster group: 16 x 2 MB of A + the streaming bank images stay L2-resident (tuned on B200)
-
-template <int G, int kStages, bool kArg>
+template <bool kArg>
 static int launch_tc(const TcParams& prm, int num_sms, cudaStream_t st) {
-  constexpr int kBRows = kMaxN / G;
   constexpr size_t kStageBytes = (size_t)kTileM * kBlockK * 2 + (size_t)kBRows * kBlockK * 2;
   const size_t smem = 1024 + kStages * kStageBytes + 2 * kMaxN * sizeof(float) + (2 * kStages + 4) * 8 + 256;
-  auto kern = mindist_tc_kernel<G, kStages, kArg>;
+  auto kern = mindist_tc_kernel<kArg>;
   AC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const long long max_workers = (G == 2) ? num_sms / 2 : num_sms;
-  const int workers = (int)std::min<long long>(max_workers, prm.total_units);
+  const int pairs = (int)std::min<long long>(num_sms / 2, prm.total_units);
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(workers * G);
+  cfg.gridDim = dim3(pairs * 2);
   cfg.blockDim = dim3(kTcThreads);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = G;
+  attr[0].val.clusterDim.x = 2;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
@@ -911,7 +818,6 @@ int launch_mindist_tc(const void* Qhi, const void* Qlo, const float* Qn2, long l
   const bool x3 = (precision == AC_PREC_F16X3 || precision == AC_PREC_BF16X3);
   if (D % 8 != 0) return AC_ERR_UNSUPPORTED;  // TMA needs a 16-byte row pitch
   if (x3 && (!Qlo || !Blo)) return AC_ERR_INVALID;
-  const int G = g_tc_cta_group;
   TcParams prm;
   memset(&prm, 0, sizeof(prm));
   // tile widths inside one bank image: multiples of 16, <= 256, as even as possible
@@ -924,58 +830,54 @@ int launch_mindist_tc(const void* Qhi, const void* Qlo, const float* Qn2, long l
   prm.Mq = Mq; prm.nb_img = nb_img; prm.P = P; prm.D = D;
   prm.nkb = ceil_div(D, kBlockK);
   prm.nseg = x3 ? 3 : 1;
-  prm.n_mblocks = (int)ceil_div64(Mq, (long long)kTileM * G);
-  prm.GM = g_tc_gm;
-  prm.l2_hint = g_tc_l2hint;
-  prm.dynamic = g_tc_dynamic;
+  prm.n_mblocks = (int)ceil_div64(Mq, (long long)kTileM * 2);
   prm.counter = (unsigned long long*)((char*)err_flag + 128);   // inside the zeroed 256-byte workspace header
   prm.sym = sym; prm.q_img0 = q_img0; prm.colmin = colmin; prm.units = nullptr;
   prm.rowarg = rowarg; prm.colkey = colkey; prm.groups = groups; prm.bank_ready = bank_ready; prm.img_rot = sym ? 0 : img_rot;
   const bool arg = (rowarg != nullptr);
   if (arg && sym && !colkey) return AC_ERR_INVALID;
   prm.win_begin = win_begin; prm.win_count = (win_count < 0) ? nb_img : win_count;
-  // bank images a raster group of GM query blocks can own: N/2 after each of the images it spans (with categories the
+  // bank images a raster group of kGM query blocks can own: N/2 after each of the images it spans (with categories the
   // group may end in the middle of one whose images wrap around: every bank image is a candidate)
-  prm.KU = groups ? nb_img : std::min(nb_img, nb_img / 2 + (int)(((long long)prm.GM * kTileM * G - 1) / P) + 1);
+  prm.KU = groups ? nb_img : std::min(nb_img, nb_img / 2 + (int)(((long long)kGM * kTileM * 2 - 1) / P) + 1);
   prm.total_units = (long long)prm.n_mblocks * nb_img;
   if (sym) {
-    // raster order: groups of GM query blocks; inside a group walk the bank images the group owns and,
+    // raster order: groups of kGM query blocks; inside a group walk the bank images the group owns and,
     // per bank image, every block of the group that owns the pair (blocks sharing a bank image run
     // together).  Built on the device (count_units_kernel + emit_units_kernel).
     // a query block spans at most rows/P + 2 images, each owns at most half of its category (<= nb_img / 2 + 1 images)
-    const long long span = ((long long)kTileM * G + P - 1) / P + 1;
+    const long long span = ((long long)kTileM * 2 + P - 1) / P + 1;
     const long long max_units = (long long)prm.n_mblocks * std::min<long long>(nb_img, span * (nb_img / 2 + 1));
     if (!unit_ws || unit_ws_bytes < 16 + (size_t)max_units * sizeof(int2) + kUnitWarps * sizeof(long long)) return AC_ERR_WORKSPACE;
     long long* d_n = (long long*)unit_ws;
     int2* d_units = (int2*)((char*)unit_ws + 16);
     long long* d_cnt = (long long*)((char*)unit_ws + 16 + (size_t)max_units * sizeof(int2));     // one count per builder warp
-    count_units_kernel<<<kUnitBlocks, 256, 0, st>>>(prm, G, d_cnt, err_flag);
+    count_units_kernel<<<kUnitBlocks, 256, 0, st>>>(prm, d_cnt, err_flag);
     AC_LAUNCH_CHECK();
-    emit_units_kernel<<<kUnitBlocks, 256, 0, st>>>(prm, G, d_cnt, d_units, d_n);
+    emit_units_kernel<<<kUnitBlocks, 256, 0, st>>>(prm, d_cnt, d_units, d_n);
     AC_LAUNCH_CHECK();
     prm.units = d_units;
     prm.n_units = d_n;
     prm.total_units = max_units;   // upper bound (sizes the grid); the kernel reads the exact count
   }
-  prm.idesc_main = make_idesc(kTileM * G, wmain, bf16);
-  prm.idesc_last = make_idesc(kTileM * G, wlast, bf16);
+  prm.idesc_main = make_idesc(kTileM * 2, wmain, bf16);
+  prm.idesc_last = make_idesc(kTileM * 2, wlast, bf16);
   const long long brows = (long long)nb_img * P;
   int rc;
   if ((rc = make_map(&prm.mapA[0], Qhi, Mq, D, kTileM, bf16))) return rc;
-  if ((rc = make_map(&prm.mapBmain[0], Bhi, brows, D, wmain / G, bf16))) return rc;
-  if ((rc = make_map(&prm.mapBlast[0], Bhi, brows, D, wlast / G, bf16))) return rc;
+  if ((rc = make_map(&prm.mapBmain[0], Bhi, brows, D, wmain / 2, bf16))) return rc;
+  if ((rc = make_map(&prm.mapBlast[0], Bhi, brows, D, wlast / 2, bf16))) return rc;
   if (x3) {
     if ((rc = make_map(&prm.mapA[1], Qlo, Mq, D, kTileM, bf16))) return rc;
-    if ((rc = make_map(&prm.mapBmain[1], Blo, brows, D, wmain / G, bf16))) return rc;
-    if ((rc = make_map(&prm.mapBlast[1], Blo, brows, D, wlast / G, bf16))) return rc;
+    if ((rc = make_map(&prm.mapBmain[1], Blo, brows, D, wmain / 2, bf16))) return rc;
+    if ((rc = make_map(&prm.mapBlast[1], Blo, brows, D, wlast / 2, bf16))) return rc;
   } else {
     prm.mapA[1] = prm.mapA[0]; prm.mapBmain[1] = prm.mapBmain[0]; prm.mapBlast[1] = prm.mapBlast[0];
   }
   int dev = 0, num_sms = 0;
   AC_CUDA(cudaGetDevice(&dev));
   AC_CUDA(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
-  if (G == 2) return arg ? launch_tc<2, 6, true>(prm, num_sms, st) : launch_tc<2, 6, false>(prm, num_sms, st);
-  return arg ? launch_tc<1, 4, true>(prm, num_sms, st) : launch_tc<1, 4, false>(prm, num_sms, st);
+  return arg ? launch_tc<true>(prm, num_sms, st) : launch_tc<false>(prm, num_sms, st);
 }
 
 int launch_mindist_simt(const float* Q, long long Mq, const float* Bk, int nb_img, int P, int D, float* dmin, cudaStream_t st);
@@ -989,23 +891,6 @@ extern "C" int ac_last_watchdog(void) {
   const int code = *reinterpret_cast<volatile int*>(g_wd_host);
   *reinterpret_cast<volatile int*>(g_wd_host) = 0;
   return code;
-}
-
-// test / tuning hook (not part of the public header): key 0 = cta group (1|2), key 1 = M-blocks per raster group
-extern "C" int ac_debug_set_embed(int value);
-extern "C" int ac_debug_set_refine(int mb);
-extern "C" int ac_debug_set_refine_dot(int on);
-extern "C" int ac_debug_set_fused(int key, int value);
-extern "C" int ac_debug_set(int key, int value) {
-  if (key == 2) return ac_debug_set_embed(value);
-  if (key == 5) return ac_debug_set_refine(value);
-  if (key == 6) return ac_debug_set_refine_dot(value);
-  if (key >= 7 && key <= 13) return ac_debug_set_fused(key, value);
-  if (key == 0 && (value == 1 || value == 2)) { g_tc_cta_group = value; return AC_OK; }
-  if (key == 1 && value >= 1) { g_tc_gm = value; return AC_OK; }
-  if (key == 3 && (value == 0 || value == 1)) { g_tc_l2hint = value; return AC_OK; }
-  if (key == 4 && (value == 0 || value == 1)) { g_tc_dynamic = value; return AC_OK; }
-  return AC_ERR_INVALID;
 }
 
 // w[r] = mean over the other images j of the category of sqrt(d2(r, j)), d2 taken from whichever of the two minima the
@@ -1136,7 +1021,8 @@ extern "C" int ac_reduce_weights_sym(const float* rowmin_d2, const float* colmin
 extern "C" size_t ac_min_dist_workspace_bytes(int64_t Mq, int nb_img, int P, int D, int precision) {
   (void)D; (void)precision;
   // 256 B pipeline-watchdog flag + (symmetric form) the raster list of (query block, bank image) units
-  // sized for the smaller block (128 rows, single-CTA MMAs): more blocks, same per-block bound as launch_mindist_tc
+  // sized for 128-row query blocks: an upper bound for the 256-row blocks of the CTA pairs (more blocks, and a per-block
+  // span bound at least that of launch_mindist_tc)
   const long long mblocks = (Mq + 127) / 128;
   const long long span = (256 + std::max(1, P) - 1) / std::max(1, P) + 1;
   const long long per_mb = std::min<long long>(nb_img, span * (nb_img / 2 + 1));

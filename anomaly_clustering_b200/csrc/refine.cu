@@ -246,8 +246,6 @@ __global__ void __launch_bounds__(kRefThreads, 2) refine_kernel(const RefinePara
   }
 }
 
-static int g_refine_dot = 1;   // debug knob (ac_debug_set key 6): 1 = |q|^2+|b|^2-2q.b when norms are given, 0 = always sum (q-b)^2
-
 template <typename T, int NIT, bool LO, bool DOT>
 static int launch_refine(const RefineParams& p, dim3 grid, size_t smem, cudaStream_t st) {
   AC_CUDA(cudaFuncSetAttribute(refine_kernel<T, NIT, LO, DOT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -259,7 +257,7 @@ static int launch_refine(const RefineParams& p, dim3 grid, size_t smem, cudaStre
 template <typename T>
 static int dispatch_refine(const RefineParams& p, dim3 grid, size_t smem, cudaStream_t st) {
   if (p.Blo) return launch_refine<T, 0, true, false>(p, grid, smem, st);      // bank given as hi + lo: generic loop
-  if (p.Bn2 && g_refine_dot) {
+  if (p.Bn2) {                                                                  // |q|^2 + |b|^2 - 2 q.b
     if (p.D == 4096) return launch_refine<T, 16, false, true>(p, grid, smem, st);
     if (p.D == 1024) return launch_refine<T, 4, false, true>(p, grid, smem, st);
     return launch_refine<T, 0, false, true>(p, grid, smem, st);
@@ -272,18 +270,8 @@ static int dispatch_refine(const RefineParams& p, dim3 grid, size_t smem, cudaSt
 
 using namespace ac;
 
-static int g_refine_l2_mb = 128;  // debug knob (ac_debug_set key 5): bytes of bank operand rows one group keeps L2-resident (evict_last;
-                                  // measured at config 2 with the policy hints: 32 / 64 / 96 / 128 / 192 / 256 MB -> 14.7 / 11.6 / 11.8 / 10.3 / 10.8 / 10.8 ms)
-extern "C" int ac_debug_set_refine(int mb) {
-  if (mb < 1 || mb > 512) return AC_ERR_INVALID;
-  g_refine_l2_mb = mb;
-  return AC_OK;
-}
-extern "C" int ac_debug_set_refine_dot(int on) {
-  if (on != 0 && on != 1) return AC_ERR_INVALID;
-  ac::g_refine_dot = on;
-  return AC_OK;
-}
+static constexpr int kRefineL2MB = 128;  // MB of bank operand rows one group keeps L2-resident (evict_last; measured at config 2
+                                         // with the policy hints: 32 / 64 / 96 / 128 / 192 / 256 MB -> 14.7 / 11.6 / 11.8 / 10.3 / 10.8 / 10.8 ms)
 
 extern "C" int ac_refine_min_dist(const float* Zq, const void* Qhi, const void* Qlo, int64_t Mq, const void* Bhi, const void* Blo,
                                   int op_dtype, int nb_img, int P, int D, const int32_t* rowarg, const uint64_t* colkey, int sym,
@@ -304,9 +292,9 @@ extern "C" int ac_refine_min_dist(const float* Zq, const void* Qhi, const void* 
   p.rowarg = rowarg; p.colkey = (const unsigned long long*)colkey; p.sym = sym; p.q_img0 = q_img0; p.q_self = q_self; p.dex = dmin;
   p.groups = sym ? groups : nullptr;
   p.Bn2 = Bn2;
-  // bank images per group: their operand rows (128 MB by default, measured best on B200) stay L2-resident while every query chunk passes
+  // bank images per group: their operand rows (kRefineL2MB, measured best on B200) stay L2-resident while every query chunk passes
   const double img_bytes = (double)P * D * 2.0 * (Blo ? 2 : 1);
-  p.Jb = (int)std::max((double)kWPR, std::min(256.0, g_refine_l2_mb * 1.0e6 / img_bytes));
+  p.Jb = (int)std::max((double)kWPR, std::min(256.0, kRefineL2MB * 1.0e6 / img_bytes));
   p.Jb -= p.Jb % kWPR;                                             // the kWPR warps of a row take every kWPR-th image
   const long long chunks = (Mq + kRQ - 1) / kRQ;
   const int nbg = (nb_img + p.Jb - 1) / p.Jb;

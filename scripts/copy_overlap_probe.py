@@ -43,9 +43,6 @@ def t(fn, with_copy):
     return e0.elapsed_time(e1)
 
 
-from anomaly_clustering_b200 import _lib  # noqa: E402
-
-lib = _lib.load()
 out = torch.empty(n, n * P, dtype=torch.float32, device="cuda")
 
 
@@ -73,12 +70,5 @@ def report(name, fn):
 
 report("cuBLAS bf16 8192^3 x24", gemm)
 report("torch elementwise x40 (HBM-bound)", elementwise)
-report("mindist sym G=2", mind)
-report("mindist all-pairs half G=2", mind_half)
-lib.ac_debug_set(3, 2)
-report("mindist sym G=2, atomics dropped", mind)
-lib.ac_debug_set(3, 0)
-lib.ac_debug_set(0, 1)
-report("mindist sym G=1 (no clusters)", mind)
-report("mindist all-pairs half G=1", mind_half)
-lib.ac_debug_set(0, 2)
+report("mindist sym", mind)
+report("mindist all-pairs half", mind_half)

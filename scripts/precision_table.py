@@ -45,20 +45,3 @@ for prec in ("f16", "bf16", "f16r", "f16r (Z-free)", "f16x3", "bf16x3"):
                                            ((w - w_ex).abs() / w_ex).max().item()) + " | ".join("%.1e" % x for x in da)
           + " | %.1e | %d |" % (((X0 - X_ex[0]).norm() / X_ex[0].norm()).item(), flips), flush=True)
     del q
-# refine blocking: bank bytes one group keeps L2-resident
-from anomaly_clustering_b200 import _lib  # noqa: E402
-
-lib = _lib.load()
-q = pipeline.embed_images(feats, 3, 1, 2048, 4096, "f16r", want_z=True)
-for mb in (24, 48, 64, 96):
-    lib.ac_debug_set(5, mb)
-    pipeline.PROFILE = []
-    for _ in range(4):
-        pipeline.min_distance_weights(q, q, "unsupervised", "f16r")
-    torch.cuda.synchronize()
-    ev = pipeline.PROFILE
-    pipeline.PROFILE = None
-    b = [e for t, e in ev if t == "refine_begin"]
-    e_ = [e for t, e in ev if t == "refine_end"]
-    print("refine group budget %3d MB: %.2f ms per pass" % (mb, sum(x.elapsed_time(y) for x, y in zip(b[1:], e_[1:])) / (len(b) - 1)), flush=True)
-lib.ac_debug_set(5, 64)

@@ -1,8 +1,6 @@
-"""Fused single-pass embed (config-2 shape, 100 images): time per launch in isolation for the knobs of the lean kernel
-(look-ahead, L2 policy of the map loads, segment length, L2 prefetch distance, streaming stores), Z-free and with fp32 Z,
-against the per-layer launches of round 1 (variant 3) and the general fused kernel -- CUDA events, L2 flushed by the
-482 MB of maps themselves."""
-import itertools
+"""Fused single-pass embed (config-2 shape, 100 images): time per launch in isolation of the lean kernel, Z-free and with
+fp32 Z, against the per-layer launches of round 1 (variant 3) and the general fused kernel -- CUDA events, L2 flushed by
+the 482 MB of maps themselves."""
 import os
 import sys
 
@@ -15,23 +13,15 @@ from anomaly_clustering_b200 import _lib, ops, pipeline, synth  # noqa: E402
 
 lib = _lib.load()
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 100
-quick = len(sys.argv) > 2 and sys.argv[2] == "quick"
 layers = [(768, 28, 28, True), (768, 28, 28, True)]
 feats, _ = synth.planted_features_device(range(n), layers, device="cuda")
 P, D = 784, 4096
 maps = sum(f[:, 1:].numel() * 4 for f in feats)
-DEFAULTS = {7: 2, 8: 3, 9: 1, 10: 1, 11: 1, 12: 1, 13: 16}
-NAMES = {7: "look-ahead", 10: "prefetch", 11: "streaming-stores", 12: "l2-policy", 13: "segment"}
-
-
-def setk(**kw):
-    for k, v in kw.items():
-        assert lib.ac_debug_set(int(k[1:]), int(v)) == 0, (k, v)
 
 
 def reset():
-    for k, v in DEFAULTS.items():
-        lib.ac_debug_set(k, v)
+    lib.ac_debug_set(2, 0)
+    lib.ac_debug_set(9, 1)
 
 
 def timed(want_z, reps=20):
@@ -61,21 +51,5 @@ for want_z in (False, True):
     lib.ac_debug_set(9, 0)
     line(want_z, "general fused kernel", timed(want_z), nbytes)
     reset()
-    line(want_z, "lean fused, defaults %s" % DEFAULTS, timed(want_z), nbytes)
-    if quick:
-        continue
-    grid = itertools.product((2, 3), (0, 1), (0, 1)) if not want_z else itertools.product((2,), (1,), (0, 1))
-    for la, pol, pd in grid:
-        reset()
-        setk(k7=la, k12=pol, k10=pd)
-        line(want_z, "lean fused  look-ahead %d  l2-policy %d  prefetch %d" % (la, pol, pd), timed(want_z), nbytes)
-    for cps in (2, 3):
-        reset()
-        setk(k8=cps)
-        line(want_z, "lean fused  CTAs/SM %d" % cps, timed(want_z), nbytes)
-    for seg, cs in ((16, 0),):
-        reset()
-        setk(k13=seg, k11=cs)
-        line(want_z, "lean fused  defaults but segment %2d  streaming-stores %d" % (seg, cs), timed(want_z), nbytes)
-reset()
+    line(want_z, "lean fused kernel", timed(want_z), nbytes)
 reset()
