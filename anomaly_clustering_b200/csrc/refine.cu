@@ -281,6 +281,8 @@ extern "C" int ac_refine_min_dist(const float* Zq, const void* Qhi, const void* 
   if (op_dtype != AC_DT_F16 && op_dtype != AC_DT_BF16) return AC_ERR_INVALID;
   if (sym && (!colkey || Pq != P)) return AC_ERR_INVALID;
   if (D % 8 != 0) return AC_ERR_UNSUPPORTED;                       // 16-byte operand vectors
+  for (const void* v : {(const void*)Zq, Qhi, Qlo, Bhi, Blo})      // ... read from 16-byte aligned rows
+    if (reinterpret_cast<uintptr_t>(v) % 16 != 0) return AC_ERR_INVALID;
   const size_t smem = (size_t)kRQ * D * sizeof(float);
   if (smem > 200 * 1024) return AC_ERR_UNSUPPORTED;
   int rc = check_device();

@@ -111,9 +111,11 @@ __global__ void __launch_bounds__(256) alpha_kernel(const float* __restrict__ w,
   }
 }
 
-// X[i, d] = sum_p alpha[i,p] * Z[i,p,d]; grid (ceil(D / (128*4)), N); each thread owns 4 columns
+// X[i, d] = sum_p alpha[i,p] * Z[i,p,d]; grid (ceil(D / (128*4)), N); each thread owns 4 columns.
+// vec (decided on the host): D % 4 == 0 and Z, X 16-byte aligned -- float4 loads and stores; else the scalar loop, which
+// sums in the same order (bit-identical results).
 __global__ void __launch_bounds__(128) weighted_embed_kernel(const float* __restrict__ alpha, const float* __restrict__ Z, int N, int P,
-                                                             int D, float* __restrict__ X) {
+                                                             int D, float* __restrict__ X, bool vec) {
   extern __shared__ float s_alpha[];
   const int i = blockIdx.y;
   for (int p = threadIdx.x; p < P; p += blockDim.x) s_alpha[p] = alpha[(long long)i * P + p];
@@ -121,7 +123,7 @@ __global__ void __launch_bounds__(128) weighted_embed_kernel(const float* __rest
   const int d0 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
   if (d0 >= D) return;
   const float* zi = Z + (long long)i * P * D;
-  if (d0 + 3 < D && (D & 3) == 0) {
+  if (vec) {
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll 4
     for (int p = 0; p < P; ++p) {
@@ -221,8 +223,15 @@ __global__ void __launch_bounds__(256) pairwise_l2_kernel(const float* __restric
 }
 
 // small N (one category: N ~ 100): one warp per (i, j >= i) pair, X stays L2-resident; the tiled
-// kernel above would run only ~N^2/2048 CTAs
-__global__ void __launch_bounds__(256) pairwise_l2_warp_kernel(const float* __restrict__ X, int N, int D, float* __restrict__ Dm) {
+// kernel above would run only ~N^2/2048 CTAs.  vec (decided on the host: X 16-byte aligned) picks float4 loads; without it
+// the same four elements are loaded one by one and summed in the same order (bit-identical results).
+__device__ __forceinline__ float4 ld4(const float* p, bool vec) {
+  if (vec) return __ldg(reinterpret_cast<const float4*>(p));
+  return make_float4(__ldg(p), __ldg(p + 1), __ldg(p + 2), __ldg(p + 3));
+}
+
+__global__ void __launch_bounds__(256) pairwise_l2_warp_kernel(const float* __restrict__ X, int N, int D, float* __restrict__ Dm,
+                                                               bool vec) {
   const long long w = blockIdx.x * (long long)(blockDim.x >> 5) + (threadIdx.x >> 5);
   if (w >= (long long)N * N) return;
   const int i = (int)(w / N), j = (int)(w - (long long)i * N);
@@ -233,8 +242,8 @@ __global__ void __launch_bounds__(256) pairwise_l2_warp_kernel(const float* __re
   float acc = 0.f;
   if ((D & 3) == 0) {
     for (int d = lane * 4; d < D; d += 128) {
-      const float4 a = __ldg(reinterpret_cast<const float4*>(xi + d));
-      const float4 b = __ldg(reinterpret_cast<const float4*>(xj + d));
+      const float4 a = ld4(xi + d, vec);
+      const float4 b = ld4(xj + d, vec);
       float t;
       t = a.x - b.x; acc = fmaf(t, t, acc);
       t = a.y - b.y; acc = fmaf(t, t, acc);
@@ -327,8 +336,10 @@ extern "C" int ac_weighted_embed(const float* alpha, const float* Z, int N, int 
   auto kern = weighted_embed_kernel;
   const size_t smem = (size_t)P * sizeof(float);
   if (smem > 48 * 1024) AC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  // float4 path only when every vector access is 16-byte aligned (a contiguous view may start anywhere)
+  const bool vec = (D % 4 == 0) && (reinterpret_cast<uintptr_t>(Z) % 16 == 0) && (reinterpret_cast<uintptr_t>(X) % 16 == 0);
   dim3 grid(ceil_div(D, 128 * 4), N);
-  kern<<<grid, 128, smem, (cudaStream_t)stream>>>(alpha, Z, N, P, D, X);
+  kern<<<grid, 128, smem, (cudaStream_t)stream>>>(alpha, Z, N, P, D, X, vec);
   AC_LAUNCH_CHECK();
   return AC_OK;
 }
@@ -380,7 +391,8 @@ extern "C" int ac_pairwise_l2(const float* X, int N, int D, float* Dmat, ac_stre
   if (N == 0) return AC_OK;
   if (N <= 384) {
     const long long warps = (long long)N * N;
-    pairwise_l2_warp_kernel<<<(unsigned)((warps + 7) / 8), 256, 0, (cudaStream_t)stream>>>(X, N, D, Dmat);
+    const bool vec = reinterpret_cast<uintptr_t>(X) % 16 == 0;   // float4 loads (rows are 16-byte aligned when D % 4 == 0)
+    pairwise_l2_warp_kernel<<<(unsigned)((warps + 7) / 8), 256, 0, (cudaStream_t)stream>>>(X, N, D, Dmat, vec);
   } else {
     dim3 grid(ceil_div(N, 32), ceil_div(N, 32));
     pairwise_l2_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(X, N, D, Dmat);

@@ -184,7 +184,8 @@ int ac_reduce_weights_sym(const float* rowmin_d2, const float* colmin_d2, int64_
  * ([ceil(Mq/Pq)] bank index of each query image, or NULL) names pairs to skip.  Bn2 (the bank operands' squared norms,
  * as for ac_min_dist; may be NULL) lets a pair cost one FFMA per element.  Feed dmin to ac_reduce_weights.
  * Costs one gathered 2*D-byte row per (query row, bank image): ~1/3 of the one-pass GEMM time at config 2.
- * Needs D % 8 == 0 and D <= 12800, else AC_ERR_UNSUPPORTED (use the X3 modes). */
+ * Needs D % 8 == 0 and D <= 12800, else AC_ERR_UNSUPPORTED (use the X3 modes).  Zq, Qhi, Qlo, Bhi and Blo (those given)
+ * must be 16-byte aligned (it reads them as 16-byte vectors), else AC_ERR_INVALID. */
 int ac_min_dist_arg(const void* Qhi, const void* Qlo, const float* Qn2, int64_t Mq, const void* Bhi, const void* Blo,
                     const float* Bn2, int nb_img, int P, int D, int precision, float* dmin, int32_t* argmin, void* ws,
                     size_t ws_bytes, ac_stream_t stream);
@@ -233,13 +234,14 @@ int ac_reduce_weights_ex(const float* dmin, int64_t Mq, int nb_img, int Pq, cons
 
 /* ---- stage 3 -----------------------------------------------------------------------------------
  * alpha[t, i, :] = softmax_p(w[i, :] / tau_t) in float64, max-subtracted (identical to
- * Matrix_Alpha_* wherever the reference's exp does not overflow, utils.py:246-255); |tau| < 1e-9
- * gives the reference's one-hot-on-max with ties split equally (:248-250).
+ * Matrix_Alpha_* wherever the reference's exp does not overflow, utils.py:246-255); tau == 0 gives
+ * one-hot (the reference's math.isclose(tau, 0)): one-hot-on-max with ties split equally (:248-250).
  * alpha64 [T,N,P] double and/or alpha32 [T,N,P] float (either may be NULL). taus_host: HOST array. */
 int ac_alpha(const float* w, int N, int P, const double* taus_host, int T, double* alpha64,
              float* alpha32, ac_stream_t stream);
 
-/* X[i, :] = sum_p alpha[i,p] * Z[i,p,:]   (torch.bmm line, examples/main.py:294-296). */
+/* X[i, :] = sum_p alpha[i,p] * Z[i,p,:]   (torch.bmm line, examples/main.py:294-296).  Any alignment of Z and X: the
+ * vector loads need D % 4 == 0 and 16-byte aligned Z and X, other calls take a scalar loop with the same result bits. */
 int ac_weighted_embed(const float* alpha, const float* Z, int N, int P, int D, float* X,
                       ac_stream_t stream);
 
@@ -267,7 +269,8 @@ int ac_copy_blocks(int n, const void* const* src_host, const int64_t* src_stride
                    ac_stream_t stream);
 
 /* Dmat[i,j] = || X[i] - X[j] ||_2, the Euclidean matrix Ward linkage consumes
- * (examples/test.py:193-195 -> scipy pdist).  Dmat [N,N] fp32, exactly symmetric, zero diagonal. */
+ * (examples/test.py:193-195 -> scipy pdist).  Dmat [N,N] fp32, exactly symmetric, zero diagonal.  Any alignment of X
+ * (vector loads only when X is 16-byte aligned; the result bits do not depend on it). */
 int ac_pairwise_l2(const float* X, int N, int D, float* Dmat, ac_stream_t stream);
 
 #ifdef __cplusplus
