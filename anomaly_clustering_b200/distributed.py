@@ -7,25 +7,25 @@ w_i, alpha_i and X_i depend only on query image i and the read-only bank
   other ranks' query rows are exchanged)  ->  all-gather of the X rows  ->  Dmat.  fp32 Z never leaves its rank.
 On CPU (gloo) the same sharding / gather logic is exercised by tests with a stand-in compute.
 
-Schedules of the symmetric sharded path (DESIGN.md section 6); the default needs no environment variable:
-  AC_SHARD_TRANSPORT=symm (default on NCCL groups with the CUDA back-end) | nccl
-        symm: the embed kernel writes into a symmetric-memory bank, every rank pulls the shards it needs with copy-engine copies
-        (symm_transport.SymmetricBank); nccl: all-gather / point-to-point collectives (automatic fallback, and always on gloo)
-  AC_SHARD_FLAGS=1 (default, symm only) | 0
-        1: ONE distance launch per step whose loader waits for per-bank-image arrival flags (ac_min_dist_sym_ready);
-        0: one launch per window of landed shards (AC_SHARD_MERGE=1 merges shards that will have landed anyway)
-  AC_SYMM_COLMIN=1 (default, symm only) | 0
-        1: column minima written into symmetric memory and collected with one ac_copy_blocks launch; 0: NCCL all_to_all
-  AC_SHARD_PIPELINE=1   (nccl transport, more than two ranks) shard-granular ring of pairwise exchanges, one launch per shard
-  AC_OVERLAP_MIN_WORLD  (nccl transport) smallest world size at which the local-shard launch overlaps the gather (default 2)"""
+The operand shards travel over one of two transports (DESIGN.md section 6):
+  symmetric memory  the embed kernel writes into this rank's slice of a symmetric-memory bank, every rank pulls the shards it
+                    needs with copy-engine copies (symm_transport.SymmetricBank), ONE distance launch waits for per-bank-image
+                    arrival flags (ac_min_dist_sym_ready), and the column minima are exchanged through symmetric memory too.
+                    Chosen by _symmetric_bank: the CUDA back-end on an NCCL group of more than one rank, a tensor-core
+                    precision, and a set-up that succeeds; run_path_sharded also needs the symmetric form with P >= 32.
+  NCCL collectives  everywhere else (gloo groups, precision 'f32', P < 32, symmetric memory that cannot be set up): the bank
+                    shards are all-gathered or sent point to point, the local shard is multiplied while they travel, and the
+                    column minima go through an all_to_all (exchange_colmin)."""
 from __future__ import annotations
 
 import functools
-import os
 from typing import List, Optional, Sequence, Tuple
 
 import torch
 import torch.distributed as dist
+
+from . import ops, pipeline
+from .symm_transport import SymmetricBank
 
 
 def pair_owned(i: int, j: int, n: int) -> bool:
@@ -143,82 +143,6 @@ def start_gather_needed_rows(local: torch.Tensor, bounds: Sequence[Tuple[int, in
     return buf, reqs
 
 
-def start_shard_pipeline(locals_: Sequence[Optional[torch.Tensor]], bounds: Sequence[Tuple[int, int]], rows_per_item: int,
-                         need: Sequence[Sequence[int]], group=None):
-    """Needed-shard transfers as a ring of pairwise steps: step k (k = 1 .. world-1) receives the shard of rank
-    (rank + k) % world and sends the local shard to rank (rank - k) % world, when the receiver needs it -- both
-    sides evaluate the same predicate, so every step is a matched exchange.  Each step is its own batch, so the
-    caller can multiply against shard k while shards k+1.. are still in flight (they arrive in the order the
-    symmetric kernel's circular bank window consumes them).  `locals_` are row blocks that travel together
-    (operand hi / lo / norms; None entries are skipped).  Returns (buffers, [(source rank, requests), ...])."""
-    rank, world = dist.get_rank(group), dist.get_world_size(group)
-    total = bounds[-1][1] * rows_per_item
-    a, b = bounds[rank]
-    bufs = []
-    for t in locals_:
-        if t is None:
-            bufs.append(None)
-            continue
-        buf = torch.empty((total,) + tuple(t.shape[1:]), dtype=t.dtype, device=t.device)
-        buf[a * rows_per_item : b * rows_per_item].copy_(t)
-        bufs.append(buf)
-    srcs = [t.contiguous() for t in locals_ if t is not None]
-    dsts = [x for x in bufs if x is not None]
-    steps = []
-    for send_to, recv_from in shard_pipeline_plan(need, rank, world):
-        ops_ = []
-        if send_to is not None:
-            ops_ += [dist.P2POp(dist.isend, t, send_to, group=group) for t in srcs]
-        if recv_from is not None:
-            sa, sb = bounds[recv_from]
-            ops_ += [dist.P2POp(dist.irecv, x[sa * rows_per_item : sb * rows_per_item], recv_from, group=group) for x in dsts]
-        reqs = dist.batch_isend_irecv(ops_) if ops_ else []
-        if recv_from is not None or reqs:
-            steps.append((recv_from, reqs))  # recv_from None = send-only step: nothing to multiply, requests must complete
-    return bufs, steps
-
-
-def shard_pipeline_plan(need: Sequence[Sequence[int]], rank: int, world: int) -> List[Tuple[Optional[int], Optional[int]]]:
-    """Pure host logic of start_shard_pipeline: for ring step k = 1 .. world-1 the pair (send_to, recv_from) of this
-    rank, None where nothing travels.  Rank r sends to d = r-k exactly when d receives from d+k = r, so the steps of all
-    ranks pair up one to one (tests/test_distributed_cpu.py simulates every rank and checks it)."""
-    plan = []
-    for k in range(1, world):
-        src, dst = (rank + k) % world, (rank - k) % world
-        plan.append((dst if rank in need[dst] else None, src if src in need[rank] else None))
-    return plan
-
-
-@functools.lru_cache(maxsize=256)
-def plan_pull_windows(bounds: Tuple[Tuple[int, int], ...], n_total: int, rank: int, order: Tuple[int, ...], P: int, D: int,
-                      row_bytes: int, pull_gbps: float = 600.0, gemm_tflops: float = 1300.0) -> Tuple[Tuple[int, ...], ...]:
-    """Groups the shards that arrive in ring order `order` into GEMM launches: a launch takes every shard expected to have
-    landed when the previous launch ends (at least one), so that the kernel never waits for data it could have been
-    given later and no launch is smaller than it has to be.  Estimates: copy-engine pulls at `pull_gbps`, the symmetric
-    kernel at `gemm_tflops` on the pairs this rank owns.  Pure host logic (cached); returns tuples of source ranks."""
-    a, b = bounds[rank]
-
-    def pairs(src):
-        sa, sb = bounds[src]
-        return sum(pair_owned(i, j, n_total) for i in range(a, b) for j in range(sa, sb))
-
-    t = pairs(rank) * 2.0 * P * P * D / (gemm_tflops * 1e12)            # the local window runs first
-    landed, acc = [], 0.0
-    for src in order:
-        acc += (bounds[src][1] - bounds[src][0]) * P * row_bytes / (pull_gbps * 1e9)
-        landed.append(acc)
-    groups, k = [], 0
-    while k < len(order):
-        take = [order[k]]
-        k += 1
-        while k < len(order) and landed[k] <= t:
-            take.append(order[k])
-            k += 1
-        t = max(t, landed[k - 1]) + sum(pairs(s_) for s_ in take) * 2.0 * P * P * D / (gemm_tflops * 1e12)
-        groups.append(tuple(take))
-    return tuple(groups)
-
-
 def start_all_gather_rows(local: torch.Tensor, counts: Sequence[int], group=None):
     """Asynchronous all-gather of row blocks into one buffer whose local slice is already valid, so work on
     the local shard can overlap the collective.  Returns (buffer, [work])."""
@@ -252,13 +176,6 @@ def start_all_gather_rows(local: torch.Tensor, counts: Sequence[int], group=None
     return buf, [work]
 
 
-def gather_needed_rows(local, bounds, rows_per_item, need, group=None) -> torch.Tensor:
-    buf, reqs = start_gather_needed_rows(local, bounds, rows_per_item, need, group)
-    for r in reqs:
-        r.wait()
-    return buf
-
-
 def _weighted_embed_all_taus(compute, a32, Z3, T: int) -> torch.Tensor:
     """[n_r, T, D]: one pass over Z for all taus when the compute back-end has the fused form (the CUDA library), else per tau."""
     if hasattr(compute, "weighted_embed_multi"):
@@ -289,6 +206,133 @@ def exchange_colmin(colmin: torch.Tensor, bounds: Sequence[Tuple[int, int]], P: 
     return torch.cat(recv, dim=0)
 
 
+class _CudaCompute:
+    """The default compute back-end of the sharded paths: the CUDA library (tests substitute a CPU stand-in)."""
+
+    embed_images = staticmethod(pipeline.embed_images)
+    min_distance_weights = staticmethod(pipeline.min_distance_weights)
+    alpha = staticmethod(ops.alpha)
+    weighted_embed = staticmethod(ops.weighted_embed)
+    weighted_embed_multi = staticmethod(ops.weighted_embed_multi)
+    weighted_embed_from_features = staticmethod(ops.weighted_embed_from_features)
+    pairwise_l2 = staticmethod(ops.pairwise_l2)
+    min_dist_sym = staticmethod(ops.min_dist_sym)
+    min_dist_sym_arg = staticmethod(ops.min_dist_sym_arg)
+    refine_min_dist = staticmethod(ops.refine_min_dist)
+    reduce_weights_sym = staticmethod(ops.reduce_weights_sym)
+    reduce_weights = staticmethod(ops.reduce_weights)
+
+
+def _symmetric_bank(compute, rows: int, D: int, precision: str, device, group) -> Optional[SymmetricBank]:
+    """The symmetric-memory bank of `rows` operand rows of width D, or None where the NCCL collectives carry the operands:
+    a back-end other than the CUDA library, a group that is not NCCL or has one rank, precision 'f32' (no tensor-core
+    operands), or a symmetric-memory set-up that fails (reported once; the transport then stays off in this process)."""
+    if not (compute is _CudaCompute and dist.get_world_size(group) > 1 and dist.get_backend(group) == "nccl"
+            and precision != "f32" and SymmetricBank.disabled_reason is None):
+        return None
+    operand, want_lo = pipeline._OPERAND_OF[precision]
+    try:
+        return SymmetricBank.get(rows, D, torch.float16 if operand == "f16" else torch.bfloat16, want_lo, device, group)
+    except Exception as e:  # noqa: BLE001 -- symmetric memory unavailable on this system: say so once, use NCCL
+        SymmetricBank.disabled_reason = repr(e)
+        import warnings
+
+        warnings.warn("symmetric-memory transport unavailable (%r): the sharded path uses NCCL collectives" % (e,))
+        return None
+
+
+def _sym_minima_symmetric_memory(compute, symm_bank: SymmetricBank, q, bounds, n_total: int, precision: str, rank: int,
+                                 world: int):
+    """Symmetric form over the symmetric-memory transport.  q's operands already sit in this rank's slice of the bank.
+    The needed shards are pulled on the copy engines while ONE distance launch runs over the whole bank: its loader waits
+    for a bank image's arrival flag before reading it (measured on one GPU with the launches of an 8-GPU config-2 rank:
+    2.40 ms in one launch against 2.59 ms in three windows of landed shards).  The column minima (keys in the refined
+    modes) are written straight into symmetric memory and collected by SymmetricBank.exchange_colmin.
+    Returns (bank, minima of the launch, column block [N, n_r*P])."""
+    P, (lo_i, hi_i) = q.P, bounds[rank]
+    refined = precision in pipeline.REFINED
+    pipeline._mark("gather_begin")
+    # every shard for the refined modes (each rank re-evaluates all of its rows against the whole bank)
+    need = [r for r in range(world) if r != rank] if refined else needed_shards(bounds, n_total)[rank]
+    ready = torch.zeros(n_total, dtype=torch.int32, device=q.hi.device)
+    ready[lo_i:hi_i] = 1
+    (hi_buf, lo_buf, n2_buf), pulls = symm_bank.publish_and_pull(bounds, P, need, rank, world, ready)
+    bank = pipeline.PatchSet(n_total, P, q.D, q.grid, hi=hi_buf, lo=lo_buf, n2=n2_buf)
+    pipeline._mark("gather_end")
+    n_max = max(b - a for a, b in bounds)
+    Mq = q.n_img * P
+    rowmin = torch.empty(n_total, Mq, dtype=torch.float32, device=q.hi.device)
+    if refined:
+        out = (rowmin, torch.zeros(n_total, Mq, dtype=torch.int32, device=q.hi.device),
+               symm_bank.colmin_buffer(q.n_img, n_max, n_total * P, torch.int64))
+    else:
+        out = (rowmin, symm_bank.colmin_buffer(q.n_img, n_max, n_total * P, torch.float32))
+    launch = compute.min_dist_sym_arg if refined else compute.min_dist_sym
+    pipeline._mark("mindist_begin")
+    out = launch(q.hi, q.lo, q.n2, lo_i, bank.hi, bank.lo, bank.n2, n_total, P, precision, init=True, out=out, ready=ready)
+    pipeline._mark("mindist_end")
+    # the launch itself does not need the pulls to have completed; refine and the next step's buffer reuse do
+    for r in pulls:
+        r.wait()
+    pipeline._mark("exchange_begin")
+    colfull = symm_bank.exchange_colmin(bounds, P, rank, world)
+    pipeline._mark("exchange_end")
+    return bank, out, colfull
+
+
+def _sym_minima_nccl(compute, q, bounds, n_total: int, precision: str, group):
+    """Symmetric form over NCCL collectives: the bank shards travel asynchronously while the pairs inside the local shard
+    are multiplied, the remote bank images follow in a second launch, and the column minima go through exchange_colmin.
+    Returns (bank, minima of the launches, column block [N, n_r*P])."""
+    rank, world = dist.get_rank(group), dist.get_world_size(group)
+    P, (lo_i, hi_i) = q.P, bounds[rank]
+    refined = precision in pipeline.REFINED
+    launch = compute.min_dist_sym_arg if refined else compute.min_dist_sym
+    pipeline._mark("gather_begin")
+    if (3 <= world <= 4 or dist.get_backend(group) != "nccl") and not refined:
+        # 3-4 ranks: point-to-point transfers of just the shards that hold bank images of pairs this rank owns (the next
+        # n_total//2 images, about 2/3 of the volume).  At 2 ranks the needed shard IS the other rank's shard and NCCL's
+        # all-gather moves it faster (0.5 vs 0.9 ms).
+        need = needed_shards(bounds, n_total)
+        hi_buf, r1 = start_gather_needed_rows(q.hi, bounds, P, need, group)
+        lo_buf, r2 = (None, []) if q.lo is None else start_gather_needed_rows(q.lo, bounds, P, need, group)
+        n2_buf, r3 = start_gather_needed_rows(q.n2, bounds, P, need, group)
+    else:
+        # many ranks: NCCL's all-gather moves the whole bank faster than 4+ send/recv pairs per rank
+        # move half of it (measured at 8 GPUs: 562 MB in 1.0 ms vs 321 MB in 1.2 ms)
+        row_counts = [(b - a) * P for a, b in bounds]
+        hi_buf, r1 = start_all_gather_rows(q.hi, row_counts, group)
+        lo_buf, r2 = (None, []) if q.lo is None else start_all_gather_rows(q.lo, row_counts, group)
+        n2_buf, r3 = start_all_gather_rows(q.n2, row_counts, group)
+    pending = list(r1) + list(r2) + list(r3)
+    bank = pipeline.PatchSet(n_total, P, q.D, q.grid, hi=hi_buf, lo=lo_buf, n2=n2_buf)
+    pipeline._mark("gather_end")
+    # NCCL's transfer kernels take a few SMs away from the persistent GEMM; its dynamic unit scheduler absorbs that (with
+    # the earlier static round-robin the overlap cost more than it hid at 2 ranks).  A one-rank group transfers nothing.
+    if pending and q.n_img > 1 and world > 1:
+        # phase 1: bank images of the local shard (no remote data needed) overlaps the NCCL transfers
+        pipeline._mark("mindist_begin")
+        out = launch(q.hi, q.lo, q.n2, lo_i, bank.hi, bank.lo, bank.n2, n_total, P, precision,
+                     bank_window=(lo_i, q.n_img), init=True)
+        pipeline._mark("mindist_end")
+        for r in pending:
+            r.wait()
+        pipeline._mark("mindist_begin")
+        out = launch(q.hi, q.lo, q.n2, lo_i, bank.hi, bank.lo, bank.n2, n_total, P, precision,
+                     bank_window=(hi_i % n_total, n_total - q.n_img), init=False, out=out)
+        pipeline._mark("mindist_end")
+    else:
+        for r in pending:
+            r.wait()
+        pipeline._mark("mindist_begin")
+        out = launch(q.hi, q.lo, q.n2, lo_i, bank.hi, bank.lo, bank.n2, n_total, P, precision)
+        pipeline._mark("mindist_end")
+    pipeline._mark("exchange_begin")
+    colfull = exchange_colmin(out[-1], bounds, P, group)   # float minima, or (distance, row) keys when refined
+    pipeline._mark("exchange_end")
+    return bank, out, colfull
+
+
 def run_path_sharded(
     local_features: Sequence[torch.Tensor],
     n_total: int,
@@ -309,215 +353,42 @@ def run_path_sharded(
     `compute` (tests only) substitutes the compute back-end -- an object with embed_images,
     min_distance_weights, alpha, weighted_embed, pairwise_l2 -- so that the sharding / gather logic
     can be exercised on CPU with gloo; the default is the CUDA library and nothing else."""
-    from . import pipeline
-
     precision = pipeline.resolve_precision(precision, taus)
     if compute is None:
-        from . import ops
-
-        class _Cuda:
-            embed_images = staticmethod(pipeline.embed_images)
-            min_distance_weights = staticmethod(pipeline.min_distance_weights)
-            alpha = staticmethod(ops.alpha)
-            weighted_embed = staticmethod(ops.weighted_embed)
-            weighted_embed_multi = staticmethod(ops.weighted_embed_multi)
-            pairwise_l2 = staticmethod(ops.pairwise_l2)
-            min_dist_sym = staticmethod(ops.min_dist_sym)
-            supports_bank_window = True
-            is_cuda_backend = True
-            weighted_embed_from_features = staticmethod(ops.weighted_embed_from_features)
-            reduce_weights_sym = staticmethod(ops.reduce_weights_sym)
-            min_dist_sym_arg = staticmethod(ops.min_dist_sym_arg)
-            refine_min_dist = staticmethod(ops.refine_min_dist)
-            reduce_weights = staticmethod(ops.reduce_weights)
-
-        compute = _Cuda
-
+        compute = _CudaCompute
     rank, world = dist.get_rank(group), dist.get_world_size(group)
     if n_total < world:
         # an empty shard has no patch grid to agree on; callers with fewer images than ranks pass a sub-group
         raise ValueError("run_path_sharded: %d images over %d ranks leaves empty shards; use a smaller group" % (n_total, world))
     bounds = shard_bounds(n_total, world)
     lo_i, hi_i = bounds[rank]
-    compute_is_cuda = getattr(compute, "is_cuda_backend", False)
     z_free = (not keep_z) and hasattr(compute, "weighted_embed_from_features") and pipeline.z_free_supported(
         local_features, patchsize, stride, pretrain_dim, target_dim, precision) and precision not in pipeline.REFINED
     refined = precision in pipeline.REFINED
-    # transport of the operand shards: copy-engine pulls from symmetric memory (symm_transport.py) on NCCL / CUDA groups
-    # with the CUDA back-end; NCCL collectives otherwise (AC_SHARD_TRANSPORT=nccl forces them)
-    views0 = local_features[0]
-    P_guess = None
-    symm_bank = None
-    want_symm = (symmetric and compute_is_cuda and world > 1 and dist.get_backend(group) == "nccl" and precision != "f32"
-                 and os.environ.get("AC_SHARD_TRANSPORT", "symm") == "symm")
-    if want_symm:
-        from . import ops as _ops
-        from .symm_transport import SymmetricBank
-
-        v0 = _ops.feature_view(views0)
-        gh, gw = _ops.patch_grid(v0.shape[2], v0.shape[3], patchsize, stride)
-        P_guess = gh * gw
-        if P_guess >= 32 and SymmetricBank.disabled_reason is None:
-            operand, want_lo = pipeline._OPERAND_OF[precision]
-            try:
-                symm_bank = SymmetricBank.get(n_total * P_guess, target_dim, torch.float16 if operand == "f16" else torch.bfloat16,
-                                              want_lo, v0.device, group)
-            except Exception as e:  # noqa: BLE001 -- symmetric memory unavailable on this system: say so once, use NCCL
-                SymmetricBank.disabled_reason = repr(e)
-                import warnings
-
-                warnings.warn("symmetric-memory transport unavailable (%r): the sharded path uses NCCL collectives" % (e,))
-    if symm_bank is not None:
-        outs = symm_bank.local_slices(lo_i * P_guess, hi_i * P_guess)
-        q = compute.embed_images(local_features, patchsize, stride, pretrain_dim, target_dim, precision, want_z=not z_free, out=outs)
-    else:
-        q = compute.embed_images(local_features, patchsize, stride, pretrain_dim, target_dim, precision, want_z=not z_free)
+    symm_bank = outs = None
+    if symmetric:
+        v0 = ops.feature_view(local_features[0])
+        gh, gw = ops.patch_grid(v0.shape[2], v0.shape[3], patchsize, stride)
+        if gh * gw >= 32:   # the symmetric kernel's shapes (use_sym below)
+            symm_bank = _symmetric_bank(compute, n_total * gh * gw, target_dim, precision, v0.device, group)
+        if symm_bank is not None:   # the embed kernel writes straight into this rank's slice of the bank
+            outs = symm_bank.local_slices(lo_i * gh * gw, hi_i * gh * gw)
+    q = compute.embed_images(local_features, patchsize, stride, pretrain_dim, target_dim, precision, want_z=not z_free, out=outs)
     assert q.n_img == hi_i - lo_i
     P = q.P
-    row_counts = [(b - a) * P for a, b in bounds]
     use_sym = symmetric and precision != "f32" and P >= 32 and hasattr(compute, "min_dist_sym")
     # refined modes ('f16r'): the tensor-core pass records arg-mins, ac_refine_min_dist re-evaluates the selected pairs
     # exactly.  Every rank refines ALL (own row, other image) entries, so it needs the whole bank (every shard) and the
     # (distance, row) keys of the column minima travel instead of the float minima.
     if refined and not (use_sym and hasattr(compute, "min_dist_sym_arg")):
         raise ValueError("precision %r needs the symmetric sharded path" % precision)
-    sym_launch = compute.min_dist_sym_arg if refined else compute.min_dist_sym
-    pipeline._mark("gather_begin")
-    pending = []
-    pipeline_steps = None
-    symm_colmin = False
-    ready_flags = None
-    # opt-in (AC_SHARD_PIPELINE=1): shard-granular pipeline -- multiply against shard k while shards k+1.. travel
-    shard_pipeline = use_sym and getattr(compute, "supports_bank_window", False) and (
-        symm_bank is not None or (world > 2 and os.environ.get("AC_SHARD_PIPELINE", "0") == "1" and not refined))
-    if symm_bank is not None and not shard_pipeline:
-        raise RuntimeError("symmetric transport chosen for a shape the windowed kernel does not take")
-    if shard_pipeline:
-        need_all = needed_shards(bounds, n_total)
-        if symm_bank is not None:
-            # every shard for the refined modes (each rank re-evaluates all of its rows against the whole bank)
-            need_rank = [r for r in range(world) if r != rank] if refined else need_all[rank]
-            if os.environ.get("AC_SHARD_FLAGS", "1") == "1":
-                # ONE distance launch for the local and all remote bank images: its loader waits for per-image arrival flags
-                # that the side stream sets after each shard's pull (ac_min_dist_sym_ready) -- measured on one GPU with the
-                # launches of an 8-GPU config-2 rank: 2.40 ms in one launch against 2.59 ms in three windows
-                ready_flags = torch.zeros(n_total, dtype=torch.int32, device=q.hi.device)
-                ready_flags[lo_i:hi_i] = 1
-            (hi_buf, lo_buf, n2_buf), pipeline_steps = symm_bank.publish_and_pull(bounds, P, need_rank, rank, world, ready=ready_flags)
-        else:
-            (hi_buf, lo_buf, n2_buf), pipeline_steps = start_shard_pipeline([q.hi, q.lo, q.n2], bounds, P, need_all, group)
-        bank = pipeline.PatchSet(n_total, P, q.D, q.grid, hi=hi_buf, lo=lo_buf, n2=n2_buf)
-    elif use_sym:
-        # only the shards that hold bank images of pairs this rank owns (the next n_total//2 images);
-        # the transfers stay in flight while the pairs inside the local shard are multiplied
-        if (3 <= world <= 4 or dist.get_backend(group) != "nccl") and not refined:
-            # 3-4 ranks: point-to-point transfers of just the needed shards (about 2/3 of the volume).  At 2 ranks
-            # the needed shard IS the other rank's shard and NCCL's all-gather moves it faster (0.5 vs 0.9 ms).
-            need = needed_shards(bounds, n_total)
-            hi_buf, r1 = start_gather_needed_rows(q.hi, bounds, P, need, group)
-            lo_buf, r2 = (None, []) if q.lo is None else start_gather_needed_rows(q.lo, bounds, P, need, group)
-            n2_buf, r3 = start_gather_needed_rows(q.n2, bounds, P, need, group)
-        else:
-            # many ranks: NCCL's all-gather moves the whole bank faster than 4+ send/recv pairs per rank
-            # move half of it (measured at 8 GPUs: 562 MB in 1.0 ms vs 321 MB in 1.2 ms)
-            hi_buf, r1 = start_all_gather_rows(q.hi, row_counts, group)
-            lo_buf, r2 = (None, []) if q.lo is None else start_all_gather_rows(q.lo, row_counts, group)
-            n2_buf, r3 = start_all_gather_rows(q.n2, row_counts, group)
-        pending = list(r1) + list(r2) + list(r3)
-        bank = pipeline.PatchSet(n_total, P, q.D, q.grid, hi=hi_buf, lo=lo_buf, n2=n2_buf)
-    elif precision == "f32":
-        bank = pipeline.PatchSet(n_total, P, q.D, q.grid, Z=all_gather_rows(q.Z, row_counts, group))
-    else:
-        bank = pipeline.PatchSet(
-            n_total, P, q.D, q.grid,
-            hi=all_gather_rows(q.hi, row_counts, group),
-            lo=None if q.lo is None else all_gather_rows(q.lo, row_counts, group),
-            n2=all_gather_rows(q.n2, row_counts, group),
-        )
-    pipeline._mark("gather_end")
     if use_sym:
         # every unordered image pair is multiplied once, by the rank that owns the pair's first image;
-        # the column minima it produces for other ranks' query rows travel in one small all-to-all
-        # NCCL's transfer kernels take a few SMs away from the persistent GEMM; its dynamic unit scheduler
-        # absorbs that (with the earlier static round-robin the overlap cost more than it hid at 2 ranks).
-        min_world = int(os.environ.get("AC_OVERLAP_MIN_WORLD", "2"))
-        two_phase = bool(pending) and q.n_img > 1 and world >= min_world and getattr(compute, "supports_bank_window", False)
-        if shard_pipeline:
-            windows = [((lo_i, q.n_img), [])] if q.n_img > 1 else []          # the local shard needs no transfer
-            if symm_bank is not None and pipeline_steps and os.environ.get("AC_SHARD_MERGE", "1") == "1":
-                # copy-engine pulls land faster than the GEMM consumes them: merge the shards that will have landed
-                # anyway into one launch (consecutive ring shards form one circular window of bank images)
-                by_src = dict(pipeline_steps)
-                order = tuple(src for src, _ in pipeline_steps)
-                row_bytes = q.D * q.hi.element_size() * (2 if q.lo is not None else 1)
-                for grp in plan_pull_windows(tuple(tuple(b_) for b_ in bounds), n_total, rank, order, P, q.D, row_bytes):
-                    count = sum(bounds[s_][1] - bounds[s_][0] for s_ in grp)
-                    windows.append(((bounds[grp[0]][0], count), by_src[grp[-1]]))  # the last shard's event covers the group
-            else:
-                for src, reqs in pipeline_steps:
-                    windows.append((None if src is None else (bounds[src][0], bounds[src][1] - bounds[src][0]), reqs))
-            out, first = None, True
-            if symm_bank is not None and os.environ.get("AC_SYMM_COLMIN", "1") == "1":
-                # the column minima (keys in the refined modes) are written straight into symmetric memory; see
-                # SymmetricBank.exchange_colmin
-                n_max = max(b_ - a_ for a_, b_ in bounds)
-                Mq_l = q.n_img * P
-                rowmin_l = torch.empty(n_total, Mq_l, dtype=torch.float32, device=q.hi.device)
-                if refined:
-                    out = (rowmin_l, torch.zeros(n_total, Mq_l, dtype=torch.int32, device=q.hi.device),
-                           symm_bank.colmin_buffer(q.n_img, n_max, n_total * P, torch.int64))
-                else:
-                    out = (rowmin_l, symm_bank.colmin_buffer(q.n_img, n_max, n_total * P, torch.float32))
-                symm_colmin = True
-            if ready_flags is not None:
-                # flags mode: a single launch over the whole bank now; the pull events are awaited after it (refine and the
-                # next step's buffer reuse need them, the launch itself does not)
-                all_reqs = [r for _, reqs in windows for r in reqs]
-                windows = [(None, [])]
-                pipeline._mark("mindist_begin")
-                out = sym_launch(q.hi, q.lo, q.n2, lo_i, bank.hi, bank.lo, bank.n2, n_total, P, precision, init=True, out=out,
-                                 ready=ready_flags)
-                pipeline._mark("mindist_end")
-                first = False
-                for r in all_reqs:
-                    r.wait()
-            for window, reqs in windows:
-                for r in reqs:
-                    r.wait()
-                if window is None:
-                    continue
-                pipeline._mark("mindist_begin")
-                out = sym_launch(q.hi, q.lo, q.n2, lo_i, bank.hi, bank.lo, bank.n2, n_total, P, precision,
-                                 bank_window=window, init=first, out=out)
-                pipeline._mark("mindist_end")
-                first = False
-            if first and symm_colmin:
-                # this rank owns no pair at all (two images on two ranks): its peers still read its column minima -- "unset"
-                out[-1].view(torch.int32).fill_(0x7F7F7F7F)
-        elif two_phase:
-            # phase 1: bank images of the local shard (no remote data needed) overlaps the NCCL transfers
-            pipeline._mark("mindist_begin")
-            out = sym_launch(q.hi, q.lo, q.n2, lo_i, bank.hi, bank.lo, bank.n2, n_total, P, precision,
-                             bank_window=(lo_i, q.n_img), init=True)
-            pipeline._mark("mindist_end")
-            for r in pending:
-                r.wait()
-            pipeline._mark("mindist_begin")
-            out = sym_launch(q.hi, q.lo, q.n2, lo_i, bank.hi, bank.lo, bank.n2, n_total, P, precision,
-                             bank_window=(hi_i % n_total, n_total - q.n_img), init=False, out=out)
-            pipeline._mark("mindist_end")
+        # the column minima it produces for other ranks' query rows travel back to their owners
+        if symm_bank is not None:
+            bank, out, colfull = _sym_minima_symmetric_memory(compute, symm_bank, q, bounds, n_total, precision, rank, world)
         else:
-            for r in pending:
-                r.wait()
-            pipeline._mark("mindist_begin")
-            out = sym_launch(q.hi, q.lo, q.n2, lo_i, bank.hi, bank.lo, bank.n2, n_total, P, precision)
-            pipeline._mark("mindist_end")
-        pipeline._mark("exchange_begin")
-        if symm_colmin:
-            colfull = symm_bank.exchange_colmin(bounds, P, rank, world)
-        else:
-            colfull = exchange_colmin(out[-1], bounds, P, group)   # float minima, or (distance, row) keys when refined
-        pipeline._mark("exchange_end")
+            bank, out, colfull = _sym_minima_nccl(compute, q, bounds, n_total, precision, group)
         if refined:
             pipeline._mark("refine_begin")
             dex = compute.refine_min_dist(q.Z, q.hi, q.lo, bank.hi, bank.lo, n_total, P, out[1], colkey=colfull, q_img0=lo_i,
@@ -528,6 +399,18 @@ def run_path_sharded(
         else:
             w = compute.reduce_weights_sym(out[0], colfull, P, lo_i).reshape(q.n_img, P)
     else:
+        row_counts = [(b - a) * P for a, b in bounds]
+        pipeline._mark("gather_begin")
+        if precision == "f32":
+            bank = pipeline.PatchSet(n_total, P, q.D, q.grid, Z=all_gather_rows(q.Z, row_counts, group))
+        else:
+            bank = pipeline.PatchSet(
+                n_total, P, q.D, q.grid,
+                hi=all_gather_rows(q.hi, row_counts, group),
+                lo=None if q.lo is None else all_gather_rows(q.lo, row_counts, group),
+                n2=all_gather_rows(q.n2, row_counts, group),
+            )
+        pipeline._mark("gather_end")
         q_self = torch.arange(lo_i, hi_i, dtype=torch.int32, device=q.hi.device if q.Z is None else q.Z.device)
         w = compute.min_distance_weights(q, bank, "unsupervised", precision, q_self=q_self)
     a64, a32 = compute.alpha(w, list(taus))
@@ -566,24 +449,9 @@ def run_path_sharded_supervised(
     the local bank shard is multiplied while the gather is in flight (`overlap`), the remote pieces after it.
     Returns (alpha64_local [T,n_r,P], X_all [T,N,D], Dmat [T,N,N], w_local) like run_path_sharded.
     `compute`: tests only, see run_path_sharded."""
-    from . import pipeline
-
     precision = pipeline.resolve_precision(precision, taus)
     if compute is None:
-        from . import ops
-
-        class _Cuda:
-            embed_images = staticmethod(pipeline.embed_images)
-            min_distance_weights = staticmethod(pipeline.min_distance_weights)
-            alpha = staticmethod(ops.alpha)
-            weighted_embed = staticmethod(ops.weighted_embed)
-            weighted_embed_multi = staticmethod(ops.weighted_embed_multi)
-            pairwise_l2 = staticmethod(ops.pairwise_l2)
-
-        compute = _CUDA_SUPERVISED = _Cuda
-    else:
-        _CUDA_SUPERVISED = None
-
+        compute = _CudaCompute
     rank, world = dist.get_rank(group), dist.get_world_size(group)
     if n_total < world or n_bank_total < world:
         raise ValueError("run_path_sharded_supervised: %d query / %d bank images over %d ranks leaves empty shards; "
@@ -602,24 +470,10 @@ def run_path_sharded_supervised(
         cut = lambda t: None if t is None else t[a * P : b * P]  # noqa: E731
         return pipeline.PatchSet(b - a, P, q.D, q.grid, Z=cut(Zb), hi=cut(hib), lo=cut(lob), n2=cut(n2b))
 
-    # Symmetric-memory transport for the bank (default on NCCL groups with the CUDA back-end, as in run_path_sharded): the bank
-    # shard is embedded straight into a symmetric buffer, every rank pulls the other shards with copy-engine copies, and ONE
-    # all-pairs launch walks the bank from the local shard on while they land (arrival flags, ac_min_dist_ready).
-    symm_bank = None
-    if (world > 1 and compute is _CUDA_SUPERVISED and precision != "f32" and dist.get_backend(group) == "nccl" and P >= 1
-            and os.environ.get("AC_SHARD_TRANSPORT", "symm") == "symm" and os.environ.get("AC_SHARD_FLAGS", "1") == "1"):
-        from .symm_transport import SymmetricBank
-
-        if SymmetricBank.disabled_reason is None:
-            operand, want_lo = pipeline._OPERAND_OF[precision]
-            try:
-                symm_bank = SymmetricBank.get(n_bank_total * P, target_dim, torch.float16 if operand == "f16" else torch.bfloat16,
-                                              want_lo, q.hi.device, group)
-            except Exception as e:  # noqa: BLE001 -- symmetric memory unavailable: say so once, use NCCL
-                SymmetricBank.disabled_reason = repr(e)
-                import warnings
-
-                warnings.warn("symmetric-memory transport unavailable (%r): the sharded path uses NCCL collectives" % (e,))
+    # Symmetric-memory transport for the bank (as in run_path_sharded): the bank shard is copied into a symmetric buffer,
+    # every rank pulls the other shards with copy-engine copies, and ONE all-pairs launch walks the bank from the local shard
+    # on while they land (arrival flags, ac_min_dist_ready).
+    symm_bank = _symmetric_bank(compute, n_bank_total * P, target_dim, precision, local_features[0].device, group)
     if symm_bank is not None:
         lo_b, hi_b = bb[rank]
         hi_s, lo_s, n2_s = symm_bank.local_slices(lo_b * P, hi_b * P)
@@ -630,17 +484,16 @@ def run_path_sharded_supervised(
         pipeline._mark("gather_begin")
         ready = torch.zeros(n_bank_total, dtype=torch.int32, device=q.hi.device)
         ready[lo_b:hi_b] = 1
-        (hib, lob, n2b), steps = symm_bank.publish_and_pull(bb, P, [r for r in range(world) if r != rank], rank, world, ready=ready)
+        (hib, lob, n2b), pulls = symm_bank.publish_and_pull(bb, P, [r for r in range(world) if r != rank], rank, world, ready)
         pipeline._mark("gather_end")
-        reqs = [r for _, rr in steps for r in rr]
 
         def landed():
-            for r in reqs:
+            for r in pulls:
                 r.wait()
 
         bank_all = pipeline.PatchSet(n_bank_total, P, q.D, q.grid, hi=hib, lo=lob, n2=n2b)
         w = compute.min_distance_weights(q, bank_all, "supervised", precision, bank_ready=ready, bank_first=lo_b, bank_landed=landed)
-        return _supervised_tail(compute, pipeline, q, w, taus, qb, P, group)
+        return _supervised_tail(compute, q, w, taus, qb, P, group)
 
     pipeline._mark("gather_begin")
     pending = []
@@ -666,10 +519,10 @@ def run_path_sharded_supervised(
         if b > a:
             wp = compute.min_distance_weights(q, piece(bufs, a, b), "supervised", precision)
             w = wp if w is None else torch.minimum(w, wp)
-    return _supervised_tail(compute, pipeline, q, w, taus, qb, P, group)
+    return _supervised_tail(compute, q, w, taus, qb, P, group)
 
 
-def _supervised_tail(compute, pipeline, q, w, taus, qb, P, group):
+def _supervised_tail(compute, q, w, taus, qb, P, group):
     """alpha, X of the local query rows, all-gather of the X rows, Dmat (stage 3 of run_path_sharded_supervised)."""
     a64, a32 = compute.alpha(w, list(taus))
     Z3 = q.Z.reshape(q.n_img, P, q.D)
@@ -685,8 +538,6 @@ def run_path_sharded_average(local_features: Sequence[torch.Tensor], n_total: in
                              target_dim: int, group=None):
     """'average' mode (examples/main.py:290-291: alpha = 1/P) sharded by query image: every rank reduces its own images,
     the X rows are all-gathered, Dmat on every rank.  Returns (X_all [1,N,D], Dmat [1,N,N])."""
-    from . import ops, pipeline
-
     rank, world = dist.get_rank(group), dist.get_world_size(group)
     bounds = shard_bounds(n_total, world)
     r = pipeline.run_path(local_features, patchsize, stride, pretrain_dim, target_dim, "average", keep_z=False)

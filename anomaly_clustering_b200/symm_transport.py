@@ -1,5 +1,5 @@
-"""Copy-engine transport of the tensor-core operands for the sharded path (default on NCCL / CUDA groups;
-AC_SHARD_TRANSPORT=nccl switches back to NCCL collectives).
+"""Copy-engine transport of the tensor-core operands for the sharded path (used on NCCL groups with the CUDA back-end;
+distributed._symmetric_bank decides, and falls back to NCCL collectives when symmetric memory cannot be set up).
 
 Why (measured at 8 B200, config 2, profiles/r02_timeline_*): NCCL moves a rank's 80 MB operand shard at 120-140 GB/s
 through its send/recv kernels and the uneven all-gather (grouped broadcasts, LL protocol) needs 1.2 ms for 562 MB -- both
@@ -9,8 +9,8 @@ allocated as torch symmetric memory (CUDA VMM allocations mapped into every rank
   * the embed kernel writes its operands and norms STRAIGHT into this rank's slice of the symmetric bank (no staging copy),
   * one device-side barrier publishes the slices,
   * every rank PULLS the shards it needs from the peer mappings with plain device-to-device copies on a side stream:
-    they run on the copy engines at NVLink speed, cost no SM while the persistent GEMM is running, and each shard has
-    its own event, so the GEMM window of shard k starts as soon as shard k has landed (ring order rank+1, rank+2, ...).
+    they run on the copy engines at NVLink speed and cost no SM while the persistent GEMM is running (ring order
+    rank+1, rank+2, ...).
 
 Two buffer sets alternate between steps, so ONE barrier per buffer kind and step is enough: a rank reaches the barrier of step
 t+1 only after its stream has consumed every shard it pulled in step t, hence after that barrier the set of step t may be
@@ -24,7 +24,7 @@ The same object carries the two later stages of the step:
     peer's buffer, instead of an NCCL all_to_all."""
 from __future__ import annotations
 
-from typing import List, Optional, Sequence, Tuple
+from typing import Optional, Sequence, Tuple
 
 import torch
 
@@ -86,17 +86,18 @@ class SymmetricBank:
         return cur["peers"][key]
 
     def publish_and_pull(self, bounds: Sequence[Tuple[int, int]], P: int, need_rank: Sequence[int], rank: int, world: int,
-                         ready: Optional[torch.Tensor] = None):
+                         ready: torch.Tensor):
         """After the local slices were written on the current stream: barrier, then pull the shards of `need_rank`.
-        Returns ((hi_buf, lo_buf, n2_buf), [(source rank, [request]), ...]) in arrival (ring) order.
         ready [n_total] int32 (zeroed by the caller on the current stream): the flags of a shard's images are set to 1 on the
-        side stream right after its copies -- the arrival flags of ac_min_dist_sym_ready."""
+        side stream right after its copies -- the arrival flags of ac_min_dist_sym_ready.
+        Returns ((hi_buf, lo_buf, n2_buf), requests): one request whose wait() orders the current stream after the last
+        pull (the side stream runs in order, so after every pull), or none when nothing is pulled."""
         cur = self.sets[self.step & 1]
         self.step += 1
         main = torch.cuda.current_stream()
         cur["handles"][0].barrier(channel=0)              # stream-ordered: every rank's slice of this set is written
         self.side.wait_stream(main)
-        steps: List[Tuple[int, list]] = []
+        pulled = False
         with torch.cuda.stream(self.side):
             for k in range(1, world):
                 src = (rank + k) % world
@@ -110,12 +111,13 @@ class SymmetricBank:
                         continue
                     peer = self._peer(cur, which, src)
                     buf[sa * P : sb * P].copy_(peer[sa * P : sb * P], non_blocking=True)
-                if ready is not None:
-                    ready[sa:sb].fill_(1)
-                ev = torch.cuda.Event()
-                ev.record(self.side)
-                steps.append((src, [_EventRequest(ev)]))
-        return cur["bufs"], steps
+                ready[sa:sb].fill_(1)
+                pulled = True
+        if not pulled:
+            return cur["bufs"], []
+        ev = torch.cuda.Event()
+        ev.record(self.side)
+        return cur["bufs"], [_EventRequest(ev)]
 
     # ---- column minima (symmetric form): every rank writes its [n_r, N*P] block straight into symmetric memory, and after ONE
     # barrier each rank pulls the columns that belong to its query rows from every peer.  Replaces the NCCL all_to_all of

@@ -1,5 +1,5 @@
 #!/bin/bash
-# First GPU calls of the next round: validate and time the two opt-in multi-GPU schedules written at the end of
+# First GPU calls of the next round: validate and time the multi-GPU path.  The two opt-in schedules it also timed, since removed, were written at the end of
 # round 1 without hardware (DESIGN.md section 8 items 1-2).  Run with:  gpurun --gpus 8 --timeout 600 -- 'bash scripts/r02_first_calls.sh 8'
 # Every command is bounded by `timeout`; a hang in a new NCCL / symmetric-memory schedule must not hold the box.
 N=${1:-8}
@@ -8,17 +8,13 @@ mkdir -p $OUT
 # 0. single GPU: random-geometry fuzz of ac_embed against the oracle (promote into tests/ once green)
 timeout 200 python scripts/fuzz_embed_gpu.py 60 > $OUT/fuzz_embed.log 2>&1; echo "fuzz embed rc=$?"; tail -3 $OUT/fuzz_embed.log
 TR="python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1"
-# 1. bit-identity of the shard-granular NCCL pipeline (and the default schedules) against one GPU
-timeout 150 $TR --master-port 29551 scripts/check_sharded.py > $OUT/check_pipeline_n$N.log 2>&1; echo "check pipeline rc=$?"
-# 2. same with the symmetric-memory copy-engine transport
-AC_CHECK_SYMM=1 timeout 150 $TR --master-port 29552 scripts/check_sharded.py > $OUT/check_symm_n$N.log 2>&1; echo "check symm rc=$?"
-# 3. A/B timing, config 2
+# 1. the sharded path (symmetric-memory transport, NCCL collectives, all-pairs form) against one GPU
+timeout 150 $TR --master-port 29551 scripts/check_sharded.py > $OUT/check_sharded_n$N.log 2>&1; echo "check sharded rc=$?"
+# 2. timing, config 2
 timeout 120 $TR --master-port 29553 bench.py --gpus $N --steps 20 --warmup 5 --no-e2e > $OUT/bench_default_n$N.json 2> $OUT/bench_default_n$N.err
-AC_SHARD_PIPELINE=1 timeout 120 $TR --master-port 29554 bench.py --gpus $N --steps 20 --warmup 5 --no-e2e > $OUT/bench_pipeline_n$N.json 2> $OUT/bench_pipeline_n$N.err
-AC_SHARD_PIPELINE=1 AC_SHARD_TRANSPORT=symm timeout 120 $TR --master-port 29555 bench.py --gpus $N --steps 20 --warmup 5 --no-e2e > $OUT/bench_symm_n$N.json 2> $OUT/bench_symm_n$N.err
-# 4. sharded supervised path at N ranks (validated at 1 and 2 ranks in round 1)
+# 3. sharded supervised path at N ranks (validated at 1 and 2 ranks in round 1)
 timeout 150 $TR --master-port 29556 scripts/check_supervised_sharded.py > $OUT/check_supervised_n$N.log 2>&1; echo "check supervised rc=$?"
-# 5. configs 3 and 5 at N ranks (1-GPU numbers: scripts/run_configs.py)
+# 4. configs 3 and 5 at N ranks (1-GPU numbers: scripts/run_configs.py)
 timeout 240 $TR --master-port 29557 scripts/run_configs_sharded.py > $OUT/configs_n$N.log 2>&1; echo "configs rc=$?"; tail -1 $OUT/configs_n$N.log
 grep -h "OK\|MISMATCH" $OUT/check_*_n$N.log | tail -40
 for f in $OUT/bench_*_n$N.json; do python - "$f" <<'PY'

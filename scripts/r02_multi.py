@@ -1,8 +1,9 @@
 """torchrun --nproc-per-node N scripts/r02_multi.py [out_dir]: every multi-GPU measurement of round 2 in ONE process group
 (one NCCL init instead of one per bench invocation; multi-GPU box time is charged N-fold):
-  1. the sharded path against one GPU (default two-phase schedule, shard pipeline, refined precision), uneven shards;
-  2. bench.py lines (same code, same JSON) for config 2 under the schedules, configs 3, 4 (joint), 4pc, 5;
-  3. a kineto timeline of three config-2 steps on rank 0 for the default schedule and the shard pipeline."""
+  1. the sharded path against one GPU (default transport, NCCL collectives, all-pairs form, refined precision), uneven shards;
+  2. bench.py lines (same code, same JSON) for config 2 (fp16 and f16r), configs 3, 4 (joint), 4pc, 5;
+  3. a kineto timeline of three config-2 steps on rank 0 for the symmetric-memory transport and the NCCL collectives.
+The NCCL collectives are forced in-process through SymmetricBank.disabled_reason."""
 import io
 import json
 import os
@@ -18,6 +19,7 @@ import torch.distributed as dist  # noqa: E402
 
 import bench  # noqa: E402
 from anomaly_clustering_b200 import distributed, pipeline, synth  # noqa: E402
+from anomaly_clustering_b200.symm_transport import SymmetricBank  # noqa: E402
 
 OUT = sys.argv[1] if len(sys.argv) > 1 else os.path.join(ROOT, "gpurun_out", "r02_multi")
 rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
@@ -29,6 +31,18 @@ if rank == 0:
     os.makedirs(OUT, exist_ok=True)
 dist.barrier()
 T0 = time.time()
+
+
+@contextlib.contextmanager
+def nccl_collectives(on):
+    """With on=True the sharded path inside the block uses the NCCL collectives instead of symmetric memory."""
+    saved = SymmetricBank.disabled_reason
+    if on:
+        SymmetricBank.disabled_reason = "NCCL collectives forced by scripts/r02_multi.py"
+    try:
+        yield
+    finally:
+        SymmetricBank.disabled_reason = saved
 
 
 def log(msg):
@@ -48,15 +62,11 @@ for n_img, layers, Dp, D in ((13, [(96, 12, 12, True), (96, 12, 12, True)], 256,
     lo, hi = bounds[rank]
     feats, _ = synth.planted_features_device(range(lo, hi), layers, device="cuda")
     allf = synth.planted_features_device(range(n_img), layers, device="cuda")[0] if rank == 0 else None
-    for name, env, prec, taus in (("default (symm)", {}, "f16", [1.0, 2.0]), ("nccl", {"AC_SHARD_TRANSPORT": "nccl"}, "f16", [1.0, 2.0]),
-                                  ("nccl pipeline", {"AC_SHARD_TRANSPORT": "nccl", "AC_SHARD_PIPELINE": "1"}, "f16", [1.0, 2.0]),
-                                  ("all-pairs", {"SYM": "0"}, "f16", [1.0]), ("refined f16r", {}, "auto", [0.1, 1.0])):
-        if name == "nccl pipeline" and world <= 2:
-            continue
-        os.environ["AC_SHARD_PIPELINE"] = env.get("AC_SHARD_PIPELINE", "0")
-        os.environ["AC_SHARD_TRANSPORT"] = env.get("AC_SHARD_TRANSPORT", "symm")
+    for name, prec, taus in (("default (symm)", "f16", [1.0, 2.0]), ("nccl", "f16", [1.0, 2.0]),
+                             ("all-pairs", "f16", [1.0]), ("refined f16r", "auto", [0.1, 1.0])):
         try:
-            a64, X, Dm, w = distributed.run_path_sharded(feats, n_img, 3, 1, Dp, D, taus, precision=prec, symmetric=env.get("SYM") != "0")
+            with nccl_collectives(name == "nccl"):
+                a64, X, Dm, w = distributed.run_path_sharded(feats, n_img, 3, 1, Dp, D, taus, precision=prec, symmetric=name != "all-pairs")
             torch.cuda.synchronize()
             if rank == 0:
                 ref = pipeline.run_path(allf, 3, 1, Dp, D, "unsupervised", taus, precision=prec)
@@ -73,16 +83,11 @@ for n_img, layers, Dp, D in ((13, [(96, 12, 12, True), (96, 12, 12, True)], 256,
             log("check N=%d %s FAILED: %r" % (n_img, name, e))
         dist.barrier()
     del feats, allf
-os.environ["AC_SHARD_PIPELINE"] = "0"
-os.environ["AC_SHARD_TRANSPORT"] = "symm"
 torch.cuda.empty_cache()
 
 
 # ---------------------------------------------------------------- 2. bench lines
-def run_bench(tag, argv, env=None):
-    saved = {k: os.environ.get(k) for k in (env or {})}
-    for k, v in (env or {}).items():
-        os.environ[k] = v
+def run_bench(tag, argv):
     buf = io.StringIO()
     t0 = time.time()
     try:
@@ -90,11 +95,6 @@ def run_bench(tag, argv, env=None):
             bench.main(argv + ["--gpus", str(world)])
     except BaseException as e:  # noqa: BLE001
         log("bench %s FAILED: %r" % (tag, e))
-    for k, v in saved.items():
-        if v is None:
-            os.environ.pop(k, None)
-        else:
-            os.environ[k] = v
     if rank == 0:
         line = [ln for ln in buf.getvalue().splitlines() if ln.startswith("{")]
         with open(os.path.join(OUT, "bench_%s_n%d.json" % (tag.replace(" ", "_"), world)), "w") as f:
@@ -112,14 +112,9 @@ def run_bench(tag, argv, env=None):
     dist.barrier()
 
 
-which = os.environ.get("AC_MULTI_WHICH", "c2,c2nccl,c2r,c3,c4,c4pc,c5,trace").split(",")
+which = os.environ.get("AC_MULTI_WHICH", "c2,c2r,c3,c4,c4pc,c5,trace").split(",")
 if "c2" in which:
     run_bench("config2 default", ["--workload", "config2", "--steps", "20", "--warmup", "5", "--no-cpu-baseline"])
-if "c2nccl" in which:
-    run_bench("config2 nccl", ["--workload", "config2", "--steps", "20", "--warmup", "5", "--no-e2e", "--no-cpu-baseline"], {"AC_SHARD_TRANSPORT": "nccl"})
-if "c2pipe" in which and world > 2:
-    run_bench("config2 nccl pipeline", ["--workload", "config2", "--steps", "20", "--warmup", "5", "--no-e2e", "--no-cpu-baseline"],
-              {"AC_SHARD_TRANSPORT": "nccl", "AC_SHARD_PIPELINE": "1"})
 if "c2r" in which:
     run_bench("config2 f16r", ["--workload", "config2", "--steps", "10", "--warmup", "3", "--no-e2e", "--precision", "f16r"])
 if "c3" in which:
@@ -138,17 +133,17 @@ if "trace" in which:
     layers = [(768, 28, 28, True), (768, 28, 28, True)]
     lo, hi = distributed.shard_bounds(100, world)[rank]
     feats, _ = synth.planted_features_device(range(lo, hi), layers, device="cuda")
-    for name, transport in (("symm", "symm"), ("nccl", "nccl")):
-        os.environ["AC_SHARD_TRANSPORT"] = transport
-        for _ in range(5):
-            distributed.run_path_sharded(feats, 100, 3, 1, 2048, 4096, [1.0], precision="f16", keep_z=False)
-        torch.cuda.synchronize()
-        dist.barrier()
-        with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
-            for _ in range(3):
+    for name in ("symm", "nccl"):
+        with nccl_collectives(name == "nccl"):
+            for _ in range(5):
                 distributed.run_path_sharded(feats, 100, 3, 1, 2048, 4096, [1.0], precision="f16", keep_z=False)
             torch.cuda.synchronize()
-        dist.barrier()
+            dist.barrier()
+            with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
+                for _ in range(3):
+                    distributed.run_path_sharded(feats, 100, 3, 1, 2048, 4096, [1.0], precision="f16", keep_z=False)
+                torch.cuda.synchronize()
+            dist.barrier()
         if rank in (0, world - 1):
             path = os.path.join(OUT, "trace_%s_n%d_rank%d.json" % (name, world, rank))
             prof.export_chrome_trace(path)
@@ -160,7 +155,6 @@ if "trace" in which:
                 for e in gpu:
                     f.write("%10.1f us  +%8.1f us  stream %s  %s\n" % (e["ts"] - t0, e["dur"], e.get("args", {}).get("stream"), e["name"][:110]))
             os.remove(path)
-    os.environ["AC_SHARD_TRANSPORT"] = "symm"
 log("all checks %s" % ("OK" if ok_all else "HAD MISMATCHES"))
 dist.barrier()
 dist.destroy_process_group()

@@ -41,23 +41,6 @@ def test_needed_shards_cover_owned_pairs_only():
             assert max(len(x) for x in need) <= 5      # about half of the 7 other ranks
 
 
-def test_shard_pipeline_steps_pair_up_on_every_rank():
-    """Simulates all ranks of the ring schedule: within each step every send has exactly one matching receive
-    on the destination (an unmatched NCCL send/recv would hang the job), and over all steps a rank receives
-    exactly its needed shards, in ring order."""
-    for n, world in ((100, 8), (1210, 8), (13, 3), (21, 4), (9, 4), (4, 4), (7, 5), (64, 8), (8, 8), (100, 7)):
-        bounds = distributed.shard_bounds(n, world)
-        need = distributed.needed_shards(bounds, n)
-        plans = [distributed.shard_pipeline_plan(need, r, world) for r in range(world)]
-        for k in range(world - 1):
-            sends = {(r, plans[r][k][0]) for r in range(world) if plans[r][k][0] is not None}
-            recvs = {(plans[r][k][1], r) for r in range(world) if plans[r][k][1] is not None}
-            assert sends == recvs, (n, world, k)
-        for r in range(world):
-            got = [p[1] for p in plans[r] if p[1] is not None]
-            assert sorted(got) == sorted(need[r]) and got == [s for s in ((r + k) % world for k in range(1, world)) if s in need[r]]
-
-
 def test_shard_bounds_and_lpt():
     assert distributed.shard_bounds(100, 8) == [(0, 13), (13, 26), (26, 39), (39, 52), (52, 64), (64, 76), (76, 88), (88, 100)]
     assert distributed.shard_bounds(3, 4) == [(0, 1), (1, 2), (2, 3), (3, 3)]
@@ -102,13 +85,20 @@ class _OracleCompute:
     """Stand-in compute for the CPU test (oracle arithmetic on CPU tensors)."""
 
     @staticmethod
-    def embed_images(features, patchsize, stride, Dp, D, precision, want_z=True):
+    def embed_images(features, patchsize, stride, Dp, D, precision, want_z=True, out=None):
+        """`out` = (hi, lo, n2) slices to write the operands into, as pipeline.embed_images takes them."""
         from oracle import restated
 
         Z = restated.embed(features, patchsize, stride, Dp, D)
         n = features[0].shape[0]
         P = Z.shape[0] // n
-        return pipeline.PatchSet(n, P, D, (0, 0), Z=Z, hi=Z.clone(), lo=None, n2=(Z * Z).sum(1))
+        if out is None:
+            return pipeline.PatchSet(n, P, D, (0, 0), Z=Z, hi=Z.clone(), lo=None, n2=(Z * Z).sum(1))
+        hi, lo, n2 = out
+        assert lo is None
+        hi.copy_(Z)
+        n2.copy_((Z * Z).sum(1))
+        return pipeline.PatchSet(n, P, D, (0, 0), Z=Z, hi=hi, lo=None, n2=n2)
 
     @staticmethod
     def min_distance_weights(q, bank, mode, precision, q_self=None):
@@ -125,29 +115,32 @@ class _OracleCompute:
             w[i] = dm[i][:, keep].mean(dim=1)
         return w
 
-    supports_bank_window = True      # exercises the two-phase (local shard first, remote shards after) schedule
-    windows = []                     # bank windows of the min_dist_sym calls, for the schedule assertions
+    launches = []                    # (begin, count, with arrival flags) of the min_dist_sym calls, for the schedule assertions
 
     @staticmethod
-    def min_dist_sym(Qhi, Qlo, Qn2, q_img0, Bhi, Blo, Bn2, nb_img, P, precision, bank_window=None, init=True, out=None):
+    def min_dist_sym(Qhi, Qlo, Qn2, q_img0, Bhi, Blo, Bn2, nb_img, P, precision, bank_window=None, init=True, out=None,
+                     ready=None):
         """What ac_min_dist_sym produces: squared minima only for the pairs the query image owns, restricted
-        to the circular bank-image window; rows of Bhi outside the window are NOT read (they may still be
-        in flight), which the NaN poisoning below enforces."""
+        to the circular bank-image window, written into `out` when it is given.  Only the bank images of owned
+        pairs are read, and with `ready` each of them must be flagged; rows of other bank images may still be in
+        flight or never arrive (NaN in the symmetric-memory test), and the NaN initialisation of rowmin makes
+        an entry the launch should have written but did not fail the comparison."""
         nq = Qhi.shape[0] // P
         begin, count = bank_window if bank_window is not None else (0, nb_img)
-        _OracleCompute.windows.append((int(begin), int(count)))
-        window = [(begin + t) % nb_img for t in range(count)]
+        _OracleCompute.launches.append((int(begin), int(count), ready is not None))
+        if out is None:
+            out = (torch.empty(nb_img, nq * P), torch.empty(nq, nb_img * P))
+        rowmin, colmin = out
         if init:
-            rowmin = torch.full((nb_img, nq * P), float("nan"))
-            colmin = torch.full((nq, nb_img * P), 3.0e38)
-        else:
-            rowmin, colmin = out
-        for j in window:
-            d2 = torch.cdist(Qhi.double(), Bhi[j * P:(j + 1) * P].double()).pow(2).float().reshape(nq, P, P)
+            rowmin.fill_(float("nan"))
+            colmin.fill_(3.0e38)
+        for j in [(begin + t) % nb_img for t in range(count)]:
             for il in range(nq):
                 if distributed.pair_owned(q_img0 + il, j, nb_img):
-                    rowmin[j, il * P:(il + 1) * P] = d2[il].min(dim=1)[0]
-                    colmin[il, j * P:(j + 1) * P] = torch.minimum(colmin[il, j * P:(j + 1) * P], d2[il].min(dim=0)[0])
+                    assert ready is None or int(ready[j]) == 1, "bank image %d read before its arrival flag" % j
+                    d2 = torch.cdist(Qhi[il * P:(il + 1) * P].double(), Bhi[j * P:(j + 1) * P].double()).pow(2).float()
+                    rowmin[j, il * P:(il + 1) * P] = d2.min(dim=1)[0]
+                    colmin[il, j * P:(j + 1) * P] = torch.minimum(colmin[il, j * P:(j + 1) * P], d2.min(dim=0)[0])
         return rowmin, colmin
 
     @staticmethod
@@ -176,13 +169,61 @@ class _OracleCompute:
         return torch.cdist(X.double(), X.double()).float()
 
 
-def _worker(rank, world, port, n_total, tmp):
+class _NoWait:
+    @staticmethod
+    def wait():
+        pass
+
+
+class _FakeSymmetricBank:
+    """CPU stand-in for symm_transport.SymmetricBank over gloo.  The whole-bank buffers start as NaN; publish_and_pull
+    all-gathers the shards but copies in only those listed in need_rank and flags only their images, so a read of a
+    shard the schedule did not ask for fails the comparison."""
+
+    def __init__(self, rows, D, group):
+        self.group = group
+        self.bufs = (torch.full((rows, D), float("nan")), None, torch.full((rows,), float("nan")))
+        self.need_rank = None
+
+    def local_slices(self, row_a, row_b):
+        hi, lo, n2 = self.bufs
+        return hi[row_a:row_b], None, n2[row_a:row_b]
+
+    def publish_and_pull(self, bounds, P, need_rank, rank, world, ready):
+        self.need_rank = list(need_rank)
+        a, b = bounds[rank]
+        counts = [(sb - sa) * P for sa, sb in bounds]
+        for buf in (self.bufs[0], self.bufs[2]):
+            full = distributed.all_gather_rows(buf[a * P:b * P], counts, self.group)
+            for src in need_rank:
+                sa, sb = bounds[src]
+                buf[sa * P:sb * P] = full[sa * P:sb * P]
+        for src in need_rank:
+            ready[bounds[src][0]:bounds[src][1]] = 1
+        return self.bufs, [_NoWait()]
+
+    def colmin_buffer(self, n_local, n_max, cols, dtype):
+        self.colmin = torch.empty(n_local, cols, dtype=dtype)
+        return self.colmin
+
+    def exchange_colmin(self, bounds, P, rank, world):
+        return distributed.exchange_colmin(self.colmin, bounds, P, self.group)
+
+
+def _worker(rank, world, port, n_total, tmp, symm_memory=False):
     sys.path.insert(0, ROOT)
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
     from anomaly_clustering_b200 import synth
 
+    banks = []
+    if symm_memory:     # the symmetric-memory schedule, which the oracle back-end on gloo would otherwise never select
+        def fake_symmetric_bank(compute, rows, D, precision, device, group):
+            banks.append(_FakeSymmetricBank(rows, D, group))
+            return banks[-1]
+
+        distributed._symmetric_bank = fake_symmetric_bank
     feats, _ = synth.planted_features(n_total, [(12, 6, 6, True), (12, 6, 6, True)], seed=3)
     lo, hi = distributed.shard_bounds(n_total, world)[rank]
     if n_total < world:     # empty shards are refused on every rank, before any collective
@@ -196,48 +237,32 @@ def _worker(rank, world, port, n_total, tmp):
     assert torch.equal(allr[:, 0], torch.arange(n_total, dtype=torch.float32))
     a64, X, Dm, w = distributed.run_path_sharded([f[lo:hi] for f in feats], n_total, 3, 1, 32, 64, [1.0, 2.0], precision="f16",
                                                  compute=_OracleCompute, symmetric=True)
-    windows = list(_OracleCompute.windows)
+    launches = list(_OracleCompute.launches)
+    if symm_memory:
+        assert len(banks) == 1 and banks[0].need_rank == distributed.needed_shards(distributed.shard_bounds(n_total, world), n_total)[rank]
     _, _, _, w_full = distributed.run_path_sharded([f[lo:hi] for f in feats], n_total, 3, 1, 32, 64, [1.0], precision="f16",
                                                    compute=_OracleCompute, symmetric=False)
     assert (w - w_full).abs().max().item() <= 1e-4      # symmetric exchange == straightforward all-pairs
     np.savez(os.path.join(tmp, "r%d.npz" % rank), a=a64.numpy(), X=X.numpy(), D=Dm.numpy(), w=w.numpy(),
-             windows=np.asarray(windows, dtype=np.int64).reshape(-1, 2))
+             launches=np.asarray(launches, dtype=np.int64).reshape(-1, 3))
     dist.destroy_process_group()
 
 
-@pytest.mark.timeout(600)
-@pytest.mark.parametrize("n_total,world,two_phase", [(5, 2, True), (5, 2, False), (7, 3, True), (3, 4, True),
-                                                     (7, 3, "pipeline"), (9, 4, "pipeline"), (4, 4, "pipeline")])
-def test_sharded_path_matches_single_process(tmp_path, monkeypatch, n_total, world, two_phase):
-    """Uneven shards (3+2, 3+2+2; 1+1+1+0 has an EMPTY rank and must be refused); with and without the two-phase schedule that
-    multiplies the local shard's pairs while the remote shards are still in flight."""
+def _check_against_single_process(tmp, n_total, world, expected_launches):
+    """Every rank's w, alpha, X and Dmat against the oracle run on all images in one process; each rank's min_dist_sym
+    calls against expected_launches(rank) = [(begin, count, with arrival flags), ...]."""
     from oracle import restated
 
     from anomaly_clustering_b200 import synth
 
-    monkeypatch.setenv("AC_OVERLAP_MIN_WORLD", "2" if two_phase else "99")
-    # "pipeline": shard-granular schedule (one launch per arriving shard; 4 images on 4 ranks = no local pairs at all)
-    monkeypatch.setenv("AC_SHARD_PIPELINE", "1" if two_phase == "pipeline" else "0")
-    port = 29500 + (os.getpid() * 7 + n_total * 13 + world * 101 + len(str(two_phase))) % 2000
-    mp.spawn(_worker, args=(world, port, n_total, str(tmp_path)), nprocs=world, join=True)
     feats, _ = synth.planted_features(n_total, [(12, 6, 6, True), (12, 6, 6, True)], seed=3)
     Z = restated.embed(feats, 3, 1, 32, 64).reshape(n_total, -1, 64)
     w = restated.weight_distance_unsupervised(Z)
     bounds = distributed.shard_bounds(n_total, world)
-    if n_total < world:
-        return
     for r in range(world):
-        g = np.load(os.path.join(str(tmp_path), "r%d.npz" % r))
+        g = np.load(os.path.join(tmp, "r%d.npz" % r))
         lo, hi = bounds[r]
-        wins = [tuple(x) for x in g["windows"]]
-        if two_phase == "pipeline":      # local shard (when it has pairs), then one launch per needed shard in ring order
-            need = distributed.needed_shards(bounds, n_total)[r]
-            ring = [s for s in ((r + k) % world for k in range(1, world)) if s in need]
-            assert wins == ([(lo, hi - lo)] if hi - lo > 1 else []) + [(bounds[s][0], bounds[s][1] - bounds[s][0]) for s in ring]
-        elif two_phase and hi - lo > 1:
-            assert wins == [(lo, hi - lo), (hi % n_total, n_total - (hi - lo))]
-        else:
-            assert wins == [(0, n_total)]
+        assert [tuple(x) for x in g["launches"]] == expected_launches(r)
         assert np.abs(g["w"] - w[lo:hi].numpy()).max() <= 1e-5
         for ti, tau in enumerate([1.0, 2.0]):
             a = restated.alpha_from_weights(w, tau)
@@ -245,6 +270,40 @@ def test_sharded_path_matches_single_process(tmp_path, monkeypatch, n_total, wor
             X = restated.weighted_embedding(a, Z)
             assert np.abs(g["X"][ti] - X).max() <= 1e-5           # every rank holds ALL X rows, in global order
             assert np.abs(g["D"][ti] - restated.pairwise_euclidean(X)).max() <= 1e-4
+
+
+@pytest.mark.timeout(600)
+@pytest.mark.parametrize("n_total,world", [(3, 2), (4, 4), (5, 2), (7, 3), (9, 4), (6, 4), (3, 4)])
+def test_sharded_path_matches_single_process(tmp_path, n_total, world):
+    """NCCL-collective schedule over gloo, uneven shards (2+1, 3+2, 3+2+2, 3+2+2+2, 2+2+1+1; 1+1+1+0 has an EMPTY rank and
+    must be refused).  A rank with more than one image runs the two-phase schedule: the local shard's pairs while the remote
+    shards are still in flight, then the remote bank images.  A rank with one image (rank 1 of (3, 2), every rank of (4, 4),
+    ranks 2 and 3 of (6, 4)) has no pair inside its shard and runs one launch over the whole bank."""
+    port = 29500 + (os.getpid() * 7 + n_total * 13 + world * 101) % 2000
+    mp.spawn(_worker, args=(world, port, n_total, str(tmp_path)), nprocs=world, join=True)
+    if n_total < world:
+        return
+    bounds = distributed.shard_bounds(n_total, world)
+
+    def expected(r):
+        lo, hi = bounds[r]
+        if hi - lo > 1:
+            return [(lo, hi - lo, False), (hi % n_total, n_total - (hi - lo), False)]
+        return [(0, n_total, False)]
+
+    _check_against_single_process(str(tmp_path), n_total, world, expected)
+
+
+@pytest.mark.timeout(600)
+@pytest.mark.parametrize("n_total,world", [(5, 2), (4, 4), (9, 4)])
+def test_symmetric_memory_schedule_matches_single_process(tmp_path, n_total, world):
+    """The symmetric-memory schedule (the default on a multi-GPU node) with a stand-in bank over gloo: the operands are
+    embedded into the bank's slices, only the needed shards are pulled and flagged, ONE distance launch covers the whole
+    bank and reads only flagged bank images, and the column minima come back through the bank's exchange.  The refined
+    modes stay uncovered here: the oracle back-end has no arg-min or refine."""
+    port = 29500 + (os.getpid() * 11 + n_total * 17 + world * 131 + 1000) % 2000
+    mp.spawn(_worker, args=(world, port, n_total, str(tmp_path), True), nprocs=world, join=True)
+    _check_against_single_process(str(tmp_path), n_total, world, lambda r: [(0, n_total, True)])
 
 
 def _worker_supervised(rank, world, port, n_total, n_bank, overlap, tmp):
