@@ -62,6 +62,12 @@ SIGNATURES = {
         [POINTER(AcLayer), c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p, c_int,
          c_void_p, c_void_p, c_size_t, c_void_p],
     ),
+    "ac_embed_workspace_bytes_dt": (c_size_t, [POINTER(AcLayer), c_int, c_int, c_int, c_int, c_int, c_int, c_int]),
+    "ac_embed_dt": (
+        c_int,
+        [POINTER(AcLayer), c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p, c_int,
+         c_void_p, c_void_p, c_size_t, c_void_p],
+    ),
     "ac_patchify": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, POINTER(c_int), c_void_p]),
     "ac_adaptive_pool1d": (c_int, [c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p]),
     "ac_split_operand": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_int, c_void_p]),
@@ -119,6 +125,12 @@ SIGNATURES = {
         c_int,
         [POINTER(AcLayer), c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p, c_size_t,
          c_void_p],
+    ),
+    "ac_weighted_embed_from_features_workspace_bytes_dt": (c_size_t, [POINTER(AcLayer), c_int, c_int, c_int, c_int]),
+    "ac_weighted_embed_from_features_dt": (
+        c_int,
+        [POINTER(AcLayer), c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p,
+         c_size_t, c_void_p],
     ),
     "ac_pairwise_l2": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "ac_copy_blocks": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -30,7 +30,7 @@ static constexpr int kTPT = 2;            // output columns per thread
 static constexpr int kStatSplit = 32;     // partial-sum blocks per (image, layer)
 
 struct LayerDev {
-  const float* ptr;
+  const float* ptr;   // element type of the map (fp32, or fp16 / bf16 in the kernels templated on it); strides in elements
   int C, H, W;
   long long sb, sc, sh, sw;
   int gh, gw;     // unfold grid of this layer
@@ -106,23 +106,47 @@ __host__ __device__ inline void bilinear_src(int dst, int in_size, int out_size,
 }
 
 // ------------------------------------------------------------------------------------------------
+// Feature-map element loads: fp16 / bf16 maps are widened to fp32 at the point of load (exactly), so every kernel computes
+// on a 16-bit map what it computes on that map upcast to fp32.
+__device__ __forceinline__ float op_to_float(float v) { return v; }
+__device__ __forceinline__ float op_to_float(__half v) { return __half2float(v); }
+__device__ __forceinline__ float op_to_float(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <typename T> __device__ __forceinline__ float ld_map(const T* p, long long i) { return op_to_float(__ldg(p + i)); }
+template <typename T> __host__ __device__ __forceinline__ const T* map_ptr(const LayerDev& ly) { return reinterpret_cast<const T*>(ly.ptr); }
+
+// 4 consecutive elements (16 bytes of fp32, 8 bytes of a 16-bit map) from an address aligned to their size
+__device__ __forceinline__ float4 ld4_map(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
+__device__ __forceinline__ float4 ld4_map(const __half* p) {
+  const uint2 u = __ldg(reinterpret_cast<const uint2*>(p));
+  const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&u.x)), b = __half22float2(*reinterpret_cast<const __half2*>(&u.y));
+  return make_float4(a.x, a.y, b.x, b.y);
+}
+__device__ __forceinline__ float4 ld4_map(const __nv_bfloat16* p) {
+  const uint2 u = __ldg(reinterpret_cast<const uint2*>(p));
+  return make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xffff0000u), __uint_as_float(u.y << 16),
+                     __uint_as_float(u.y & 0xffff0000u));
+}
+
+// ------------------------------------------------------------------------------------------------
 // per-(image, layer) sum / sum of squares partials for the whole-map LayerNorm (patchcore.py:384)
+template <typename T>
 __global__ void __launch_bounds__(256) ln_stats_kernel(EmbedParams p, double* stats) {
   const int l = blockIdx.y, b = p.b0 + blockIdx.z;
   const LayerDev ly = p.layers[l];
   const long long n = (long long)ly.C * ly.H * ly.W;
-  const float* base = ly.ptr + (long long)b * ly.sb;
+  const T* base = map_ptr<T>(ly) + (long long)b * ly.sb;
   // dense images (any axis permutation) can be walked flat
   long long lo_e = n * blockIdx.x / gridDim.x, hi_e = n * (blockIdx.x + 1) / gridDim.x;
   float s = 0.f, q = 0.f;
   const bool tok = (ly.sc == 1 && ly.sw == ly.C && ly.sh == (long long)ly.W * ly.C);
   const bool cnn = (ly.sw == 1 && ly.sh == ly.W && ly.sc == (long long)ly.H * ly.W);
-  if ((tok || cnn) && (n % (4LL * gridDim.x) == 0) && ((reinterpret_cast<uintptr_t>(base) & 15) == 0)) {
-    // dense image, 16-byte aligned slices: 128-bit loads, 4 independent accumulator pairs
-    const float4* b4 = reinterpret_cast<const float4*>(base);
+  // the branch depends on the element offset of the image (a multiple of 4), not on the element size, so a 16-bit map and
+  // its fp32 upcast sum in the same order
+  if ((tok || cnn) && (n % (4LL * gridDim.x) == 0) && ((reinterpret_cast<uintptr_t>(base) & (4 * sizeof(T) - 1)) == 0)) {
+    // dense image, aligned slices: 4 elements per load, 4 independent accumulator pairs
     float s2 = 0.f, q2 = 0.f, s3 = 0.f, q3 = 0.f, s4 = 0.f, q4 = 0.f;
     for (long long e = lo_e / 4 + threadIdx.x; e < hi_e / 4; e += blockDim.x) {
-      const float4 v = __ldg(b4 + e);
+      const float4 v = ld4_map(base + 4 * e);
       s += v.x; q = fmaf(v.x, v.x, q);
       s2 += v.y; q2 = fmaf(v.y, v.y, q2);
       s3 += v.z; q3 = fmaf(v.z, v.z, q3);
@@ -132,7 +156,7 @@ __global__ void __launch_bounds__(256) ln_stats_kernel(EmbedParams p, double* st
     q = (q + q2) + (q3 + q4);
   } else if (tok || cnn) {
     for (long long e = lo_e + threadIdx.x; e < hi_e; e += blockDim.x) {
-      const float v = __ldg(base + e);
+      const float v = ld_map(base, e);
       s += v;
       q = fmaf(v, v, q);
     }
@@ -142,7 +166,7 @@ __global__ void __launch_bounds__(256) ln_stats_kernel(EmbedParams p, double* st
       const int c = (int)(e / HW);
       const int r = (int)(e - (long long)c * HW);
       const int y = r / ly.W, x = r - y * ly.W;
-      const float v = __ldg(base + c * ly.sc + y * ly.sh + x * ly.sw);
+      const float v = ld_map(base, c * ly.sc + y * ly.sh + x * ly.sw);
       s += v;
       q = fmaf(v, v, q);
     }
@@ -165,8 +189,6 @@ __global__ void __launch_bounds__(256) ln_stats_kernel(EmbedParams p, double* st
 template <typename T> __device__ __forceinline__ T to_op(float v);
 template <> __device__ __forceinline__ __half to_op<__half>(float v) { return __float2half_rn(v); }
 template <> __device__ __forceinline__ __nv_bfloat16 to_op<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
-__device__ __forceinline__ float op_to_float(__half v) { return __half2float(v); }
-__device__ __forceinline__ float op_to_float(__nv_bfloat16 v) { return __bfloat162float(v); }
 
 __device__ __forceinline__ void store_out(const EmbedParams& p, long long row, int t, float v) {
   const long long idx = row * p.ldz + t;
@@ -793,7 +815,8 @@ static constexpr int kPP = 2;            // periods per thread
 
 __device__ __forceinline__ void consumer_bar_f() { asm volatile("bar.sync 1, %0;" ::"n"(kFT) : "memory"); }
 
-template <int A, int B, int R>
+// T: element type of the feature maps (staged as they are, widened to fp32 when read from the ring)
+template <int A, int B, int R, typename T>
 __global__ void __launch_bounds__(kFT + 32, 3) embed_fused_kernel(const __grid_constant__ FusedParams fp) {
   constexpr int K = 3;
   constexpr int CPP = A / (K * K);
@@ -801,9 +824,9 @@ __global__ void __launch_bounds__(kFT + 32, 3) embed_fused_kernel(const __grid_c
   constexpr int TCH = kPP * CPP;                 // channels per thread
   constexpr int NCH = kFT * TCH;                 // channels per ring row
   const EmbedParams& p = fp.e;
-  extern __shared__ __align__(128) float smem_f[];
-  float* ring = smem_f;                                    // [kRing][K][NCH]
-  float* s_nacc = smem_f + (size_t)kRing * K * NCH;        // [kMaxSeg][kFT] per-thread share of the row norms
+  extern __shared__ __align__(128) unsigned char smem_b[];
+  T* ring = reinterpret_cast<T*>(smem_b);                                               // [kRing][K][NCH]
+  float* s_nacc = reinterpret_cast<float*>(smem_b + (size_t)kRing * K * NCH * sizeof(T));  // [kMaxSeg][kFT] per-thread share of the row norms
   __shared__ __align__(8) uint64_t s_full[kRing], s_empty[kRing];
   __shared__ float s_red[2][kFT / 32];
   __shared__ float s_mu[kMaxLayers], s_rs[kMaxLayers];
@@ -823,7 +846,7 @@ __global__ void __launch_bounds__(kFT + 32, 3) embed_fused_kernel(const __grid_c
   const bool vec8 = (NOUT % 8 == 0) && (((p.ldz | fp.t_stride) & 7) == 0);
   const bool vec4 = (NOUT % 4 == 0) && (((p.ldz | fp.t_stride) & 3) == 0);
   const bool f16 = (p.op_dtype == AC_DT_F16);
-  const float* ring_t = ring + tid * TCH;
+  const T* ring_t = ring + tid * TCH;
 
   for (;;) {
     if (tid == 0) s_item = (long long)atomicAdd(fp.counter, 1u);
@@ -846,8 +869,8 @@ __global__ void __launch_bounds__(kFT + 32, 3) embed_fused_kernel(const __grid_c
             const LayerDev& ly = p.layers[l];
             for (int cx = 0; cx < fp.gx; ++cx) {
               const int c_start = cx * NCH;
-              const uint32_t bytes = (uint32_t)min(NCH, ly.C - c_start) * 4u;
-              const float* src = ly.ptr + (long long)(p.b0 + bA) * ly.sb + c_start + (long long)y * ly.sh + (long long)xa * ly.sw;
+              const uint32_t bytes = (uint32_t)min(NCH, ly.C - c_start) * (uint32_t)sizeof(T);
+              const T* src = map_ptr<T>(ly) + (long long)(p.b0 + bA) * ly.sb + c_start + (long long)y * ly.sh + (long long)xa * ly.sw;
               for (int t = 0; t < nA; ++t) {
                 e_mbar_wait(empty0 + slot * 8, ph ^ 1u);
                 const int ntok = min(K, npos - K * t);
@@ -865,8 +888,8 @@ __global__ void __launch_bounds__(kFT + 32, 3) embed_fused_kernel(const __grid_c
             const LayerDev& ly = p.layers[l];
             for (int cx = 0; cx < fp.gx; ++cx) {
               const int c_start = cx * NCH;
-              const uint32_t bytes = (uint32_t)min(NCH, ly.C - c_start) * 4u;
-              const float* src = ly.ptr + (long long)(p.b0 + bE) * ly.sb + c_start;
+              const uint32_t bytes = (uint32_t)min(NCH, ly.C - c_start) * (uint32_t)sizeof(T);
+              const T* src = map_ptr<T>(ly) + (long long)(p.b0 + bE) * ly.sb + c_start;
               for (int j = 0; j < ncols; ++j) {
                 e_mbar_wait(empty0 + slot * 8, ph ^ 1u);
                 const int ix = xa - p.pad + j;
@@ -906,13 +929,13 @@ __global__ void __launch_bounds__(kFT + 32, 3) embed_fused_kernel(const __grid_c
             for (int t = 0; t < nA; ++t) {
               e_mbar_wait(full0 + slot * 8, ph);
               const int ntok = min(K, npos - K * t);
-              const float* col = ring_t + (size_t)slot * K * NCH;
+              const T* col = ring_t + (size_t)slot * K * NCH;
 #pragma unroll
               for (int ki = 0; ki < K; ++ki)
                 if (ki < ntok) {
 #pragma unroll
                   for (int c = 0; c < TCH; ++c)
-                    if (m0 + c / CPP < fp.nperiods) { const float v = col[ki * NCH + c]; s += v; qq = fmaf(v, v, qq); }
+                    if (m0 + c / CPP < fp.nperiods) { const float v = op_to_float(col[ki * NCH + c]); s += v; qq = fmaf(v, v, qq); }
                 }
               __syncwarp();
               if (lane == 0) e_mbar_arrive(empty0 + slot * 8);
@@ -995,12 +1018,12 @@ __global__ void __launch_bounds__(kFT + 32, 3) embed_fused_kernel(const __grid_c
               const int ix = xa - p.pad + j;
               const bool cin = (ix >= 0) && (ix < ly.W);
               e_mbar_wait(full0 + slot * 8, ph);
-              const float* col = ring_t + (size_t)slot * K * NCH;
+              const T* col = ring_t + (size_t)slot * K * NCH;
 #pragma unroll
               for (int ki = 0; ki < K; ++ki) {
                 if (cin && rowok[ki]) {                      // warp-uniform
 #pragma unroll
-                  for (int c = 0; c < CPP; ++c) v[c][ki][SLOT] = make_float2(col[ki * NCH + c], col[ki * NCH + CPP + c]);
+                  for (int c = 0; c < CPP; ++c) v[c][ki][SLOT] = make_float2(op_to_float(col[ki * NCH + c]), op_to_float(col[ki * NCH + CPP + c]));
                 } else {
 #pragma unroll
                   for (int c = 0; c < CPP; ++c) v[c][ki][SLOT] = mu2;
@@ -1103,16 +1126,43 @@ __global__ void __launch_bounds__(kFT + 32, 3) embed_fused_kernel(const __grid_c
 //   * staged values are read with 32-bit ld.shared straight into the halves of the packed registers (immediate offsets
 //     from one base register per step),
 //   * the output set is a template parameter.
-__device__ __forceinline__ float2 e_lds64(uint32_t addr) {
+// channels (c, c + 1) of a staged row as one float2: one 64-bit load of fp32, one 32-bit load of a 16-bit pair
+__device__ __forceinline__ float2 e_lds_pair(uint32_t addr, float) {
   float2 v;
   asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(addr));
   return v;
 }
+__device__ __forceinline__ uint32_t e_lds_u32(uint32_t addr) {
+  uint32_t v;
+  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(v) : "r"(addr));
+  return v;
+}
+__device__ __forceinline__ float2 e_lds_pair(uint32_t addr, __half) {
+  const uint32_t u = e_lds_u32(addr);
+  return __half22float2(*reinterpret_cast<const __half2*>(&u));
+}
+__device__ __forceinline__ float2 e_lds_pair(uint32_t addr, __nv_bfloat16) {
+  const uint32_t u = e_lds_u32(addr);
+  return make_float2(__uint_as_float(u << 16), __uint_as_float(u & 0xffff0000u));
+}
+// one staged element at an immediate offset, widened to fp32 (bf16: a 16-bit shift, fp16: cvt.f32.f16)
 template <int OFF>
-__device__ __forceinline__ float e_lds32(uint32_t base) {
+__device__ __forceinline__ float e_lds1(uint32_t base, float) {
   float v;
   asm volatile("ld.shared.f32 %0, [%1+%2];" : "=f"(v) : "r"(base), "n"(OFF));
   return v;
+}
+template <int OFF>
+__device__ __forceinline__ float e_lds1(uint32_t base, __half) {
+  unsigned short h;
+  asm volatile("ld.shared.b16 %0, [%1+%2];" : "=h"(h) : "r"(base), "n"(OFF));
+  return __half2float(__ushort_as_half(h));
+}
+template <int OFF>
+__device__ __forceinline__ float e_lds1(uint32_t base, __nv_bfloat16) {
+  unsigned short h;
+  asm volatile("ld.shared.b16 %0, [%1+%2];" : "=h"(h) : "r"(base), "n"(OFF));
+  return __uint_as_float((uint32_t)h << 16);
 }
 __device__ __forceinline__ void e_mbar_wait_spin(uint32_t bar, uint32_t parity) {
   while (!e_mbar_try(bar, parity)) {}
@@ -1146,13 +1196,16 @@ __device__ __forceinline__ float e_sq_acc(__half h, float acc) {
 }
 
 // one staged row of this thread: .x = channel c of its first period, .y = channel c of its second period, which lies
-// HALF floats further (periods tid and tid + FT): far enough apart that ptxas keeps the 32-bit loads apart and lets each
-// land in its half of the packed register pair (adjacent periods became LDS.64 + two moves per pair)
-template <int KI, int NCH_, int HALF>
+// HALF elements further (periods tid and tid + FT): far enough apart that ptxas keeps the 32-bit loads apart and lets each
+// land in its half of the packed register pair (adjacent periods became LDS.64 + two moves per pair).  16-bit maps: the
+// lane stride is 6 bytes, so a warp's 32 loads span 48 words and half the lanes share a bank with another lane's word
+// (2 wavefronts per load instead of 1 for fp32's 12-byte stride)
+template <typename T, int KI, int NCH_, int HALF>
 __device__ __forceinline__ void e_load_row3(uint32_t base, float2& a, float2& b, float2& c) {
-  a = make_float2(e_lds32<(KI * NCH_ + 0) * 4>(base), e_lds32<(KI * NCH_ + HALF + 0) * 4>(base));
-  b = make_float2(e_lds32<(KI * NCH_ + 1) * 4>(base), e_lds32<(KI * NCH_ + HALF + 1) * 4>(base));
-  c = make_float2(e_lds32<(KI * NCH_ + 2) * 4>(base), e_lds32<(KI * NCH_ + HALF + 2) * 4>(base));
+  constexpr int E = (int)sizeof(T);
+  a = make_float2(e_lds1<(KI * NCH_ + 0) * E>(base, T{}), e_lds1<(KI * NCH_ + HALF + 0) * E>(base, T{}));
+  b = make_float2(e_lds1<(KI * NCH_ + 1) * E>(base, T{}), e_lds1<(KI * NCH_ + HALF + 1) * E>(base, T{}));
+  c = make_float2(e_lds1<(KI * NCH_ + 2) * E>(base, T{}), e_lds1<(KI * NCH_ + HALF + 2) * E>(base, T{}));
 }
 
 // "The data is the flag": a partial statistic (sum, sum of squares) and a final (mean, 1/std) travel as ONE 64-bit relaxed
@@ -1196,24 +1249,27 @@ __device__ __forceinline__ void e_prefetch_l2(const void* src, uint32_t bytes) {
   asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
 }
 
-static constexpr int kRingL = 7;         // ring depth of the lean kernel (72 KB of shared memory per CTA at 768 channels, 3 CTAs per SM; a 5-slot ring
+static constexpr int kRingL = 7;         // ring depth of the lean kernel (72 KB of shared memory per CTA at 768 fp32 channels, 3 CTAs per SM; a 5-slot ring
                                          // at 4 CTAs per SM and 96 registers was measured 20 % slower: more images in flight than L2 holds)
 static constexpr int kItemQ = 2;         // items the producer may be ahead of the consumers
 
-template <int A, int B, int R, int FT, bool WZ, int RING, int MINB>
+// T: element type of the feature maps.  The ring stages them as they are (a 16-bit map halves the slot bytes, the L2 -> SM
+// traffic and the shared memory of the ring); every value is widened to fp32 as it is read from the ring.
+template <int A, int B, int R, int FT, bool WZ, int RING, int MINB, typename T>
 __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const __grid_constant__ FusedParams fp) {
   constexpr int K = 3;
   constexpr int CPP = A / (K * K);
   constexpr int NOUT = B / R;
   constexpr int TCH = kPP * CPP;                 // channels per thread (two periods)
   constexpr int NCH = FT * TCH;                  // channels per ring row == C of every layer (host checks)
+  constexpr uint32_t E = (uint32_t)sizeof(T);
   static_assert(NOUT % 8 == 0 || NOUT == 4, "operand rows are written in 16-byte pieces");
   static_assert(TCH % 2 == 0, "the statistics phase reads channel pairs");
   static_assert(CPP == 3, "three channels per period (9C : Dp = 27 : B)");
   const EmbedParams& p = fp.e;
-  extern __shared__ __align__(128) float smem_f[];
-  float* ring = smem_f;                                    // [RING][K][NCH]
-  float* s_nacc = smem_f + (size_t)RING * K * NCH;       // [kMaxSeg][FT] per-thread share of the row norms
+  extern __shared__ __align__(128) unsigned char smem_b[];
+  T* ring = reinterpret_cast<T*>(smem_b);                                                // [RING][K][NCH]
+  float* s_nacc = reinterpret_cast<float*>(smem_b + (size_t)RING * K * NCH * E);        // [kMaxSeg][FT] per-thread share of the row norms
   __shared__ __align__(8) uint64_t s_full[RING], s_empty[RING];
   __shared__ __align__(8) uint64_t s_qfull[kItemQ], s_qempty[kItemQ];
   __shared__ long long s_items[kItemQ];
@@ -1233,10 +1289,10 @@ __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const _
   __syncthreads();
   uint32_t slot = 0, ph = 0;                               // ring position: identical sequence in both roles
   const uint32_t full0 = e_smem_u32(&s_full[0]), empty0 = e_smem_u32(&s_empty[0]);
-  const uint32_t ring_a = e_smem_u32(ring) + (uint32_t)tid * TCH * 4u;      // statistics phase: TCH consecutive channels of a ring row
-  const uint32_t ring_t = e_smem_u32(ring) + (uint32_t)tid * CPP * 4u;      // embed phase: periods tid and tid + FT
-  constexpr uint32_t kSlotBytes = (uint32_t)K * NCH * 4u;
-  constexpr uint32_t kRowBytes = (uint32_t)NCH * 4u;
+  const uint32_t ring_a = e_smem_u32(ring) + (uint32_t)tid * TCH * E;      // statistics phase: TCH consecutive channels of a ring row
+  const uint32_t ring_t = e_smem_u32(ring) + (uint32_t)tid * CPP * E;      // embed phase: periods tid and tid + FT
+  constexpr uint32_t kSlotBytes = (uint32_t)K * NCH * E;
+  constexpr uint32_t kRowBytes = (uint32_t)NCH * E;
 
   // Items are claimed by the PRODUCER, which publishes them through a kItemQ-deep queue and keeps staging: the copies of
   // the next item (its statistics slots come from DRAM) are in flight while the consumers still work on this one.  (With
@@ -1291,6 +1347,7 @@ __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const _
       // select per row.
       const bool hasA = (bA >= 0) && p.layernorm, hasB = (bE >= 0);
       const uint32_t ring_u = e_smem_u32(ring);
+      const T* zrow = reinterpret_cast<const T*>(fp.zero_row);
       if (hasA) {
         // statistics rows of the item just claimed (its first copies wait behind the ring slots of the previous item):
         // DRAM -> L2 ahead of time, so that the statistics slots at the head of the item's in-order ring are L2 hits like
@@ -1298,13 +1355,13 @@ __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const _
         for (int l = 0; l < p.L; ++l) {
           const LayerDev& ly = p.layers[l];
           if (ly.sw == NCH)      // the tokens of a row are contiguous
-            e_prefetch_l2(ly.ptr + (long long)bA * ly.sb + (long long)yA * ly.sh + (long long)xaA * ly.sw, (uint32_t)nposA * kRowBytes);
+            e_prefetch_l2(map_ptr<T>(ly) + (long long)bA * ly.sb + (long long)yA * ly.sh + (long long)xaA * ly.sw, (uint32_t)nposA * kRowBytes);
         }
         for (int l = 0; l < p.L; ++l) {
           const LayerDev& ly = p.layers[l];
           const long long sw = ly.sw;
           const bool contig = (sw == NCH);                   // K tokens = one copy
-          const float* cur = ly.ptr + (long long)bA * ly.sb + (long long)yA * ly.sh + (long long)xaA * sw;
+          const T* cur = map_ptr<T>(ly) + (long long)bA * ly.sb + (long long)yA * ly.sh + (long long)xaA * sw;
           int rem = nposA;                                   // tokens left (>= 1 at every slot)
           for (int t = 0; t < nA; ++t, rem -= K, cur += K * sw) {
             e_mbar_wait_sleep(empty0 + slot * 8, ph ^ 1u);
@@ -1314,7 +1371,7 @@ __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const _
               e_bulk_g2s_hint(dst, cur, kSlotBytes, fb, pol_keep);
             } else {
 #pragma unroll
-              for (int ki = 0; ki < K; ++ki) e_bulk_g2s_hint(dst + ki * kRowBytes, (ki < rem) ? cur + ki * sw : fp.zero_row, kRowBytes, fb, pol_keep);
+              for (int ki = 0; ki < K; ++ki) e_bulk_g2s_hint(dst + ki * kRowBytes, (ki < rem) ? cur + ki * sw : zrow, kRowBytes, fb, pol_keep);
             }
             if (++slot == RING) { slot = 0; ph ^= 1u; }
           }
@@ -1328,20 +1385,20 @@ __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const _
           const LayerDev& ly = p.layers[l];
           const long long sw = ly.sw;
           const bool one = ok0 && ok2 && (sw == NCH);        // the K tokens x-1 .. x+1 of a row: one copy
-          const float* r0 = ly.ptr + (long long)bE * ly.sb + (long long)(ya - 1) * ly.sh + (long long)(x - 1) * sw;
+          const T* r0 = map_ptr<T>(ly) + (long long)bE * ly.sb + (long long)(ya - 1) * ly.sh + (long long)(x - 1) * sw;
           for (int j = 0; j < nrows; ++j, r0 += ly.sh) {
             e_mbar_wait_sleep(empty0 + slot * 8, ph ^ 1u);
             const bool rin = (j != jlo) && (j != jhi);
             const uint32_t fb = full0 + slot * 8, dst = ring_u + slot * kSlotBytes;
             e_mbar_expect_tx(fb, kSlotBytes);
             if (!rin) {
-              e_bulk_g2s_hint(dst, fp.zero_row, kSlotBytes, fb, pol_keep);
+              e_bulk_g2s_hint(dst, zrow, kSlotBytes, fb, pol_keep);
             } else if (one) {
               e_bulk_g2s_hint(dst, r0, kSlotBytes, fb, pol_keep);
             } else {
-              e_bulk_g2s_hint(dst, ok0 ? r0 : fp.zero_row, kRowBytes, fb, pol_keep);
+              e_bulk_g2s_hint(dst, ok0 ? r0 : zrow, kRowBytes, fb, pol_keep);
               e_bulk_g2s_hint(dst + kRowBytes, r0 + sw, kRowBytes, fb, pol_keep);
-              e_bulk_g2s_hint(dst + 2 * kRowBytes, ok2 ? r0 + 2 * sw : fp.zero_row, kRowBytes, fb, pol_keep);
+              e_bulk_g2s_hint(dst + 2 * kRowBytes, ok2 ? r0 + 2 * sw : zrow, kRowBytes, fb, pol_keep);
             }
             if (++slot == RING) { slot = 0; ph ^= 1u; }
           }
@@ -1360,7 +1417,7 @@ __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const _
         for (int ki = 0; ki < K; ++ki)
 #pragma unroll
           for (int c = 0; c < TCH; c += 2) {
-            const float2 v = e_lds64(base + (uint32_t)(ki * NCH + c) * 4u);
+            const float2 v = e_lds_pair(base + (uint32_t)(ki * NCH + c) * E, T{});
             s2 = __fadd2_rn(s2, v);
             q2 = __ffma2_rn(v, v, q2);
           }
@@ -1449,9 +1506,9 @@ __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const _
             e_mbar_wait_spin(full0 + slot * 8, ph);
             const uint32_t base = ring_t + slot * kSlotBytes;
             // the slot holds map row ya - 1 + j: tokens x-1, x, x+1 (kj = 0, 1, 2), NCH channels each
-            e_load_row3<0, NCH, FT * CPP>(base, v[0][SLOT][0], v[1][SLOT][0], v[2][SLOT][0]);
-            e_load_row3<1, NCH, FT * CPP>(base, v[0][SLOT][1], v[1][SLOT][1], v[2][SLOT][1]);
-            e_load_row3<2, NCH, FT * CPP>(base, v[0][SLOT][2], v[1][SLOT][2], v[2][SLOT][2]);
+            e_load_row3<T, 0, NCH, FT * CPP>(base, v[0][SLOT][0], v[1][SLOT][0], v[2][SLOT][0]);
+            e_load_row3<T, 1, NCH, FT * CPP>(base, v[0][SLOT][1], v[1][SLOT][1], v[2][SLOT][1]);
+            e_load_row3<T, 2, NCH, FT * CPP>(base, v[0][SLOT][2], v[1][SLOT][2], v[2][SLOT][2]);
             __syncwarp();
             if (lane == 0) e_mbar_arrive(empty0 + slot * 8);
             if (++slot == RING) { slot = 0; ph ^= 1u; }
@@ -1573,24 +1630,26 @@ __global__ void init_words_kernel(unsigned int* __restrict__ ones, long long n_o
 
 // ------------------------------------------------------------------------------------------------
 // Layout / grid adapters that let every layer take the periodic fast path:
-//  * nchw_to_nhwc_kernel: CNN maps [B,C,H,W] -> channel-contiguous scratch (32x32 smem tile transpose).
+//  * nchw_to_nhwc_kernel: CNN maps [B,C,H,W] -> channel-contiguous fp32 scratch (32x32 smem tile transpose); it reads any
+//    strides and element type, and is also how the per-layer forms take a 16-bit map (exact fp32 copy, same values).
 //  * upsample_store_kernel: a layer whose patch grid differs from layer 0 is pooled at ITS OWN grid into a
 //    small scratch and then resampled; the reference resamples the unfolded planes and pools afterwards
 //    (patchcore.py:398-421), but both maps are linear and act on different axes (positions vs. the flat
 //    patch vector), so they commute -- same bilinear weights (align_corners=False), 1/9 of the gathers.
+template <typename T>
 __global__ void __launch_bounds__(256) nchw_to_nhwc_kernel(LayerDev ly, int b0, float* __restrict__ out) {
   __shared__ float tile[32][33];
   const int b = blockIdx.z;
   const int HW = ly.H * ly.W;
   const int p0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;   // 32 x 8
-  const float* src = ly.ptr + (long long)(b0 + b) * ly.sb;
+  const T* src = map_ptr<T>(ly) + (long long)(b0 + b) * ly.sb;
   for (int r = ty; r < 32; r += 8) {
     const int c = c0 + r, pos = p0 + tx;
     float v = 0.f;
     if (c < ly.C && pos < HW) {
       const int y = pos / ly.W, x = pos - y * ly.W;
-      v = __ldg(src + (long long)c * ly.sc + (long long)y * ly.sh + (long long)x * ly.sw);
+      v = ld_map(src, (long long)c * ly.sc + (long long)y * ly.sh + (long long)x * ly.sw);
     }
     tile[r][tx] = v;
   }
@@ -1651,7 +1710,7 @@ __global__ void __launch_bounds__(256) upsample_store_kernel(EmbedParams p, cons
 //   xpool_kernel : X[i,t] = sum over taps of wt * (sum of partials)
 static constexpr int kXSplit = 4;
 
-template <int K>
+template <int K, typename T>
 __global__ void __launch_bounds__(256) xcorr_kernel(EmbedParams p, int layer, const float* __restrict__ alpha /*[B, P0]*/,
                                                     float* __restrict__ part /*[B, kXSplit, K*K, C]*/) {
   extern __shared__ float s_alpha[];   // (h0 + 2*pad) x (w0 + 2*pad), zero halo
@@ -1679,10 +1738,10 @@ __global__ void __launch_bounds__(256) xcorr_kernel(EmbedParams p, int layer, co
 #pragma unroll
     for (int kj = 0; kj < K; ++kj) acc[ki][kj] = 0.f;
   const int y0 = (int)((long long)ly.H * split / kXSplit), y1 = (int)((long long)ly.H * (split + 1) / kXSplit);
-  const float* src = ly.ptr + (long long)(p.b0 + b) * ly.sb + (long long)c * ly.sc;
+  const T* src = map_ptr<T>(ly) + (long long)(p.b0 + b) * ly.sb + (long long)c * ly.sc;
   for (int iy = y0; iy < y1; ++iy)
     for (int ix = 0; ix < ly.W; ++ix) {
-      const float v = (__ldg(src + (long long)iy * ly.sh + (long long)ix * ly.sw) - mu) * rstd;
+      const float v = (ld_map(src, (long long)iy * ly.sh + (long long)ix * ly.sw) - mu) * rstd;
       // input (iy, ix) is tap (ki, kj) of output position (iy - ki + pad, ix - kj + pad); s_alpha is offset by pad
       const float* a = s_alpha + (iy + 2 * p.pad) * aw + (ix + 2 * p.pad);
 #pragma unroll
@@ -2000,14 +2059,17 @@ static bool periodic_instantiated(const Periodic& pr) {
 
 static int g_embed_variant = 0;   // test hook (ac_debug_set key 2): 0 = auto, 1 = force LDG periodic, 2 = force generic tap kernel, 3 = per-layer TMA launches
 
-static bool tma_aligned(const EmbedParams& p, int l) {
+// bulk copies need 16-byte aligned sources and sizes: rows of C elements of `esize` bytes at 16-byte aligned addresses
+static bool tma_aligned(const EmbedParams& p, int l, int esize) {
   const LayerDev& ly = p.layers[l];
-  if (ly.C % 4 != 0) return false;
+  const int per16 = 16 / esize;   // elements per 16 bytes
+  if (ly.C % per16 != 0) return false;
   if ((reinterpret_cast<uintptr_t>(ly.ptr) & 15) != 0) return false;
-  return (ly.sb % 4 == 0) && (ly.sh % 4 == 0) && (ly.sw % 4 == 0);
+  return (ly.sb % per16 == 0) && (ly.sh % per16 == 0) && (ly.sw % per16 == 0);
 }
 
-static int launch_periodic(EmbedParams p, const Periodic& pr, int l, int num_sms, cudaStream_t st) {
+// aligned: the layer meets the alignment of the TMA-staged kernel (tma_aligned)
+static int launch_periodic(EmbedParams p, const Periodic& pr, int l, bool aligned, int num_sms, cudaStream_t st) {
   // split rows into x segments until the launch has a few waves of CTAs
   const int gx = ceil_div(pr.nperiods, kThreads);
   const long long base_blocks = (long long)gx * p.h0 * p.B;
@@ -2015,7 +2077,7 @@ static int launch_periodic(EmbedParams p, const Periodic& pr, int l, int num_sms
   p.xseg_len = ceil_div(p.w0, nxseg);
   p.nxseg = ceil_div(p.w0, p.xseg_len);
   dim3 grid(gx, p.h0 * p.nxseg, p.B);
-  const bool use_tma = (g_embed_variant == 0 || g_embed_variant == 3) && tma_aligned(p, l);
+  const bool use_tma = (g_embed_variant == 0 || g_embed_variant == 3) && aligned;
 #define X(a, b, r)                                                                                         \
   if (pr.A == a && pr.B == b && pr.R == r) {                                                               \
     if (use_tma) {                                                                                         \
@@ -2038,10 +2100,10 @@ static int launch_periodic(EmbedParams p, const Periodic& pr, int l, int num_sms
 static constexpr int kLookAhead = 2;   // images the statistics run ahead of the embedding
 static constexpr int kCtasPerSm = 3;   // persistent CTAs per SM (the lean kernel: at most its MINB)
 
-static bool fused_eligible(const Plan& plan, const EmbedParams& p, const Periodic* pr, int L) {
+static bool fused_eligible(const Plan& plan, const EmbedParams& p, const Periodic* pr, int L, int esize) {
   if (g_embed_variant != 0 || !plan.fused || p.k != 3 || p.s != 1) return false;
   for (int l = 0; l < L; ++l) {
-    if (plan.pl[l].nchunks == 0 || !tma_aligned(p, l)) return false;
+    if (plan.pl[l].nchunks == 0 || !tma_aligned(p, l, esize)) return false;
     if (!pr[l].ok || !periodic_instantiated(pr[l]) || pr[l].transpose || pr[l].upsample) return false;
     if (pr[l].A != pr[0].A || pr[l].B != pr[0].B || pr[l].R != pr[0].R) return false;
     if (p.layers[l].C != p.layers[0].C || p.layers[l].H != p.layers[0].H || p.layers[l].W != p.layers[0].W) return false;
@@ -2050,7 +2112,7 @@ static bool fused_eligible(const Plan& plan, const EmbedParams& p, const Periodi
   return true;
 }
 
-static constexpr size_t kZeroRowBytes = 12288;  // lean kernel: zeros that stand in for taps outside the map (one ring slot: 3 tokens x <= 768 channels)
+static constexpr size_t kZeroRowBytes = 12288;  // lean kernel: zeros that stand in for taps outside the map (one ring slot: 3 tokens x <= 768 fp32 channels)
 
 static constexpr int kMinSeg = 4;   // the workspace sizes the lean kernel's statistics slots for x segments this short
 
@@ -2069,6 +2131,7 @@ static size_t fused_ws_bytes(int L, int B, int h0, int w0) {
 
 static int g_fused_lean = 1;      // test hook (ac_debug_set key 9): 0 = always the general fused kernel
 
+template <typename T>
 static int launch_fused(EmbedParams p, const Periodic& pr, float* n2, void* ws, int num_sms, cudaStream_t st) {
   FusedParams fp;
   memset(&fp, 0, sizeof(fp));
@@ -2103,9 +2166,9 @@ static int launch_fused(EmbedParams p, const Periodic& pr, float* n2, void* ws, 
   AC_LAUNCH_CHECK();
 #define XLK(b, ft, wz, ring, minb)                                                                                    \
   {                                                                                                                   \
-    const size_t smem = ((size_t)ring * 3 * ft * kPP * 3 + (size_t)kMaxSeg * ft) * sizeof(float);                     \
+    const size_t smem = (size_t)ring * 3 * ft * kPP * 3 * sizeof(T) + (size_t)kMaxSeg * ft * sizeof(float);           \
     const int grid_l = (int)std::min<long long>(fp.n_items, (long long)num_sms * std::min(kCtasPerSm, minb));         \
-    auto kern = embed_fused_fast_kernel<27, b, 1, ft, wz, ring, minb>;                                                \
+    auto kern = embed_fused_fast_kernel<27, b, 1, ft, wz, ring, minb, T>;                                             \
     AC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                      \
     kern<<<grid_l, ft + 32, smem, st>>>(fp);                                                                          \
     AC_LAUNCH_CHECK();                                                                                                \
@@ -2121,8 +2184,8 @@ static int launch_fused(EmbedParams p, const Periodic& pr, float* n2, void* ws, 
   const int grid = (int)std::min<long long>(fp.n_items, (long long)num_sms * kCtasPerSm);
 #define X(a, b, r)                                                                                                   \
   if (pr.A == a && pr.B == b && pr.R == r) {                                                                         \
-    auto kern = embed_fused_kernel<a, b, r>;                                                                         \
-    const size_t smem = ((size_t)kRing * 3 * kFT * kPP * (a / 9) + (size_t)kMaxSeg * kFT) * sizeof(float);           \
+    auto kern = embed_fused_kernel<a, b, r, T>;                                                                      \
+    const size_t smem = (size_t)kRing * 3 * kFT * kPP * (a / 9) * sizeof(T) + (size_t)kMaxSeg * kFT * sizeof(float); \
     AC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                     \
     kern<<<grid, kFT + 32, smem, st>>>(fp);                                                                          \
     AC_LAUNCH_CHECK();                                                                                               \
@@ -2169,6 +2232,16 @@ static int get_plan(const ac_layer_t* layers, int L, int k, int s, int Dp, int D
   return AC_OK;
 }
 
+// calls f(T{}) with T the element type of feature-map dtype dt (callers validate dt)
+template <typename F>
+static int with_feat_type(int dt, F&& f) {
+  if (dt == AC_DT_F16) return f(__half{});
+  if (dt == AC_DT_BF16) return f(__nv_bfloat16{});
+  return f(float{});
+}
+static bool feat_dtype_ok(int dt) { return dt == AC_DT_F32 || dt == AC_DT_F16 || dt == AC_DT_BF16; }
+static int feat_esize(int dt) { return dt == AC_DT_F32 ? 4 : 2; }
+
 }  // namespace ac
 
 using namespace ac;
@@ -2200,8 +2273,10 @@ static size_t adapter_bytes(const ac_layer_t* layers, int L, int B, int k, int s
   return total;
 }
 
-extern "C" size_t ac_embed_workspace_bytes(const ac_layer_t* layers, int L, int B, int patchsize, int stride, int Dp, int D) {
+extern "C" size_t ac_embed_workspace_bytes_dt(const ac_layer_t* layers, int L, int feat_dtype, int B, int patchsize, int stride,
+                                              int Dp, int D) {
   if (!layers || L < 1 || L > kMaxLayers || B < 1 || patchsize < 1 || stride < 1 || Dp < 1 || D < 1) return 0;
+  if (!feat_dtype_ok(feat_dtype)) return 0;
   const int pad = (patchsize - 1) / 2;
   const long long P = (long long)((layers[0].H + 2 * pad - (patchsize - 1) - 1) / stride + 1) *
                       ((layers[0].W + 2 * pad - (patchsize - 1) - 1) / stride + 1);
@@ -2210,8 +2285,9 @@ extern "C" size_t ac_embed_workspace_bytes(const ac_layer_t* layers, int L, int 
   size_t chunks = align256(((size_t)L * Dp / 32 + (size_t)D / 32 + 2 * L + 16) * sizeof(ChunkDesc));
   // the [B*P, L*Dp] concat scratch exists only when an Aggregator window straddles two layers
   size_t concat = aggregator_fusable(L, Dp, D) ? 0 : align256((size_t)B * P * (size_t)L * Dp * sizeof(float));
-  // channel-contiguous copies of CNN-layout maps + coarse pooled tiles of resampled layers (fast path)
-  bool any_adapter = false;
+  // channel-contiguous copies of CNN-layout maps + coarse pooled tiles of resampled layers (fast path); the per-layer forms
+  // read a 16-bit map through the same fp32 channel-contiguous copy
+  bool any_adapter = (feat_dtype != AC_DT_F32);
   for (int l = 0; l < L; ++l) {
     const int gh = (layers[l].H + 2 * pad - (patchsize - 1) - 1) / stride + 1, gw = (layers[l].W + 2 * pad - (patchsize - 1) - 1) / stride + 1;
     if (layers[l].sc != 1 || (long long)gh * gw != P) any_adapter = true;
@@ -2222,10 +2298,15 @@ extern "C" size_t ac_embed_workspace_bytes(const ac_layer_t* layers, int L, int 
   return stats + chunks + concat + adapters + fused_ws_bytes(L, B, gh0, gw0) + 256;
 }
 
-extern "C" int ac_embed_ex(const ac_layer_t* layers, int L, int B, int patchsize, int stride, int Dp, int D, int layernorm,
-                           float eps, float* Z, void* Zhi, void* Zlo, int op_dtype, float* n2, void* ws, size_t ws_bytes,
-                           ac_stream_t stream) {
+extern "C" size_t ac_embed_workspace_bytes(const ac_layer_t* layers, int L, int B, int patchsize, int stride, int Dp, int D) {
+  return ac_embed_workspace_bytes_dt(layers, L, AC_DT_F32, B, patchsize, stride, Dp, D);
+}
+
+extern "C" int ac_embed_dt(const ac_layer_t* layers, int L, int feat_dtype, int B, int patchsize, int stride, int Dp, int D,
+                           int layernorm, float eps, float* Z, void* Zhi, void* Zlo, int op_dtype, float* n2, void* ws,
+                           size_t ws_bytes, ac_stream_t stream) {
   if (!layers || !ws) return AC_ERR_INVALID;
+  if (!feat_dtype_ok(feat_dtype)) return AC_ERR_INVALID;
   if (!Z && !Zhi) return AC_ERR_INVALID;
   if (n2 && !Zhi) return AC_ERR_INVALID;
   if (Zhi && op_dtype != AC_DT_F16 && op_dtype != AC_DT_BF16) return AC_ERR_INVALID;
@@ -2259,6 +2340,8 @@ extern "C" int ac_embed_ex(const ac_layer_t* layers, int L, int B, int patchsize
   ChunkDesc* dchunks = (ChunkDesc*)(w8 + stats_b);
   float* dconcat = (float*)(w8 + stats_b + chunks_b);
 
+  const bool f32 = (feat_dtype == AC_DT_F32);
+  const int esize = feat_esize(feat_dtype);
   Periodic pr[kMaxLayers];
   bool need_chunks = false, any_adapter = false;
   for (int l = 0; l < L; ++l) {
@@ -2266,6 +2349,7 @@ extern "C" int ac_embed_ex(const ac_layer_t* layers, int L, int B, int patchsize
     if (pr[l].ok && (!periodic_instantiated(pr[l]) || g_embed_variant == 2)) pr[l].ok = 0;
     if (!pr[l].ok && plan.pl[l].nchunks > 0) need_chunks = true;
     if (pr[l].ok && (pr[l].transpose || pr[l].upsample)) any_adapter = true;
+    if (!f32 && plan.pl[l].nchunks > 0) any_adapter = true;   // per-layer forms read 16-bit maps through an fp32 copy
   }
   // scratch of the layout / grid adapters (only carved when a fast-path layer needs one)
   size_t tb[kMaxLayers], cb[kMaxLayers];
@@ -2294,11 +2378,12 @@ extern "C" int ac_embed_ex(const ac_layer_t* layers, int L, int B, int patchsize
   AC_CUDA(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
 
   // Single-pass fused form (one persistent launch: statistics, every layer, operand norms) when the shape allows it
-  if (fused_eligible(plan, p, pr, L)) {
+  if (fused_eligible(plan, p, pr, L, esize)) {
     const size_t fb = fused_ws_bytes(L, B, p.h0, p.w0) + 256;
     if (fb > ws_bytes || (reinterpret_cast<uintptr_t>(ws) & 15) != 0) return AC_ERR_WORKSPACE;
     p.B = B;
-    return launch_fused(p, pr[0], n2, w8 + ((ws_bytes - fb) & ~(size_t)255), num_sms, st);
+    void* fws = w8 + ((ws_bytes - fb) & ~(size_t)255);
+    return with_feat_type(feat_dtype, [&](auto tag) { return launch_fused<decltype(tag)>(p, pr[0], n2, fws, num_sms, st); });
   }
 
   // One statistics launch and one embed launch per layer for the whole batch.  Measured on B200:
@@ -2309,26 +2394,39 @@ extern "C" int ac_embed_ex(const ac_layer_t* layers, int L, int B, int patchsize
     p.b0 = b0;
     p.B = std::min(nb, B - b0);
     if (layernorm) {
-      ln_stats_kernel<<<dim3(kStatSplit, L, p.B), 256, 0, st>>>(p, dstats);
-      AC_LAUNCH_CHECK();
+      // the statistics always come from the map as given (its own element type and layout: same summation order)
+      rc = with_feat_type(feat_dtype, [&](auto tag) {
+        ln_stats_kernel<decltype(tag)><<<dim3(kStatSplit, L, p.B), 256, 0, st>>>(p, dstats);
+        AC_LAUNCH_CHECK();
+        return AC_OK;
+      });
+      if (rc) return rc;
     }
     for (int l = 0; l < L; ++l) {
       if (plan.pl[l].nchunks == 0) continue;
-      if (!pr[l].ok) {
-        rc = p.layers[l].resample ? dispatch_taps<true>(p, plan, l, dchunks, st) : dispatch_taps<false>(p, plan, l, dchunks, st);
-        if (rc) return rc;
-        continue;
-      }
       EmbedParams q = p;
       Periodic prl = pr[l];
       LayerDev& ly = q.layers[l];
-      if (prl.transpose) {
-        // CNN layout -> channel-contiguous scratch [B, H*W, C]
+      // the TMA form takes a layer where the map as given meets its alignment (a CNN layout: where its fp32 copy does)
+      const bool transpose = prl.ok && prl.transpose;
+      const bool aligned = transpose || tma_aligned(p, l, esize);
+      if (transpose || !f32) {
+        // CNN layout or 16-bit map -> fp32 channel-contiguous scratch [B, H*W, C] (exact values; the per-layer forms compute
+        // the same bits on it as on the map itself)
         dim3 tg(ceil_div(ly.H * ly.W, 32), ceil_div(ly.C, 32), q.B);
-        nchw_to_nhwc_kernel<<<tg, 256, 0, st>>>(p.layers[l], q.b0, tbuf[l]);
-        AC_LAUNCH_CHECK();
+        rc = with_feat_type(feat_dtype, [&](auto tag) {
+          nchw_to_nhwc_kernel<decltype(tag)><<<tg, 256, 0, st>>>(p.layers[l], q.b0, tbuf[l]);
+          AC_LAUNCH_CHECK();
+          return AC_OK;
+        });
+        if (rc) return rc;
         ly.ptr = tbuf[l] - (long long)q.b0 * ly.C * ly.H * ly.W;   // kernels index images as b0 + blockIdx.z
         ly.sb = (long long)ly.C * ly.H * ly.W; ly.sc = 1; ly.sh = (long long)ly.W * ly.C; ly.sw = ly.C;
+      }
+      if (!prl.ok) {
+        rc = ly.resample ? dispatch_taps<true>(q, plan, l, dchunks, st) : dispatch_taps<false>(q, plan, l, dchunks, st);
+        if (rc) return rc;
+        continue;
       }
       if (prl.upsample) {
         // pool at the layer's own patch grid into scratch [B, gh*gw, ncols], resample afterwards
@@ -2337,7 +2435,7 @@ extern "C" int ac_embed_ex(const ac_layer_t* layers, int L, int B, int patchsize
         q.Zhi = nullptr; q.Zlo = nullptr; q.op_dtype = 0; q.ldz = prl.ncols;
         prl.t_base = 0;
       }
-      rc = launch_periodic(q, prl, l, num_sms, st);
+      rc = launch_periodic(q, prl, l, aligned && tma_aligned(q, l, 4), num_sms, st);
       if (rc) return rc;
       if (prl.upsample) {
         const long long groups = (long long)p.B * p.h0 * p.w0 * ((prl.ncols + 3) / 4);
@@ -2365,10 +2463,17 @@ extern "C" int ac_embed_ex(const ac_layer_t* layers, int L, int B, int patchsize
   return AC_OK;
 }
 
+extern "C" int ac_embed_ex(const ac_layer_t* layers, int L, int B, int patchsize, int stride, int Dp, int D, int layernorm,
+                           float eps, float* Z, void* Zhi, void* Zlo, int op_dtype, float* n2, void* ws, size_t ws_bytes,
+                           ac_stream_t stream) {
+  return ac_embed_dt(layers, L, AC_DT_F32, B, patchsize, stride, Dp, D, layernorm, eps, Z, Zhi, Zlo, op_dtype, n2, ws, ws_bytes, stream);
+}
+
 extern "C" int ac_embed(const ac_layer_t* layers, int L, int B, int patchsize, int stride, int Dp, int D, int layernorm,
                         float eps, float* Z, void* Zhi, void* Zlo, int op_dtype, void* ws, size_t ws_bytes,
                         ac_stream_t stream) {
-  return ac_embed_ex(layers, L, B, patchsize, stride, Dp, D, layernorm, eps, Z, Zhi, Zlo, op_dtype, nullptr, ws, ws_bytes, stream);
+  return ac_embed_dt(layers, L, AC_DT_F32, B, patchsize, stride, Dp, D, layernorm, eps, Z, Zhi, Zlo, op_dtype, nullptr, ws, ws_bytes,
+                     stream);
 }
 
 // test hook (not part of the public header): forces the embedding paths the library otherwise picks from the input.
@@ -2380,18 +2485,23 @@ extern "C" int ac_debug_set(int key, int value) {
   return AC_ERR_INVALID;
 }
 
-extern "C" size_t ac_weighted_embed_from_features_workspace_bytes(const ac_layer_t* layers, int L, int B, int patchsize) {
-  if (!layers || L < 1 || L > kMaxLayers || B < 1 || patchsize < 1) return 0;
+extern "C" size_t ac_weighted_embed_from_features_workspace_bytes_dt(const ac_layer_t* layers, int L, int feat_dtype, int B,
+                                                                     int patchsize) {
+  if (!layers || L < 1 || L > kMaxLayers || B < 1 || patchsize < 1 || !feat_dtype_ok(feat_dtype)) return 0;
   size_t stats = align256((size_t)B * L * kStatSplit * 2 * sizeof(double));
   size_t part = 0;
   for (int l = 0; l < L; ++l) part = std::max(part, align256((size_t)B * kXSplit * patchsize * patchsize * layers[l].C * sizeof(float)));
   return stats + part;
 }
 
-extern "C" int ac_weighted_embed_from_features(const ac_layer_t* layers, int L, int B, int patchsize, int stride, int Dp, int D,
-                                               int layernorm, float eps, const float* alpha, float* X, void* ws, size_t ws_bytes,
-                                               ac_stream_t stream) {
-  if (!layers || !alpha || !X || !ws || B < 1) return AC_ERR_INVALID;
+extern "C" size_t ac_weighted_embed_from_features_workspace_bytes(const ac_layer_t* layers, int L, int B, int patchsize) {
+  return ac_weighted_embed_from_features_workspace_bytes_dt(layers, L, AC_DT_F32, B, patchsize);
+}
+
+extern "C" int ac_weighted_embed_from_features_dt(const ac_layer_t* layers, int L, int feat_dtype, int B, int patchsize, int stride,
+                                                  int Dp, int D, int layernorm, float eps, const float* alpha, float* X, void* ws,
+                                                  size_t ws_bytes, ac_stream_t stream) {
+  if (!layers || !alpha || !X || !ws || B < 1 || !feat_dtype_ok(feat_dtype)) return AC_ERR_INVALID;
   int rc = check_device();
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
@@ -2408,7 +2518,7 @@ extern "C" int ac_weighted_embed_from_features(const ac_layer_t* layers, int L, 
     p.layers[l].ptr = layers[l].ptr;
     p.layers[l].sb = layers[l].sb;
   }
-  const size_t need = ac_weighted_embed_from_features_workspace_bytes(layers, L, B, patchsize);
+  const size_t need = ac_weighted_embed_from_features_workspace_bytes_dt(layers, L, feat_dtype, B, patchsize);
   if (ws_bytes < need) return AC_ERR_WORKSPACE;
   const size_t stats_b = align256((size_t)B * L * kStatSplit * 2 * sizeof(double));
   double* dstats = (double*)ws;
@@ -2417,27 +2527,37 @@ extern "C" int ac_weighted_embed_from_features(const ac_layer_t* layers, int L, 
   const int nb = std::min(B, 65535);
   const size_t smem = (size_t)(p.h0 + 2 * p.pad) * (p.w0 + 2 * p.pad) * sizeof(float);
   if (smem > 200 * 1024) return AC_ERR_UNSUPPORTED;
-  if (smem > 48 * 1024) AC_CUDA(cudaFuncSetAttribute(xcorr_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  for (int b0 = 0; b0 < B; b0 += nb) {
-    p.b0 = b0;
-    p.B = std::min(nb, B - b0);
-    if (layernorm) {
-      ln_stats_kernel<<<dim3(kStatSplit, L, p.B), 256, 0, st>>>(p, dstats);
-      AC_LAUNCH_CHECK();
+  return with_feat_type(feat_dtype, [&](auto tag) {
+    using T = decltype(tag);
+    if (smem > 48 * 1024) AC_CUDA(cudaFuncSetAttribute(xcorr_kernel<3, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    for (int b0 = 0; b0 < B; b0 += nb) {
+      p.b0 = b0;
+      p.B = std::min(nb, B - b0);
+      if (layernorm) {
+        ln_stats_kernel<T><<<dim3(kStatSplit, L, p.B), 256, 0, st>>>(p, dstats);
+        AC_LAUNCH_CHECK();
+      }
+      for (int l = 0; l < L; ++l) {
+        // output columns owned by layer l (fused Aggregator: contiguous range)
+        int ta = -1, tb = -1;
+        for (int t = 0; t < p.agg_out; ++t)
+          if (pool_start(t, p.agg_in, p.agg_out) / Dp == l) { if (ta < 0) ta = t; tb = t + 1; }
+        if (ta < 0) continue;
+        xcorr_kernel<3, T><<<dim3(ceil_div(p.layers[l].C, 256), kXSplit, p.B), 256, smem, st>>>(p, l, alpha + (long long)b0 * p.h0 * p.w0, part);
+        AC_LAUNCH_CHECK();
+        xpool_kernel<<<dim3(ceil_div(tb - ta, 256), p.B), 256, 0, st>>>(p, l, ta, tb, part, X);
+        AC_LAUNCH_CHECK();
+      }
     }
-    for (int l = 0; l < L; ++l) {
-      // output columns owned by layer l (fused Aggregator: contiguous range)
-      int ta = -1, tb = -1;
-      for (int t = 0; t < p.agg_out; ++t)
-        if (pool_start(t, p.agg_in, p.agg_out) / Dp == l) { if (ta < 0) ta = t; tb = t + 1; }
-      if (ta < 0) continue;
-      xcorr_kernel<3><<<dim3(ceil_div(p.layers[l].C, 256), kXSplit, p.B), 256, smem, st>>>(p, l, alpha + (long long)b0 * p.h0 * p.w0, part);
-      AC_LAUNCH_CHECK();
-      xpool_kernel<<<dim3(ceil_div(tb - ta, 256), p.B), 256, 0, st>>>(p, l, ta, tb, part, X);
-      AC_LAUNCH_CHECK();
-    }
-  }
-  return AC_OK;
+    return AC_OK;
+  });
+}
+
+extern "C" int ac_weighted_embed_from_features(const ac_layer_t* layers, int L, int B, int patchsize, int stride, int Dp, int D,
+                                               int layernorm, float eps, const float* alpha, float* X, void* ws, size_t ws_bytes,
+                                               ac_stream_t stream) {
+  return ac_weighted_embed_from_features_dt(layers, L, AC_DT_F32, B, patchsize, stride, Dp, D, layernorm, eps, alpha, X, ws, ws_bytes,
+                                            stream);
 }
 
 extern "C" int ac_patchify(const float* x, int B, int C, int H, int W, int patchsize, int stride, float* out,

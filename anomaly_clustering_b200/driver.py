@@ -14,6 +14,8 @@ import torch
 from . import io, pipeline
 from .patchcore.patchcore import AnomalyClusteringCore
 
+_HALF_MAPS = (torch.float16, torch.bfloat16)   # feature-map dtypes the embed kernels read natively besides float32
+
 
 def _images(loader: Iterable) -> torch.Tensor:
     """Concatenates the 'image' entries of a reference-style loader (dicts or tensors)."""
@@ -53,6 +55,7 @@ def make_category_data(
     info_root: Optional[str] = None,
     keep_weights: bool = False,
     allow_random_init: bool = False,
+    backbone_dtype: Optional[torch.dtype] = None,
 ):
     """Returns (matrix_alpha [N,1,P] f32 device tensor, X [N,D] f32 ndarray) for a scalar tau, a list of
     such tuples for a list of taus, and writes the reference's pickle(s) when `save_path` is given.
@@ -61,7 +64,12 @@ def make_category_data(
     tau-independent weights next to the pickles so a later tau sweep can skip the distance pass.
     `backbone` (a torch module with the reference's pretrained weights loaded) is REQUIRED: the offline stand-ins of
     `backbones.load` are random-init and would silently write meaningless results under the reference's file names.
-    `allow_random_init=True` permits them for shape / smoke runs (the CLI then tags the backbone directory `-randinit`)."""
+    `allow_random_init=True` permits them for shape / smoke runs (the CLI then tags the backbone directory `-randinit`).
+    `backbone_dtype` torch.bfloat16 / torch.float16 casts the backbone module (in place) and the images to that dtype; its
+    16-bit feature maps go to the embed kernels as they are (the result equals the fp32 embedding of those maps upcast).
+    None keeps the backbone in float32."""
+    if backbone_dtype not in (None, torch.float32, torch.bfloat16, torch.float16):
+        raise ValueError("backbone_dtype must be None, torch.float32, torch.bfloat16 or torch.float16, got %s" % (backbone_dtype,))
     if test_dataloader is None:
         raise ValueError("inject test_dataloader: the MVTec walker (datasets/mvtec.py) is out of scope and `path` is not read")
     device = device or torch.device("cuda", torch.cuda.current_device())
@@ -75,6 +83,9 @@ def make_category_data(
     elif getattr(backbone, "random_init", False) and not allow_random_init:
         raise ValueError("the injected backbone is a RANDOM-INIT stand-in (backbones.load); pass allow_random_init=True for a shape / "
                          "smoke run, or a module with the pretrained weights loaded")
+    image_dtype = torch.float if backbone_dtype is None else backbone_dtype
+    if backbone_dtype is not None:
+        backbone = backbone.to(backbone_dtype)
     core = AnomalyClusteringCore(device).load(
         backbone=backbone, layers_to_extract_from=layers_to_extract_from, device=device, input_shape=input_shape,
         pretrain_embed_dimension=pretrain_embed_dimension, target_embed_dimension=target_embed_dimension, patchsize=patchsize,
@@ -88,7 +99,8 @@ def make_category_data(
         ims = _images(loader)
         sets = []
         for b0 in range(0, len(ims), batch_size):
-            feats = [f.float() for f in core._features(ims[b0:b0 + batch_size].to(torch.float).to(device))]
+            feats = [f if f.dtype in _HALF_MAPS else f.float()
+                     for f in core._features(ims[b0:b0 + batch_size].to(image_dtype).to(device))]
             sets.append(pipeline.embed_images(feats, patchsize, 1, pretrain_embed_dimension, target_embed_dimension, precision,
                                               want_z=want_z))
         cat = lambda xs: None if xs[0] is None else torch.cat(xs, dim=0)  # noqa: E731

@@ -53,6 +53,17 @@ def write_cli_csv(save_path, layers, pretrain_dim, target_dim, supervised, taus,
     return io.write_result_csv(io.result_csv_path(save_path, layers, pretrain_dim, target_dim), supervised, blocks)
 
 
+# --backbone_dtype: None keeps the fp32 backbone; a 16-bit run tags its backbone directory
+BACKBONE_DTYPES = {"float32": None, "bfloat16": torch.bfloat16, "float16": torch.float16}
+_DTYPE_TAGS = {"float32": "", "bfloat16": "-bf16", "float16": "-fp16"}
+
+
+def backbone_dir_name(backbone: str, random_init: bool, backbone_dtype: str = "float32") -> str:
+    """Output directory of a backbone.  A random-init or 16-bit run is tagged, so it never writes under the reference's own
+    directory name."""
+    return backbone + ("-randinit" if random_init else "") + _DTYPE_TAGS[backbone_dtype]
+
+
 def _device() -> torch.device:
     return torch.device("cuda", torch.cuda.current_device())
 
@@ -74,6 +85,8 @@ def main(argv=None):
     parser.add_argument("--synthetic_images", type=int, default=20)
     parser.add_argument("--synthetic_classes", type=int, default=4)
     parser.add_argument("--categories", nargs="+", default=["bottle"])
+    parser.add_argument("--backbone_dtype", default="float32", choices=sorted(BACKBONE_DTYPES),
+                        help="Run the backbone in this dtype; 16-bit feature maps go to the embed kernels as they are.")
     args = parser.parse_args(argv)
     print("\n".join("%s: %s" % (k, str(v)) for k, v in sorted(dict(vars(args)).items())))
     if args.dataset != "synthetic":
@@ -82,7 +95,7 @@ def main(argv=None):
     device = _device()
     # --dataset synthetic is a shape / smoke run by construction: random-init network, said loudly, tagged output directory
     net = backbones.load(args.backbone_names[0], allow_random_init=True)
-    backbone_dir = args.backbone_names[0] + ("-randinit" if getattr(net, "random_init", True) else "")   # never the reference's own name
+    backbone_dir = backbone_dir_name(args.backbone_names[0], getattr(net, "random_init", True), args.backbone_dtype)
     save_path = os.path.join(args.output_dir, args.dataset, backbone_dir, args.supervised)
     os.makedirs(save_path, exist_ok=True)
     rows = []
@@ -96,7 +109,8 @@ def main(argv=None):
                                         train_ratio=args.train_ratio, tau=list(args.tau), supervised=args.supervised,
                                         dataset=args.dataset, test_dataloader=loader, train_dataloader=train, backbone=net,
                                         device=device, precision=args.precision,
-                                        info_root=args.output_dir, allow_random_init=True)
+                                        info_root=args.output_dir, allow_random_init=True,
+                                        backbone_dtype=BACKBONE_DTYPES[args.backbone_dtype])
         from . import ops
 
         for (alpha, X), tau in zip(res, args.tau):

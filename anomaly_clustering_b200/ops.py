@@ -120,20 +120,12 @@ def embed(
     out_n2: Optional[torch.Tensor] = None,
 ):
     """Fused stage 1.  Returns (Z [B*P, D] fp32 | None, Zhi | None, Zlo | None, (h, w)).  out_n2 [B*P] fp32 (needs an
-    operand) receives the squared norms of the operand rows (ac_embed_ex)."""
+    operand) receives the squared norms of the operand rows (ac_embed_dt).  The maps are float32, float16 or bfloat16, one
+    dtype for all layers; 16-bit maps give the same bits as their float32 upcast."""
     lib = _lib.load()
-    views = [feature_view(f) for f in features]
-    _need_cuda(*views)
-    for v in views:
-        if v.dtype != torch.float32:
-            raise ValueError("features must be float32")
+    views, arr, feat_dt = _layer_array(features)
     B = views[0].shape[0]
     L = len(views)
-    arr = (AcLayer * L)()
-    for i, v in enumerate(views):
-        _, C, H, W = v.shape
-        sb, sc, sh, sw = v.stride()
-        arr[i] = AcLayer(v.data_ptr(), C, H, W, sb, sc, sh, sw)
     h, w = patch_grid(views[0].shape[2], views[0].shape[3], patchsize, stride)
     rows = B * h * w
     dev = views[0].device
@@ -146,12 +138,12 @@ def embed(
         hi = out_hi if out_hi is not None else torch.empty(rows, target_dim, dtype=tdt, device=dev)
         if want_lo:
             lo = out_lo if out_lo is not None else torch.empty(rows, target_dim, dtype=tdt, device=dev)
-    ws_bytes = lib.ac_embed_workspace_bytes(arr, L, B, patchsize, stride, pretrain_dim, target_dim)
+    ws_bytes = lib.ac_embed_workspace_bytes_dt(arr, L, feat_dt, B, patchsize, stride, pretrain_dim, target_dim)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
     if out_n2 is not None:
         assert hi is not None and out_n2.dtype == torch.float32 and out_n2.numel() == rows and out_n2.is_contiguous()
-    rc = lib.ac_embed_ex(arr, L, B, patchsize, stride, pretrain_dim, target_dim, int(layernorm), float(eps), _ptr(Z), _ptr(hi),
-                         _ptr(lo), op_code, _ptr(out_n2), _ptr(ws), ws_bytes, _stream())
+    rc = lib.ac_embed_dt(arr, L, feat_dt, B, patchsize, stride, pretrain_dim, target_dim, int(layernorm), float(eps), _ptr(Z),
+                         _ptr(hi), _ptr(lo), op_code, _ptr(out_n2), _ptr(ws), ws_bytes, _stream())
     check(rc, "ac_embed")
     return Z, hi, lo, (h, w)
 
@@ -397,16 +389,20 @@ def weighted_embed_multi(alpha32: torch.Tensor, Z: torch.Tensor) -> torch.Tensor
 
 
 def _layer_array(features):
+    """(views, AcLayer array, AC_DT_* code of the maps).  float32, float16 and bfloat16 maps, one dtype for all layers."""
     views = [feature_view(f) for f in features]
     _need_cuda(*views)
+    dt = views[0].dtype
+    if dt not in _TORCH_TO_AC:
+        raise ValueError("features must be float32, float16 or bfloat16, got %s" % dt)
+    if any(v.dtype != dt for v in views):
+        raise ValueError("all feature maps must share one dtype, got %s" % sorted({str(v.dtype) for v in views}))
     arr = (AcLayer * len(views))()
     for i, v in enumerate(views):
-        if v.dtype != torch.float32:
-            raise ValueError("features must be float32")
         _, C, H, W = v.shape
         sb, sc, sh, sw = v.stride()
         arr[i] = AcLayer(v.data_ptr(), C, H, W, sb, sc, sh, sw)
-    return views, arr
+    return views, arr, _TORCH_TO_AC[dt]
 
 
 def weighted_embed_from_features(features: Sequence[torch.Tensor], alpha32: torch.Tensor, patchsize: int, stride: int,
@@ -414,14 +410,14 @@ def weighted_embed_from_features(features: Sequence[torch.Tensor], alpha32: torc
     """X [B, D] = sum_p alpha[b,p] Z[b,p] computed from the feature maps (no Z).  Raises AcError(AC_ERR_UNSUPPORTED)
     for shapes outside the fast form (callers fall back to embed + weighted_embed)."""
     lib = _lib.load()
-    views, arr = _layer_array(features)
+    views, arr, feat_dt = _layer_array(features)
     B, L = views[0].shape[0], len(views)
     a = alpha32.reshape(B, -1).contiguous().float()
     X = torch.empty(B, target_dim, dtype=torch.float32, device=views[0].device)
-    ws_bytes = lib.ac_weighted_embed_from_features_workspace_bytes(arr, L, B, patchsize)
+    ws_bytes = lib.ac_weighted_embed_from_features_workspace_bytes_dt(arr, L, feat_dt, B, patchsize)
     ws = torch.empty(max(ws_bytes, 256), dtype=torch.uint8, device=views[0].device)
-    rc = lib.ac_weighted_embed_from_features(arr, L, B, patchsize, stride, pretrain_dim, target_dim, int(layernorm), float(eps),
-                                             _ptr(a), _ptr(X), _ptr(ws), ws_bytes, _stream())
+    rc = lib.ac_weighted_embed_from_features_dt(arr, L, feat_dt, B, patchsize, stride, pretrain_dim, target_dim, int(layernorm),
+                                                float(eps), _ptr(a), _ptr(X), _ptr(ws), ws_bytes, _stream())
     check(rc, "ac_weighted_embed_from_features")
     return X
 

@@ -96,6 +96,7 @@ class NetworkFeatureAggregator(torch.nn.Module):
 
     def feature_dimensions(self, input_shape) -> List[int]:
         """common.py:270-275 (shape[1] of every hooked output for a dummy input)."""
-        _input = torch.ones([1] + list(input_shape)).to(self.device)
+        p = next(self.backbone.parameters(), None)
+        _input = torch.ones([1] + list(input_shape), dtype=p.dtype if p is not None else torch.float32).to(self.device)
         _output = self(_input)
         return [_output[layer].shape[1] for layer in self.layers_to_extract_from]

@@ -76,8 +76,10 @@ class AnomalyClusteringCore(torch.nn.Module):
         return [feats[layer] for layer in self.layers_to_extract_from]
 
     def embed_device(self, images, operand=None, want_lo=False):
-        """Addition: images [B,3,H,W] -> (Z [B*P, D] device fp32, hi, lo, patch grid); B > 1 allowed."""
-        feats = [f.float() for f in self._features(images.to(torch.float).to(self.device))]
+        """Addition: images [B,3,H,W] -> (Z [B*P, D] device fp32, hi, lo, patch grid); B > 1 allowed.  16-bit hooked maps
+        (a backbone run under bf16 / fp16 autocast) go to the kernels as they are: same result as their fp32 upcast."""
+        feats = [f if f.dtype in (torch.float16, torch.bfloat16) else f.float()
+                 for f in self._features(images.to(torch.float).to(self.device))]
         return ops.embed(feats, self.patch_maker.patchsize, self.patch_maker.stride or 1, self.pretrain_embed_dimension,
                          self.target_embed_dimension, layernorm=True, operand=operand, want_lo=want_lo)
 

@@ -100,6 +100,20 @@ int ac_embed_ex(const ac_layer_t* layers_host, int L, int B, int patchsize, int 
                 int layernorm, float eps, float* Z, void* Zhi, void* Zlo, int op_dtype, float* n2, void* ws,
                 size_t ws_bytes, ac_stream_t stream);
 
+/* 16-bit backbone feature maps (a backbone run in bf16 or fp16): the same as ac_embed_ex / ac_embed_workspace_bytes
+ * with every layer's ptr read as feat_dtype elements (AC_DT_F32, AC_DT_F16 or AC_DT_BF16, one type for all layers);
+ * strides stay in elements.  Each 16-bit value is widened to fp32 as it is loaded and the LayerNorm and everything
+ * after it run in fp32, so every output is BIT-IDENTICAL to the fp32 call on the upcast maps with the same strides and
+ * the same element offsets.  (The forms that stage rows with bulk copies need 16-byte aligned rows: C % 8 == 0 for
+ * 16-bit maps; the statistics pre-pass picks its vector loads from the element offset of each image, offset % 4 == 0.)
+ * The workspace of a 16-bit call also holds an fp32 channel-contiguous copy of each map for the per-layer forms.
+ * An unknown feat_dtype: AC_ERR_INVALID (workspace: 0). */
+size_t ac_embed_workspace_bytes_dt(const ac_layer_t* layers_host, int L, int feat_dtype, int B, int patchsize, int stride,
+                                   int Dp, int D);
+int ac_embed_dt(const ac_layer_t* layers_host, int L, int feat_dtype, int B, int patchsize, int stride, int Dp, int D,
+                int layernorm, float eps, float* Z, void* Zhi, void* Zlo, int op_dtype, float* n2, void* ws,
+                size_t ws_bytes, ac_stream_t stream);
+
 /* PatchMaker.patchify standalone (models/patchcore/patchcore.py:439-465):
  * x [B,C,H,W] contiguous -> out [B, h*w, C, k, k]; grid_host[2] receives (h, w). */
 int ac_patchify(const float* x, int B, int C, int H, int W, int patchsize, int stride, float* out,
@@ -259,6 +273,13 @@ size_t ac_weighted_embed_from_features_workspace_bytes(const ac_layer_t* layers_
 int ac_weighted_embed_from_features(const ac_layer_t* layers_host, int L, int B, int patchsize, int stride, int Dp,
                                     int D, int layernorm, float eps, const float* alpha, float* X, void* ws,
                                     size_t ws_bytes, ac_stream_t stream);
+/* The same for feature maps of element type feat_dtype (see ac_embed_dt): X is bit-identical to the fp32 call on the
+ * upcast maps with the same strides and element offsets. */
+size_t ac_weighted_embed_from_features_workspace_bytes_dt(const ac_layer_t* layers_host, int L, int feat_dtype, int B,
+                                                          int patchsize);
+int ac_weighted_embed_from_features_dt(const ac_layer_t* layers_host, int L, int feat_dtype, int B, int patchsize,
+                                       int stride, int Dp, int D, int layernorm, float eps, const float* alpha, float* X,
+                                       void* ws, size_t ws_bytes, ac_stream_t stream);
 
 /* Multi-GPU plumbing (no counterpart in the reference, which is single-device: examples/main.py:38): up to 16 strided 2-D blocks
  * (rows x row_bytes, row_bytes a multiple of 4, own row strides in bytes) copied in ONE launch.  Sources / destinations may be
