@@ -58,9 +58,15 @@ struct EmbedParams {
   void* Zhi;
   void* Zlo;
   int op_dtype;
+  int vec;               // kVecZ / kVecOp: the output may take 16-byte vector stores (host: vec_flags)
   long long ldz;
   const double* stats;   // [B][L][kStatSplit][2]
 };
+
+// Bits of EmbedParams::vec.  A kernel stores 16-byte vectors only where the element offset is a multiple of the vector
+// width AND the base pointer is 16-byte aligned; any other output takes scalar stores of the same bits.
+static constexpr int kVecZ = 1;    // Z is 16-byte aligned
+static constexpr int kVecOp = 2;   // Zhi and (if present) Zlo are 16-byte aligned
 
 struct LaunchGeom {
   int chan_contig;       // smem tile is [row][col][chan] (token layout) else [chan][row][col]
@@ -137,6 +143,9 @@ __global__ void __launch_bounds__(256) ln_stats_kernel(EmbedParams p, double* st
   const T* base = map_ptr<T>(ly) + (long long)b * ly.sb;
   // dense images (any axis permutation) can be walked flat
   long long lo_e = n * blockIdx.x / gridDim.x, hi_e = n * (blockIdx.x + 1) / gridDim.x;
+  // every value is summed relative to the image's first element (a pivot): sums of x - pivot keep E[x^2] - mean^2 accurate
+  // for maps whose mean is large against their spread
+  const float piv = ld_map(base, 0);
   float s = 0.f, q = 0.f;
   const bool tok = (ly.sc == 1 && ly.sw == ly.C && ly.sh == (long long)ly.W * ly.C);
   const bool cnn = (ly.sw == 1 && ly.sh == ly.W && ly.sc == (long long)ly.H * ly.W);
@@ -146,7 +155,8 @@ __global__ void __launch_bounds__(256) ln_stats_kernel(EmbedParams p, double* st
     // dense image, aligned slices: 4 elements per load, 4 independent accumulator pairs
     float s2 = 0.f, q2 = 0.f, s3 = 0.f, q3 = 0.f, s4 = 0.f, q4 = 0.f;
     for (long long e = lo_e / 4 + threadIdx.x; e < hi_e / 4; e += blockDim.x) {
-      const float4 v = ld4_map(base + 4 * e);
+      float4 v = ld4_map(base + 4 * e);
+      v.x -= piv; v.y -= piv; v.z -= piv; v.w -= piv;
       s += v.x; q = fmaf(v.x, v.x, q);
       s2 += v.y; q2 = fmaf(v.y, v.y, q2);
       s3 += v.z; q3 = fmaf(v.z, v.z, q3);
@@ -156,7 +166,7 @@ __global__ void __launch_bounds__(256) ln_stats_kernel(EmbedParams p, double* st
     q = (q + q2) + (q3 + q4);
   } else if (tok || cnn) {
     for (long long e = lo_e + threadIdx.x; e < hi_e; e += blockDim.x) {
-      const float v = ld_map(base, e);
+      const float v = ld_map(base, e) - piv;
       s += v;
       q = fmaf(v, v, q);
     }
@@ -166,7 +176,7 @@ __global__ void __launch_bounds__(256) ln_stats_kernel(EmbedParams p, double* st
       const int c = (int)(e / HW);
       const int r = (int)(e - (long long)c * HW);
       const int y = r / ly.W, x = r - y * ly.W;
-      const float v = ld_map(base, c * ly.sc + y * ly.sh + x * ly.sw);
+      const float v = ld_map(base, c * ly.sc + y * ly.sh + x * ly.sw) - piv;
       s += v;
       q = fmaf(v, v, q);
     }
@@ -207,8 +217,19 @@ __device__ __forceinline__ void store_out(const EmbedParams& p, long long row, i
 }
 
 
-// Warp-collective: mean / rstd of (image b, layer) from the statistics pre-pass partials
-// (biased variance, eps inside the sqrt -- nn.LayerNorm semantics, patchcore.py:384-385).
+// mean / rstd from the sums of x - pivot over n values (fixed fp64 order; biased variance, eps inside the sqrt --
+// nn.LayerNorm semantics, patchcore.py:384-385)
+__device__ __forceinline__ void ln_from_sums(double a, double q, double n, float piv, float eps, float& mu, float& rstd) {
+  const double m = a / n;
+  double var = q / n - m * m;
+  if (var < 0) var = 0;
+  mu = (float)((double)piv + m);
+  rstd = (float)(1.0 / sqrt(var + (double)eps));
+}
+
+// Warp-collective: mean / rstd of (image b, layer) from the statistics pre-pass partials.  T: element type of ly.ptr (the
+// pivot of ln_stats_kernel is the image's first element).
+template <typename T = float>
 __device__ __forceinline__ void warp_ln_params(const EmbedParams& p, const LayerDev& ly, int b, int layer, int lane, float& mu,
                                                float& rstd) {
   mu = 0.f;
@@ -219,12 +240,7 @@ __device__ __forceinline__ void warp_ln_params(const EmbedParams& p, const Layer
   for (int i = lane; i < kStatSplit; i += 32) { a += st[2 * i]; q += st[2 * i + 1]; }
   a = warp_sum(a);
   q = warp_sum(q);
-  const double n = (double)ly.C * ly.H * ly.W;
-  const double m = a / n;
-  double var = q / n - m * m;
-  if (var < 0) var = 0;
-  mu = (float)m;
-  rstd = (float)(1.0 / sqrt(var + (double)p.eps));
+  ln_from_sums(a, q, (double)ly.C * ly.H * ly.W, ld_map(map_ptr<T>(ly) + (long long)b * ly.sb, 0), p.eps, mu, rstd);
 }
 
 // MAXTAPS > 0: per-thread tap tables in registers.  MAXTAPS == 0: taps re-enumerated on the fly
@@ -428,7 +444,7 @@ __device__ __forceinline__ void store_operand(void* Zhi, void* Zlo, long long id
 template <int NOUT>
 __device__ __forceinline__ void store_outputs(const EmbedParams& p, long long idx, int t_base, const float (&out)[NOUT]) {
   if (p.Z) {
-    if (NOUT % 4 == 0 && ((p.ldz | t_base) & 3) == 0) {
+    if (NOUT % 4 == 0 && (p.vec & kVecZ) && ((p.ldz | t_base) & 3) == 0) {
 #pragma unroll
       for (int o = 0; o + 4 <= NOUT; o += 4)
         *reinterpret_cast<float4*>(p.Z + idx + o) = make_float4(out[o], out[o + 1], out[o + 2], out[o + 3]);
@@ -438,7 +454,7 @@ __device__ __forceinline__ void store_outputs(const EmbedParams& p, long long id
     }
   }
   if (p.Zhi) {
-    const bool vec = (NOUT % 8 == 0) && (((p.ldz | t_base) & 7) == 0);
+    const bool vec = (NOUT % 8 == 0) && (p.vec & kVecOp) && (((p.ldz | t_base) & 7) == 0);
     if (p.op_dtype == AC_DT_F16) store_operand<__half, NOUT>(p.Zhi, p.Zlo, idx, vec, out);
     else store_operand<__nv_bfloat16, NOUT>(p.Zhi, p.Zlo, idx, vec, out);
   }
@@ -843,8 +859,8 @@ __global__ void __launch_bounds__(kFT + 32, 3) embed_fused_kernel(const __grid_c
   __syncthreads();
   uint32_t slot = 0, ph = 0;                               // ring position: identical sequence in both roles
   const uint32_t full0 = e_smem_u32(&s_full[0]), empty0 = e_smem_u32(&s_empty[0]);
-  const bool vec8 = (NOUT % 8 == 0) && (((p.ldz | fp.t_stride) & 7) == 0);
-  const bool vec4 = (NOUT % 4 == 0) && (((p.ldz | fp.t_stride) & 3) == 0);
+  const bool vec8 = (NOUT % 8 == 0) && (p.vec & kVecOp) && (((p.ldz | fp.t_stride) & 7) == 0);
+  const bool vec4 = (NOUT % 4 == 0) && (p.vec & kVecZ) && (((p.ldz | fp.t_stride) & 3) == 0);
   const bool f16 = (p.op_dtype == AC_DT_F16);
   const T* ring_t = ring + tid * TCH;
 
@@ -924,6 +940,7 @@ __global__ void __launch_bounds__(kFT + 32, 3) embed_fused_kernel(const __grid_c
       if (bA >= 0 && p.layernorm) {
         for (int l = 0; l < p.L; ++l) {
           float s = 0.f, qq = 0.f;
+          const float piv = ld_map(map_ptr<T>(p.layers[l]) + (long long)(p.b0 + bA) * p.layers[l].sb, 0);   // see ln_stats_kernel
           for (int cx = 0; cx < fp.gx; ++cx) {
             const int m0 = (cx * kFT + tid) * kPP;            // first period of this thread
             for (int t = 0; t < nA; ++t) {
@@ -935,7 +952,7 @@ __global__ void __launch_bounds__(kFT + 32, 3) embed_fused_kernel(const __grid_c
                 if (ki < ntok) {
 #pragma unroll
                   for (int c = 0; c < TCH; ++c)
-                    if (m0 + c / CPP < fp.nperiods) { const float v = op_to_float(col[ki * NCH + c]); s += v; qq = fmaf(v, v, qq); }
+                    if (m0 + c / CPP < fp.nperiods) { const float v = op_to_float(col[ki * NCH + c]) - piv; s += v; qq = fmaf(v, v, qq); }
                 }
               __syncwarp();
               if (lane == 0) e_mbar_arrive(empty0 + slot * 8);
@@ -978,11 +995,10 @@ __global__ void __launch_bounds__(kFT + 32, 3) embed_fused_kernel(const __grid_c
               for (int i = lane; i < fp.S; i += 32) { a += __ldcg(st + 2 * i); c2 += __ldcg(st + 2 * i + 1); }
               a = warp_sum(a);
               c2 = warp_sum(c2);
-              const double n = (double)p.layers[l].C * p.layers[l].H * p.layers[l].W;
-              const double m = a / n;
-              double var = c2 / n - m * m;
-              if (var < 0) var = 0;
-              if (lane == 0) { s_mu[l] = (float)m; s_rs[l] = (float)(1.0 / sqrt(var + (double)p.eps)); }
+              float mu, rs;
+              ln_from_sums(a, c2, (double)p.layers[l].C * p.layers[l].H * p.layers[l].W,
+                           ld_map(map_ptr<T>(p.layers[l]) + (long long)(p.b0 + bE) * p.layers[l].sb, 0), p.eps, mu, rs);
+              if (lane == 0) { s_mu[l] = mu; s_rs[l] = rs; }
             }
           }
           consumer_bar_f();
@@ -1409,17 +1425,20 @@ __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const _
       const bool hasA = (bA >= 0) && p.layernorm, hasB = (bE >= 0);
       constexpr int NW = FT / 32;
       float2 s2 = make_float2(0.f, 0.f), q2 = make_float2(0.f, 0.f);
-      // one statistics slot: K tokens of image bA (all channels of this thread's share), sum and sum of squares
-      auto stats_slot = [&]() {
+      // one statistics slot: the first ntok of its K tokens of image bA (all channels of this thread's share; the others are
+      // zero rows), sum and sum of squares of x - pivot (see ln_stats_kernel)
+      auto stats_slot = [&](int ntok, float2 npiv) {
         e_mbar_wait_spin(full0 + slot * 8, ph);
         const uint32_t base = ring_a + slot * kSlotBytes;
 #pragma unroll
         for (int ki = 0; ki < K; ++ki)
+          if (ki < ntok) {                                 // warp-uniform
 #pragma unroll
-          for (int c = 0; c < TCH; c += 2) {
-            const float2 v = e_lds_pair(base + (uint32_t)(ki * NCH + c) * E, T{});
-            s2 = __fadd2_rn(s2, v);
-            q2 = __ffma2_rn(v, v, q2);
+            for (int c = 0; c < TCH; c += 2) {
+              const float2 v = __fadd2_rn(e_lds_pair(base + (uint32_t)(ki * NCH + c) * E, T{}), npiv);
+              s2 = __fadd2_rn(s2, v);
+              q2 = __ffma2_rn(v, v, q2);
+            }
           }
         __syncwarp();
         if (lane == 0) e_mbar_arrive(empty0 + slot * 8);
@@ -1439,7 +1458,8 @@ __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const _
       // S * NW partials behind two CTA barriers: 11 % of the consumers' samples in the round-2 ncu capture.)
       if (hasA) {
         for (int l = 0; l < p.L; ++l) {
-          for (int t = 0; t < nA; ++t) stats_slot();
+          const float piv = ld_map(map_ptr<T>(p.layers[l]) + (long long)bA * p.layers[l].sb, 0);
+          for (int t = 0; t < nA; ++t) stats_slot(min(K, nposA - K * t), make_float2(-piv, -piv));
           stats_flush(l);
         }
         int old = 0;
@@ -1470,11 +1490,10 @@ __global__ void __launch_bounds__(FT + 32, MINB) embed_fused_fast_kernel(const _
             }
             a = warp_sum(a);
             c2 = warp_sum(c2);
-            const double nn = (double)p.layers[l].C * p.layers[l].H * p.layers[l].W;
-            const double m = a / nn;
-            double var = c2 / nn - m * m;
-            if (var < 0) var = 0;
-            if (lane == 0) e_st_relaxed_u64(fp.murs + (long long)bA * p.L + l, e_pack2((float)m, (float)(1.0 / sqrt(var + (double)p.eps))));
+            float mu, rs;
+            ln_from_sums(a, c2, (double)p.layers[l].C * p.layers[l].H * p.layers[l].W,
+                         ld_map(map_ptr<T>(p.layers[l]) + (long long)bA * p.layers[l].sb, 0), p.eps, mu, rs);
+            if (lane == 0) e_st_relaxed_u64(fp.murs + (long long)bA * p.L + l, e_pack2(mu, rs));
           }
         }
       }
@@ -1726,7 +1745,7 @@ __global__ void __launch_bounds__(256) xcorr_kernel(EmbedParams p, int layer, co
   }
   if (threadIdx.x < 32) {
     float mu, rstd;
-    warp_ln_params(p, ly, p.b0 + b, layer, lane, mu, rstd);
+    warp_ln_params<T>(p, ly, p.b0 + b, layer, lane, mu, rstd);
     if (lane == 0) { s_mu = mu; s_rstd = rstd; }
   }
   __syncthreads();
@@ -2137,8 +2156,8 @@ static int launch_fused(EmbedParams p, const Periodic& pr, float* n2, void* ws, 
   memset(&fp, 0, sizeof(fp));
   // lean kernel: fp16 operands + norms (+ fp32 Z), every consumer thread owns two periods of every layer
   const bool lean_out = g_fused_lean && p.Zhi && !p.Zlo && p.op_dtype == AC_DT_F16 && n2 && pr.R == 1 && pr.A == 27 &&
-                        (p.ldz % 8 == 0) && (pr.ncols % 8 == 0) && (reinterpret_cast<uintptr_t>(p.Zhi) % 16 == 0) &&
-                        (!p.Z || reinterpret_cast<uintptr_t>(p.Z) % 16 == 0) && p.h0 == p.w0;   // slices: row runs / column runs
+                        (p.ldz % 8 == 0) && (pr.ncols % 8 == 0) && (p.vec & kVecOp) &&
+                        (!p.Z || (p.vec & kVecZ)) && p.h0 == p.w0;   // slices: row runs / column runs
   p.nxseg = ceil_div(p.w0, kMaxSeg);
   p.xseg_len = ceil_div(p.w0, p.nxseg);
   p.nxseg = ceil_div(p.w0, p.xseg_len);
@@ -2239,6 +2258,11 @@ static int with_feat_type(int dt, F&& f) {
   if (dt == AC_DT_BF16) return f(__nv_bfloat16{});
   return f(float{});
 }
+static bool aligned16(const void* ptr) { return (reinterpret_cast<uintptr_t>(ptr) & 15) == 0; }
+// EmbedParams::vec for the outputs (Z, Zhi, Zlo): which of them the kernels may write with 16-byte vector stores
+static int vec_flags(const float* Z, const void* Zhi, const void* Zlo) {
+  return (aligned16(Z) ? kVecZ : 0) | (aligned16(Zhi) && aligned16(Zlo) ? kVecOp : 0);
+}
 static bool feat_dtype_ok(int dt) { return dt == AC_DT_F32 || dt == AC_DT_F16 || dt == AC_DT_BF16; }
 static int feat_esize(int dt) { return dt == AC_DT_F32 ? 4 : 2; }
 
@@ -2311,7 +2335,7 @@ extern "C" int ac_embed_dt(const ac_layer_t* layers, int L, int feat_dtype, int 
   if (n2 && !Zhi) return AC_ERR_INVALID;
   if (Zhi && op_dtype != AC_DT_F16 && op_dtype != AC_DT_BF16) return AC_ERR_INVALID;
   if (Zlo && !Zhi) return AC_ERR_INVALID;
-  if (B < 1) return AC_ERR_INVALID;
+  if (B < 1 || !aligned16(ws)) return AC_ERR_INVALID;
   int rc = check_device();
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
@@ -2373,6 +2397,7 @@ extern "C" int ac_embed_dt(const ac_layer_t* layers, int L, int feat_dtype, int 
   } else {
     p.Z = dconcat; p.Zhi = nullptr; p.Zlo = nullptr; p.op_dtype = 0;
   }
+  p.vec = vec_flags(p.Z, p.Zhi, p.Zlo);
   int dev = 0, num_sms = 148;
   AC_CUDA(cudaGetDevice(&dev));
   AC_CUDA(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
@@ -2380,7 +2405,7 @@ extern "C" int ac_embed_dt(const ac_layer_t* layers, int L, int feat_dtype, int 
   // Single-pass fused form (one persistent launch: statistics, every layer, operand norms) when the shape allows it
   if (fused_eligible(plan, p, pr, L, esize)) {
     const size_t fb = fused_ws_bytes(L, B, p.h0, p.w0) + 256;
-    if (fb > ws_bytes || (reinterpret_cast<uintptr_t>(ws) & 15) != 0) return AC_ERR_WORKSPACE;
+    if (fb > ws_bytes) return AC_ERR_WORKSPACE;
     p.B = B;
     void* fws = w8 + ((ws_bytes - fb) & ~(size_t)255);
     return with_feat_type(feat_dtype, [&](auto tag) { return launch_fused<decltype(tag)>(p, pr[0], n2, fws, num_sms, st); });
@@ -2433,6 +2458,7 @@ extern "C" int ac_embed_dt(const ac_layer_t* layers, int L, int feat_dtype, int 
         q.h0 = ly.gh; q.w0 = ly.gw;
         q.Z = cbuf[l] - (long long)q.b0 * ly.gh * ly.gw * prl.ncols;
         q.Zhi = nullptr; q.Zlo = nullptr; q.op_dtype = 0; q.ldz = prl.ncols;
+        q.vec = vec_flags(q.Z, nullptr, nullptr);
         prl.t_base = 0;
       }
       rc = launch_periodic(q, prl, l, aligned && tma_aligned(q, l, 4), num_sms, st);
@@ -2501,7 +2527,7 @@ extern "C" size_t ac_weighted_embed_from_features_workspace_bytes(const ac_layer
 extern "C" int ac_weighted_embed_from_features_dt(const ac_layer_t* layers, int L, int feat_dtype, int B, int patchsize, int stride,
                                                   int Dp, int D, int layernorm, float eps, const float* alpha, float* X, void* ws,
                                                   size_t ws_bytes, ac_stream_t stream) {
-  if (!layers || !alpha || !X || !ws || B < 1 || !feat_dtype_ok(feat_dtype)) return AC_ERR_INVALID;
+  if (!layers || !alpha || !X || !ws || !aligned16(ws) || B < 1 || !feat_dtype_ok(feat_dtype)) return AC_ERR_INVALID;
   int rc = check_device();
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;

@@ -122,19 +122,23 @@ def embed(
     """Fused stage 1.  Returns (Z [B*P, D] fp32 | None, Zhi | None, Zlo | None, (h, w)).  out_n2 [B*P] fp32 (needs an
     operand) receives the squared norms of the operand rows (ac_embed_dt).  The maps are float32, float16 or bfloat16, one
     dtype for all layers; 16-bit maps give the same bits as their float32 upcast."""
+    view0 = feature_view(features[0])
+    B = view0.shape[0]
+    h, w = patch_grid(view0.shape[2], view0.shape[3], patchsize, stride)
+    rows = B * h * w
+    dev = view0.device
+    tdt, op_code = _OP_DTYPES[operand] if operand is not None else (None, 0)
+    # caller buffers are written as dense [rows, target_dim] arrays: anything else would be written out of bounds
+    _out_ok(out_z if want_z else None, "out_z", (rows, target_dim), torch.float32, dev)
+    _out_ok(out_hi if operand is not None else None, "out_hi", (rows, target_dim), tdt, dev)
+    _out_ok(out_lo if operand is not None and want_lo else None, "out_lo", (rows, target_dim), tdt, dev)
     lib = _lib.load()
     views, arr, feat_dt = _layer_array(features)
-    B = views[0].shape[0]
     L = len(views)
-    h, w = patch_grid(views[0].shape[2], views[0].shape[3], patchsize, stride)
-    rows = B * h * w
-    dev = views[0].device
     Z = hi = lo = None
     if want_z:
         Z = out_z if out_z is not None else torch.empty(rows, target_dim, dtype=torch.float32, device=dev)
-    op_code = 0
     if operand is not None:
-        tdt, op_code = _OP_DTYPES[operand]
         hi = out_hi if out_hi is not None else torch.empty(rows, target_dim, dtype=tdt, device=dev)
         if want_lo:
             lo = out_lo if out_lo is not None else torch.empty(rows, target_dim, dtype=tdt, device=dev)
@@ -146,6 +150,15 @@ def embed(
                          _ptr(hi), _ptr(lo), op_code, _ptr(out_n2), _ptr(ws), ws_bytes, _stream())
     check(rc, "ac_embed")
     return Z, hi, lo, (h, w)
+
+
+def _out_ok(t: Optional[torch.Tensor], name: str, shape, dtype, dev) -> None:
+    """A caller-provided output buffer of ops.embed: exactly `shape`, `dtype`, on `dev`, contiguous (any storage offset)."""
+    if t is None:
+        return
+    if tuple(t.shape) != tuple(shape) or t.dtype != dtype or t.device != dev or not t.is_contiguous():
+        raise ValueError("%s must be a contiguous %s tensor of shape %s on %s, got %s %s on %s (contiguous: %s)"
+                         % (name, dtype, tuple(shape), dev, t.dtype, tuple(t.shape), t.device, t.is_contiguous()))
 
 
 def patchify(x: torch.Tensor, patchsize: int, stride: int):

@@ -279,7 +279,9 @@ def z_free_supported(features, patchsize, stride, pretrain_dim, target_dim, prec
     L = len(views)
     if (L * pretrain_dim) % target_dim != 0 or pretrain_dim % ((L * pretrain_dim) // target_dim) != 0:
         return False
-    return True
+    # the alpha map of an image with its one-position zero halo is staged in shared memory: at most 200 KB of fp32
+    h, w = ops.patch_grid(views[0].shape[2], views[0].shape[3], patchsize, stride)
+    return (h + 2) * (w + 2) * 4 <= 200 * 1024
 
 
 def run_path(

@@ -87,7 +87,10 @@ int ac_last_watchdog(void);
  *                 the tensor-core operands of ac_min_dist
  *   layernorm   : 1 = AnomalyClusteringCore._embed, 0 = PatchCore._embed (patchcore.py:92-146)
  * Workspace: ac_embed_workspace_bytes(layers_host, L, B, patchsize, stride, Dp, D) (statistics partials,
- * chunk table, and -- only for CNN-layout or resampled layers -- channel-contiguous / coarse-grid scratch). */
+ * chunk table, and -- only for CNN-layout or resampled layers -- channel-contiguous / coarse-grid scratch).
+ * ws must be 16-byte aligned, else AC_ERR_INVALID.  Z, Zhi and Zlo may have any element alignment: an output whose
+ * base pointer is 16-byte aligned is written with 16-byte vector stores where the row pitch allows, any other with
+ * scalar stores, and the bits written are the same either way. */
 size_t ac_embed_workspace_bytes(const ac_layer_t* layers_host, int L, int B, int patchsize, int stride, int Dp,
                                 int D);
 int ac_embed(const ac_layer_t* layers_host, int L, int B, int patchsize, int stride, int Dp, int D,
@@ -268,7 +271,8 @@ int ac_weighted_embed_multi(const float* alpha, const float* Z, int T, int N, in
  * a 3x3 correlation of the alpha map with every channel, then the MeanMapper / Aggregator windows once per
  * image.  Same result as ac_embed + ac_weighted_embed (examples/main.py:266-296) while fp32 Z is never stored.
  * alpha [B, P] fp32, X [B, D] fp32.  Needs patchsize 3, stride 1, every layer on the layer-0 grid and Aggregator
- * windows that do not straddle layers, else AC_ERR_UNSUPPORTED (use ac_embed + ac_weighted_embed). */
+ * windows that do not straddle layers, and a (h0 + 2) x (w0 + 2) fp32 alpha tile of at most 200 KB (h0 = w0 <= 224),
+ * else AC_ERR_UNSUPPORTED (use ac_embed + ac_weighted_embed).  ws must be 16-byte aligned, else AC_ERR_INVALID. */
 size_t ac_weighted_embed_from_features_workspace_bytes(const ac_layer_t* layers_host, int L, int B, int patchsize);
 int ac_weighted_embed_from_features(const ac_layer_t* layers_host, int L, int B, int patchsize, int stride, int Dp,
                                     int D, int layernorm, float eps, const float* alpha, float* X, void* ws,

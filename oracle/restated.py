@@ -63,17 +63,20 @@ def embed(
     target_dim: int,
     layernorm: bool = True,
     eps: float = 1e-5,
+    dtype: torch.dtype = torch.float32,
 ) -> torch.Tensor:
     """AnomalyClusteringCore._embed after the backbone (models/patchcore/patchcore.py:368-431)
     + Preprocessing/MeanMapper (models/patchcore/common.py:145-170) + Aggregator (:173-183).
 
-    features: per-layer [B,C,H,W] maps or [B,1+P,C] token tensors.  Returns Z [B*P0, D] fp32,
+    features: per-layer [B,C,H,W] maps or [B,1+P,C] token tensors.  Returns Z [B*P0, D] in `dtype`,
     P0 = patch count of layer 0.  `layernorm=False` gives PatchCore._embed (patchcore.py:92-146).
+    Every op is computed in `dtype`: float32 is the reference's own arithmetic, float64 the high-precision
+    reference the CUDA kernels are tested against.
     """
     planes = []
     grids = []
     for f in features:
-        f = tokens_to_map(f.float())
+        f = tokens_to_map(f.to(dtype))
         if layernorm:
             f = whole_map_layernorm(f, eps)
         u, g = unfold_patches(f, patchsize, stride)
@@ -175,6 +178,11 @@ def matrix_alpha_supervised(tau: float, Z: torch.Tensor, Z_train: torch.Tensor) 
 def matrix_alpha_average(N: int, P: int) -> torch.Tensor:
     """'average' mode (examples/main.py:290-291)."""
     return torch.ones(N, P) / P
+
+
+def weighted_embedding64(alpha: torch.Tensor, Z: torch.Tensor) -> torch.Tensor:
+    """X[i] = sum_p alpha[i,p] Z[i,p] summed in float64 (the reference for the X kernels).  alpha [N,P], Z [N,P,D] -> [N,D]."""
+    return torch.einsum("np,npd->nd", alpha.double(), Z.double())
 
 
 def weighted_embedding(alpha: torch.Tensor, Z: torch.Tensor) -> np.ndarray:
