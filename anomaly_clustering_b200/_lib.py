@@ -113,6 +113,16 @@ SIGNATURES = {
         [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int,
          c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p],
     ),
+    "ac_min_dist_sym_grow": (
+        c_int,
+        [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int,
+         c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p],
+    ),
+    "ac_refine_min_dist_grow": (
+        c_int,
+        [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
+    ),
+    "ac_accumulate_weights_grow": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "ac_reduce_weights_sym_ex": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "ac_reduce_weights_ex": (c_int, [c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     "ac_reduce_weights_sym": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_void_p, c_void_p]),

@@ -46,6 +46,26 @@ __host__ __device__ inline int pool_end(int d, int Lin, int Lout) {
   return (int)((((int64_t)d + 1) * Lin + Lout - 1) / Lout);
 }
 
+// Ownership of the unordered pair {i, j} of N images in the symmetric distance form: the image that sees the other one
+// within the next floor((N-1)/2) positions of the circular order (ties at N/2 go to the smaller index).
+__host__ __device__ inline bool pair_owned(int i, int j, int N) {
+  int d = j - i;
+  if (d < 0) d += N;
+  if (d == 0) return false;
+  if (2 * d < N) return true;
+  if (2 * d == N) return i < j;
+  return false;
+}
+
+// Ownership when images [n_old, N) join images [0, n_old) whose pairs are already known (ac_min_dist_sym_grow): a new
+// image owns every pair with an old one, two new images follow pair_owned among the new images, and a pair of two old
+// images has no owner.  n_old = 0 is pair_owned.
+__host__ __device__ inline bool pair_owned_grow(int n_old, int i, int j, int N) {
+  if (i < n_old) return false;
+  if (j < n_old) return true;
+  return pair_owned(i - n_old, j - n_old, N - n_old);
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -62,6 +62,7 @@ struct __align__(64) TcParams {
   // symmetric (self-bank) mode: every unordered image pair is multiplied once
   int sym;                   // 0 = every (query block, bank image) unit; 1 = only pairs owned by the query image
   int q_img0;                // global image index of query row 0 (query slice of a sharded run)
+  int n_old;                 // growth (ac_min_dist_sym_grow): bank images [0, n_old) are already clustered, see pair_owned_grow
   int KU;                    // units per query block in sym mode
   unsigned int* colmin;      // [nq_img, nb_img*P] squared distances (fp32 bits), atomicMin target
   const int2* units;         // sym mode: explicit (query block, bank image) list in raster order (device-built)
@@ -81,20 +82,11 @@ struct __align__(64) TcParams {
   unsigned long long* colkey;    // sym: [nq_img, nb_img*P] (fp32 bits of d2 << 32) | row inside the query image, atomicMin target
 };
 
-// Ownership of the unordered pair {i, j} of N images: the image that sees the other one within the
-// next floor((N-1)/2) positions of the circular order (ties at N/2 go to the smaller index).
-__host__ __device__ inline bool pair_owned(int i, int j, int N) {
-  int d = j - i;
-  if (d < 0) d += N;
-  if (d == 0) return false;
-  if (2 * d < N) return true;
-  if (2 * d == N) return i < j;
-  return false;
-}
-
-// ownership with categories: image i owns the pair {i, j} iff both lie in the category of j and i owns it there
-__host__ __device__ inline bool pair_owned_grouped(const int* groups, int i, int j, int N) {
-  if (!groups) return pair_owned(i, j, N);
+// The ownership rule every part of the symmetric form reads (epilogue, unit builder, reductions): with categories, image i
+// owns the pair {i, j} iff both lie in the category of j and i owns it there; without, the growth rule (pair_owned when
+// n_old = 0).  Growth runs take no categories (the entry point refuses them).
+__host__ __device__ inline bool pair_owned_grouped(const int* groups, int n_old, int i, int j, int N) {
+  if (!groups) return pair_owned_grow(n_old, i, j, N);
 #ifdef __CUDA_ARCH__
   const int g0 = __ldg(groups + 2 * j), gn = __ldg(groups + 2 * j + 1);
 #else
@@ -490,7 +482,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) mindist_tc_kernel(const __grid_
       const bool rvalid = row < p.Mq;
       // sym mode: this row contributes (row-min and column-min) only if its image owns the pair
       const int irow = p.q_img0 + (int)((rvalid ? row : p.Mq - 1) / p.P);
-      const bool act = rvalid && (!p.sym || pair_owned_grouped(p.groups, irow, img, p.nb_img));
+      const bool act = rvalid && (!p.sym || pair_owned_grouped(p.groups, p.n_old, irow, img, p.nb_img));
       const float qn = rvalid ? __ldg(p.qn2 + row) : 0.f;
       // images covered by this warp's 32 consecutive rows (at most two when P >= 32)
       const long long wrow0 = row - lane;
@@ -654,7 +646,7 @@ __device__ __forceinline__ long long walk_units(const TcParams& p, int2* units, 
     int i0, i1;
     if (tab) { i0 = s_i0[mb]; i1 = s_i1[mb]; } else mb_range(mb, i0, i1);
     for (int i = i0; i <= i1; ++i)
-      if (pair_owned_grouped(p.groups, i, img, p.nb_img)) return true;
+      if (pair_owned_grouped(p.groups, p.n_old, i, img, p.nb_img)) return true;
     return false;
   };
   const int n_groups = (p.n_mblocks + kGM - 1) / kGM;
@@ -813,7 +805,7 @@ int launch_mindist_tc(const void* Qhi, const void* Qlo, const float* Qn2, long l
                       const float* Bn2, int nb_img, int P, int D, int precision, float* dmin, int* err_flag, cudaStream_t st,
                       int sym = 0, int q_img0 = 0, unsigned int* colmin = nullptr, void* unit_ws = nullptr, size_t unit_ws_bytes = 0,
                       int win_begin = 0, int win_count = -1, int* rowarg = nullptr, unsigned long long* colkey = nullptr,
-                      const int* groups = nullptr, const int* bank_ready = nullptr, int img_rot = 0) {
+                      const int* groups = nullptr, const int* bank_ready = nullptr, int img_rot = 0, int n_old = 0) {
   const bool bf16 = (precision == AC_PREC_BF16 || precision == AC_PREC_BF16X3);
   const bool x3 = (precision == AC_PREC_F16X3 || precision == AC_PREC_BF16X3);
   if (D % 8 != 0) return AC_ERR_UNSUPPORTED;  // TMA needs a 16-byte row pitch
@@ -832,20 +824,22 @@ int launch_mindist_tc(const void* Qhi, const void* Qlo, const float* Qn2, long l
   prm.nseg = x3 ? 3 : 1;
   prm.n_mblocks = (int)ceil_div64(Mq, (long long)kTileM * 2);
   prm.counter = (unsigned long long*)((char*)err_flag + 128);   // inside the zeroed 256-byte workspace header
-  prm.sym = sym; prm.q_img0 = q_img0; prm.colmin = colmin; prm.units = nullptr;
+  prm.sym = sym; prm.q_img0 = q_img0; prm.n_old = n_old; prm.colmin = colmin; prm.units = nullptr;
   prm.rowarg = rowarg; prm.colkey = colkey; prm.groups = groups; prm.bank_ready = bank_ready; prm.img_rot = sym ? 0 : img_rot;
   const bool arg = (rowarg != nullptr);
   if (arg && sym && !colkey) return AC_ERR_INVALID;
   prm.win_begin = win_begin; prm.win_count = (win_count < 0) ? nb_img : win_count;
   // bank images a raster group of kGM query blocks can own: N/2 after each of the images it spans (with categories the
-  // group may end in the middle of one whose images wrap around: every bank image is a candidate)
-  prm.KU = groups ? nb_img : std::min(nb_img, nb_img / 2 + (int)(((long long)kGM * kTileM * 2 - 1) / P) + 1);
+  // group may end in the middle of one whose images wrap around, and a new image of a growth run owns its pairs with every
+  // old one: every bank image is a candidate, still walked circularly from the one after the group's first query image)
+  prm.KU = (groups || n_old > 0) ? nb_img : std::min(nb_img, nb_img / 2 + (int)(((long long)kGM * kTileM * 2 - 1) / P) + 1);
   prm.total_units = (long long)prm.n_mblocks * nb_img;
   if (sym) {
     // raster order: groups of kGM query blocks; inside a group walk the bank images the group owns and,
     // per bank image, every block of the group that owns the pair (blocks sharing a bank image run
     // together).  Built on the device (count_units_kernel + emit_units_kernel).
-    // a query block spans at most rows/P + 2 images, each owns at most half of its category (<= nb_img / 2 + 1 images)
+    // a query block spans at most rows/P + 2 images, each owns at most half of its category (<= nb_img / 2 + 1 images);
+    // a new image of a growth run may own pairs with all of them, which the cap at nb_img per block covers
     const long long span = ((long long)kTileM * 2 + P - 1) / P + 1;
     const long long max_units = (long long)prm.n_mblocks * std::min<long long>(nb_img, span * (nb_img / 2 + 1));
     if (!unit_ws || unit_ws_bytes < 16 + (size_t)max_units * sizeof(int2) + kUnitWarps * sizeof(long long)) return AC_ERR_WORKSPACE;
@@ -918,7 +912,7 @@ __global__ void __launch_bounds__(256) reduce_weights_sym_kernel(const float* __
         const int j = jq + u;
         d[u] = -1.f;
         if (j < jb && j != i) {
-          const float* src = pair_owned_grouped(groups, i, j, nb_img) ? rowmin : colmin;
+          const float* src = pair_owned_grouped(groups, 0, i, j, nb_img) ? rowmin : colmin;
           d[u] = __ldg(src + (long long)j * Mq + r);
         }
       }
@@ -939,7 +933,8 @@ __global__ void __launch_bounds__(256) reduce_weights_sym_kernel(const float* __
 static int min_dist_sym_impl(const void* Qhi, const void* Qlo, const float* Qn2, int64_t Mq, int q_img0, const void* Bhi,
                              const void* Blo, const float* Bn2, int nb_img, int P, int D, int precision, int bank_begin,
                              int bank_count, int init_colmin, float* rowmin_d2, float* colmin_d2, int32_t* rowarg, uint64_t* colkey,
-                             const int32_t* groups, void* ws, size_t ws_bytes, ac_stream_t stream, const int32_t* bank_ready = nullptr) {
+                             const int32_t* groups, void* ws, size_t ws_bytes, ac_stream_t stream, const int32_t* bank_ready = nullptr,
+                             int n_old = 0) {
   const bool arg = (rowarg != nullptr);
   if (!Qhi || !Bhi || !Qn2 || !Bn2 || !rowmin_d2 || (!arg && !colmin_d2) || (arg && !colkey) || Mq < 0 || nb_img < 1 || P < 1 ||
       D < 1 || q_img0 < 0)
@@ -963,7 +958,7 @@ static int min_dist_sym_impl(const void* Qhi, const void* Qlo, const float* Qn2,
   }
   return launch_mindist_tc(Qhi, Qlo, Qn2, Mq, Bhi, Blo, Bn2, nb_img, P, D, precision, rowmin_d2, (int*)ws, st, 1, q_img0,
                            (unsigned int*)colmin_d2, (char*)ws + 256, ws_bytes - 256, bank_begin, bank_count, rowarg,
-                           (unsigned long long*)colkey, groups, bank_ready);
+                           (unsigned long long*)colkey, groups, bank_ready, 0, n_old);
 }
 
 extern "C" int ac_min_dist_sym(const void* Qhi, const void* Qlo, const float* Qn2, int64_t Mq, int q_img0, const void* Bhi,
@@ -992,6 +987,17 @@ extern "C" int ac_min_dist_sym_ready(const void* Qhi, const void* Qlo, const flo
                            rowmin_d2, colmin_d2, rowarg, colkey, groups, ws, ws_bytes, stream, bank_ready);
 }
 
+extern "C" int ac_min_dist_sym_grow(const void* Qhi, const void* Qlo, const float* Qn2, int64_t Mq, int q_img0, const void* Bhi,
+                                    const void* Blo, const float* Bn2, int nb_img, int P, int D, int precision, int bank_begin,
+                                    int bank_count, int init, float* rowmin_d2, float* colmin_d2, int32_t* rowarg, uint64_t* colkey,
+                                    const int32_t* groups, int n_old, void* ws, size_t ws_bytes, ac_stream_t stream) {
+  if ((rowarg != nullptr) != (colkey != nullptr)) return AC_ERR_INVALID;
+  if (groups) return AC_ERR_UNSUPPORTED;                      // growth of per-category batches is not implemented
+  if (n_old < 0 || n_old >= nb_img || q_img0 != n_old || Mq != (int64_t)(nb_img - n_old) * P) return AC_ERR_INVALID;
+  return min_dist_sym_impl(Qhi, Qlo, Qn2, Mq, q_img0, Bhi, Blo, Bn2, nb_img, P, D, precision, bank_begin, bank_count, init,
+                           rowmin_d2, colmin_d2, rowarg, colkey, nullptr, ws, ws_bytes, stream, nullptr, n_old);
+}
+
 extern "C" int ac_min_dist_sym_arg(const void* Qhi, const void* Qlo, const float* Qn2, int64_t Mq, int q_img0, const void* Bhi,
                                    const void* Blo, const float* Bn2, int nb_img, int P, int D, int precision, int bank_begin,
                                    int bank_count, int init_colkey, float* rowmin_d2, int32_t* rowarg, uint64_t* colkey, void* ws,
@@ -1016,6 +1022,41 @@ extern "C" int ac_reduce_weights_sym_ex(const float* rowmin_d2, const float* col
 extern "C" int ac_reduce_weights_sym(const float* rowmin_d2, const float* colmin_d2, int64_t Mq, int nb_img, int Pq, int q_img0,
                                      float* w, ac_stream_t stream) {
   return ac_reduce_weights_sym_ex(rowmin_d2, colmin_d2, Mq, nb_img, Pq, q_img0, nullptr, w, stream);
+}
+
+// Running sums of a growing category: S[R] += d(R, j) for every NEW pair {image of R, j} of one growth launch, partner images
+// j in increasing order, then w[R] = S[R] / (N - 1) for every row.  One thread per row of the whole category, so the order of
+// the fp64 additions is fixed by the data alone: the same sequence of updates gives the same bits on any launch geometry.
+// rowv [N, Mq] (new rows r = R - n_old*P, partner j; pairs the new image owns) and colv [N - n_old, N*P] (partner j - n_old, row
+// R; pairs a new image j owns) hold squared distances (squared = 1: the growth launch's minima) or distances (the refine pass).
+__global__ void __launch_bounds__(256) accumulate_weights_grow_kernel(const float* __restrict__ rowv, const float* __restrict__ colv,
+                                                                      int squared, int n_old, int nb_img, int P, double* __restrict__ S,
+                                                                      float* __restrict__ w) {
+  const long long rows = (long long)nb_img * P, Mq = (long long)(nb_img - n_old) * P;
+  const long long R = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (R >= rows) return;
+  const int i = (int)(R / P);
+  double s = (R < (long long)n_old * P) ? S[R] : 0.0;
+  for (int j = (i < n_old) ? n_old : 0; j < nb_img; ++j) {
+    if (j == i) continue;
+    const float v = pair_owned_grow(n_old, i, j, nb_img) ? __ldg(rowv + (long long)j * Mq + (R - (long long)n_old * P))
+                                                         : __ldg(colv + (long long)(j - n_old) * rows + R);
+    s += (double)(squared ? sqrtf(v) : v);
+  }
+  S[R] = s;
+  w[R] = nb_img > 1 ? (float)(s / (double)(nb_img - 1)) : nanf("");
+}
+
+extern "C" int ac_accumulate_weights_grow(const float* rowv, const float* colv, int squared, int n_old, int nb_img, int P,
+                                          double* S, float* w, ac_stream_t stream) {
+  if (!rowv || !colv || !S || !w || n_old < 0 || nb_img <= n_old || P < 1) return AC_ERR_INVALID;
+  int rc = check_device();
+  if (rc) return rc;
+  const long long rows = (long long)nb_img * P;
+  accumulate_weights_grow_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, (cudaStream_t)stream>>>(rowv, colv, squared, n_old, nb_img,
+                                                                                                     P, S, w);
+  AC_LAUNCH_CHECK();
+  return AC_OK;
 }
 
 extern "C" size_t ac_min_dist_workspace_bytes(int64_t Mq, int nb_img, int P, int D, int precision) {

@@ -23,6 +23,8 @@ namespace ac {
 static constexpr int kRQ = 4;            // query rows per block (fp32 in shared memory)
 static constexpr int kWPR = 4;           // warps per query row: they take every kWPR-th bank image of the group
 static constexpr int kRefThreads = kRQ * kWPR * 32;
+static constexpr int kRefineL2MB = 128;  // MB of bank operand rows one group keeps L2-resident (evict_last; measured at config 2
+                                         // with the policy hints: 32 / 64 / 96 / 128 / 192 / 256 MB -> 14.7 / 11.6 / 11.8 / 10.3 / 10.8 / 10.8 ms)
 
 // L2 policies: the gathered bank rows of a group (<= 96 MB) are re-read by every query chunk and must stay L2-resident while
 // the 16 KB fp32 query rows, the arg-min tables and the results stream through once per group (round-2 capture before the
@@ -54,15 +56,6 @@ __device__ __forceinline__ float4 ld_hint(const float4* p, uint64_t pol) {
   return v;
 }
 
-__host__ __device__ inline bool pair_owned_r(int i, int j, int N) {   // same rule as mindist_tc.cu: pair_owned
-  int d = j - i;
-  if (d < 0) d += N;
-  if (d == 0) return false;
-  if (2 * d < N) return true;
-  if (2 * d == N) return i < j;
-  return false;
-}
-
 struct RefineParams {
   const float* Zq;                    // [Mq, D] fp32 or null
   const void* Qhi; const void* Qlo;   // [Mq, D] operand copies (used when Zq is null)
@@ -77,6 +70,12 @@ struct RefineParams {
   const float* Bn2;                   // [nb_img*P] squared norms of the bank rows as gathered (hi, or hi + lo), or null
   float* dex;                         // [nb_img, Mq]
   int Jb;
+  // growth (ac_refine_min_dist_grow): query row r is row r0 + r of the whole category (its fp32 Z row: Zq + r*D), partners are
+  // images [jbase, nb_img); rowarg / dex [nb_img, Mn] over the Mn = (nb_img - n_old) * P new rows, colkey / dcol [nb_img - n_old,
+  // nb_img * P] over every row of the category
+  int n_old, jbase;
+  long long r0, Mn;
+  float* dcol;
 };
 
 template <typename T> __device__ __forceinline__ void unpack8(const uint4& u, float (&f)[8]);
@@ -148,7 +147,7 @@ __device__ __forceinline__ float row_dist2(const uint4* __restrict__ bh, const u
   return (a0 + a1) + (a2 + a3);
 }
 
-template <typename T, int NIT, bool LO, bool DOT>
+template <typename T, int NIT, bool LO, bool DOT, bool GROW>
 __global__ void __launch_bounds__(kRefThreads, 2) refine_kernel(const RefineParams p) {
   // query rows as fp32, split so that a lane's 8 values are two conflict-free 16-byte reads:
   // element 8g+t lives in lo4[g] (t < 4) or hi4[g] (t >= 4)
@@ -217,23 +216,34 @@ __global__ void __launch_bounds__(kRefThreads, 2) refine_kernel(const RefinePara
   const long long r = m0 + rr;
   if (r >= p.Mq) return;
   const int qi = (int)(r / p.Pq);
-  const int i = p.sym ? p.q_img0 + qi : (p.q_self ? __ldg(p.q_self + qi) : -1);
+  const long long R = p.r0 + r;                            // GROW: row of the whole category
+  const int i = GROW ? (int)(R / p.P) : (p.sym ? p.q_img0 + qi : (p.q_self ? __ldg(p.q_self + qi) : -1));
   const float4* qlo4 = s_q + (rr * 2 + 0) * G8;
   const float4* qhi4 = s_q + (rr * 2 + 1) * G8;
-  const int j0 = blockIdx.y * p.Jb, j1 = min(p.nb_img, j0 + p.Jb);
+  const int j0 = (GROW ? p.jbase : 0) + blockIdx.y * p.Jb, j1 = min(p.nb_img, j0 + p.Jb);
   // categories: only the images of the query image's own category are its bank (the rest is never read by the reduction)
   int g0 = 0, gn = p.nb_img;
   if (p.sym && p.groups) { g0 = __ldg(p.groups + 2 * i); gn = __ldg(p.groups + 2 * i + 1); }
   for (int j = j0 + par; j < j1; j += kWPR) {
-    if (j < g0 || j >= g0 + gn) continue;
-    if (j == i) {
-      if (lane == 0) p.dex[(long long)j * p.Mq + r] = 0.f;     // own image: excluded by the reduction
-      continue;
+    bool col;          // arg-min from the column minima (the partner image owns the pair)
+    long long e;
+    if (GROW) {
+      // only the pairs the growth launch computed: never two old images
+      if (j == i || (i < p.n_old && j < p.n_old)) continue;
+      col = !pair_owned_grow(p.n_old, i, j, p.nb_img);
+      e = col ? (long long)(j - p.n_old) * ((long long)p.nb_img * p.P) + R : (long long)j * p.Mn + (R - (long long)p.n_old * p.P);
+    } else {
+      if (j < g0 || j >= g0 + gn) continue;
+      if (j == i) {
+        if (lane == 0) p.dex[(long long)j * p.Mq + r] = 0.f;     // own image: excluded by the reduction
+        continue;
+      }
+      col = p.sym && !pair_owned(i - g0, j - g0, gn);
+      e = (long long)j * p.Mq + r;
     }
     int c = 0;
     if (lane == 0) {
-      const long long e = (long long)j * p.Mq + r;
-      if (p.sym && !pair_owned_r(i - g0, j - g0, gn)) c = (int)(unsigned int)(__ldg(p.colkey + e) & 0xffffffffull);
+      if (col) c = (int)(unsigned int)(__ldg(p.colkey + e) & 0xffffffffull);
       else c = __ldg(p.rowarg + e);
       c = min(max(c, 0), p.P - 1);
     }
@@ -242,36 +252,49 @@ __global__ void __launch_bounds__(kRefThreads, 2) refine_kernel(const RefinePara
     const uint4* bl = LO ? reinterpret_cast<const uint4*>(reinterpret_cast<const T*>(p.Blo) + ((long long)j * p.P + c) * p.D) : nullptr;
     float s = warp_sum(row_dist2<T, NIT, LO, DOT>(bh, bl, qlo4, qhi4, G8, lane, pol_keep));
     if (DOT) s = fmaxf(fmaf(-2.f, s, s_qn2[rr] + __ldg(p.Bn2 + (long long)j * p.P + c)), 0.f);
-    if (lane == 0) p.dex[(long long)j * p.Mq + r] = sqrtf(s);
+    if (lane == 0) (GROW && col ? p.dcol : p.dex)[e] = sqrtf(s);
   }
 }
 
-template <typename T, int NIT, bool LO, bool DOT>
+template <typename T, int NIT, bool LO, bool DOT, bool GROW>
 static int launch_refine(const RefineParams& p, dim3 grid, size_t smem, cudaStream_t st) {
-  AC_CUDA(cudaFuncSetAttribute(refine_kernel<T, NIT, LO, DOT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  refine_kernel<T, NIT, LO, DOT><<<grid, kRefThreads, smem, st>>>(p);
+  AC_CUDA(cudaFuncSetAttribute(refine_kernel<T, NIT, LO, DOT, GROW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  refine_kernel<T, NIT, LO, DOT, GROW><<<grid, kRefThreads, smem, st>>>(p);
   AC_LAUNCH_CHECK();
   return AC_OK;
 }
 
-template <typename T>
+template <typename T, bool GROW>
 static int dispatch_refine(const RefineParams& p, dim3 grid, size_t smem, cudaStream_t st) {
-  if (p.Blo) return launch_refine<T, 0, true, false>(p, grid, smem, st);      // bank given as hi + lo: generic loop
-  if (p.Bn2) {                                                                  // |q|^2 + |b|^2 - 2 q.b
-    if (p.D == 4096) return launch_refine<T, 16, false, true>(p, grid, smem, st);
-    if (p.D == 1024) return launch_refine<T, 4, false, true>(p, grid, smem, st);
-    return launch_refine<T, 0, false, true>(p, grid, smem, st);
+  if (p.Blo) return launch_refine<T, 0, true, false, GROW>(p, grid, smem, st);      // bank given as hi + lo: generic loop
+  if (p.Bn2) {                                                                        // |q|^2 + |b|^2 - 2 q.b
+    if (p.D == 4096) return launch_refine<T, 16, false, true, GROW>(p, grid, smem, st);
+    if (p.D == 1024) return launch_refine<T, 4, false, true, GROW>(p, grid, smem, st);
+    return launch_refine<T, 0, false, true, GROW>(p, grid, smem, st);
   }
-  if (p.D == 4096) return launch_refine<T, 16, false, false>(p, grid, smem, st);
-  return launch_refine<T, 0, false, false>(p, grid, smem, st);
+  if (p.D == 4096) return launch_refine<T, 16, false, false, GROW>(p, grid, smem, st);
+  return launch_refine<T, 0, false, false, GROW>(p, grid, smem, st);
+}
+
+// grid = (query chunks of kRQ rows, groups of p.Jb of the n_part partner images); p.Jb is set here
+template <bool GROW>
+static int run_refine(RefineParams& p, int op_dtype, int n_part, cudaStream_t st) {
+  const size_t smem = (size_t)kRQ * p.D * sizeof(float);
+  // bank images per group: their operand rows (kRefineL2MB, measured best on B200) stay L2-resident while every query chunk passes
+  const double img_bytes = (double)p.P * p.D * 2.0 * (p.Blo ? 2 : 1);
+  p.Jb = (int)std::max((double)kWPR, std::min(256.0, kRefineL2MB * 1.0e6 / img_bytes));
+  p.Jb -= p.Jb % kWPR;                                             // the kWPR warps of a row take every kWPR-th image
+  const long long chunks = (p.Mq + kRQ - 1) / kRQ;
+  const int nbg = (n_part + p.Jb - 1) / p.Jb;
+  if (chunks > 0x7fffffffLL || nbg > 65535) return AC_ERR_UNSUPPORTED;
+  if (chunks == 0 || nbg == 0) return AC_OK;
+  dim3 grid((unsigned)chunks, (unsigned)nbg);
+  return op_dtype == AC_DT_F16 ? dispatch_refine<__half, GROW>(p, grid, smem, st) : dispatch_refine<__nv_bfloat16, GROW>(p, grid, smem, st);
 }
 
 }  // namespace ac
 
 using namespace ac;
-
-static constexpr int kRefineL2MB = 128;  // MB of bank operand rows one group keeps L2-resident (evict_last; measured at config 2
-                                         // with the policy hints: 32 / 64 / 96 / 128 / 192 / 256 MB -> 14.7 / 11.6 / 11.8 / 10.3 / 10.8 / 10.8 ms)
 
 extern "C" int ac_refine_min_dist(const float* Zq, const void* Qhi, const void* Qlo, int64_t Mq, const void* Bhi, const void* Blo,
                                   int op_dtype, int nb_img, int P, int D, const int32_t* rowarg, const uint64_t* colkey, int sym,
@@ -288,20 +311,37 @@ extern "C" int ac_refine_min_dist(const float* Zq, const void* Qhi, const void* 
   int rc = check_device();
   if (rc) return rc;
   if (Mq == 0) return AC_OK;
-  RefineParams p;
+  RefineParams p = {};
   p.Zq = Zq; p.Qhi = Qhi; p.Qlo = Qlo; p.Bhi = Bhi; p.Blo = Blo;
   p.Mq = Mq; p.nb_img = nb_img; p.P = P; p.D = D; p.Pq = Pq;
   p.rowarg = rowarg; p.colkey = (const unsigned long long*)colkey; p.sym = sym; p.q_img0 = q_img0; p.q_self = q_self; p.dex = dmin;
   p.groups = sym ? groups : nullptr;
   p.Bn2 = Bn2;
-  // bank images per group: their operand rows (kRefineL2MB, measured best on B200) stay L2-resident while every query chunk passes
-  const double img_bytes = (double)P * D * 2.0 * (Blo ? 2 : 1);
-  p.Jb = (int)std::max((double)kWPR, std::min(256.0, kRefineL2MB * 1.0e6 / img_bytes));
-  p.Jb -= p.Jb % kWPR;                                             // the kWPR warps of a row take every kWPR-th image
-  const long long chunks = (Mq + kRQ - 1) / kRQ;
-  const int nbg = (nb_img + p.Jb - 1) / p.Jb;
-  if (chunks > 0x7fffffffLL || nbg > 65535) return AC_ERR_UNSUPPORTED;
+  return run_refine<false>(p, op_dtype, nb_img, (cudaStream_t)stream);
+}
+
+extern "C" int ac_refine_min_dist_grow(const float* Z, const void* Bhi, const void* Blo, int op_dtype, int n_old, int nb_img, int P,
+                                       int D, const int32_t* rowarg, const uint64_t* colkey, const float* Bn2, float* drow, float* dcol,
+                                       ac_stream_t stream) {
+  if (!Z || !Bhi || !rowarg || !colkey || !drow || !dcol || n_old < 0 || nb_img <= n_old || P < 1 || D < 1) return AC_ERR_INVALID;
+  if (op_dtype != AC_DT_F16 && op_dtype != AC_DT_BF16) return AC_ERR_INVALID;
+  if (D % 8 != 0) return AC_ERR_UNSUPPORTED;
+  for (const void* v : {(const void*)Z, Bhi, Blo})
+    if (reinterpret_cast<uintptr_t>(v) % 16 != 0) return AC_ERR_INVALID;
+  if ((size_t)kRQ * D * sizeof(float) > 200 * 1024) return AC_ERR_UNSUPPORTED;
+  int rc = check_device();
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  dim3 grid((unsigned)chunks, (unsigned)nbg);
-  return op_dtype == AC_DT_F16 ? dispatch_refine<__half>(p, grid, smem, st) : dispatch_refine<__nv_bfloat16>(p, grid, smem, st);
+  RefineParams p = {};
+  p.Bhi = Bhi; p.Blo = Blo; p.Bn2 = Bn2;
+  p.nb_img = nb_img; p.P = P; p.D = D; p.Pq = P;
+  p.rowarg = rowarg; p.colkey = (const unsigned long long*)colkey; p.sym = 1; p.dex = drow; p.dcol = dcol;
+  p.n_old = n_old;
+  p.Mn = (long long)(nb_img - n_old) * P;
+  // the new rows against every other image ...
+  p.r0 = (long long)n_old * P; p.Zq = Z + p.r0 * D; p.Mq = p.Mn; p.jbase = 0;
+  if ((rc = run_refine<true>(p, op_dtype, nb_img, st))) return rc;
+  // ... and the old rows against the new images only: the cost follows the number of new pairs
+  p.r0 = 0; p.Zq = Z; p.Mq = (long long)n_old * P; p.jbase = n_old;
+  return run_refine<true>(p, op_dtype, nb_img - n_old, st);
 }

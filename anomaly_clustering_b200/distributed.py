@@ -40,6 +40,16 @@ def pair_owned(i: int, j: int, n: int) -> bool:
     return False
 
 
+def pair_owned_grow(n_old: int, i: int, j: int, n: int) -> bool:
+    """Host mirror of the growth ownership rule (csrc/common.cuh: pair_owned_grow): images [n_old, n) join images [0, n_old); a
+    new image owns its pairs with the old ones, two new images follow pair_owned among the new, two old images have no owner."""
+    if i < n_old:
+        return False
+    if j < n_old:
+        return True
+    return pair_owned(i - n_old, j - n_old, n - n_old)
+
+
 def shard_bounds(n_items: int, world: int) -> List[Tuple[int, int]]:
     """Contiguous, balanced slices: the first n % world ranks get one extra item."""
     base, extra = divmod(n_items, world)

@@ -307,6 +307,70 @@ def min_dist_sym_arg(Qhi, Qlo, Qn2, q_img0: int, Bhi, Blo, Bn2, nb_img: int, P: 
     return rowmin, rowarg, colkey
 
 
+def min_dist_sym_grow(hi, lo, n2, n_old: int, nb_img: int, P: int, precision: str, arg: bool = False):
+    """ac_min_dist_sym_grow: the new pairs of a category whose images [n_old, nb_img) have just joined images [0, n_old).
+    hi / lo / n2 are the operands and norms of all nb_img images (new ones last); the query window is the new images.
+    Returns (rowmin_d2 [nb_img, M*P], colmin_d2 [M, nb_img*P]) or, arg=True, (rowmin_d2, rowarg, colkey [M, nb_img*P] int64)."""
+    lib = _lib.load()
+    _need_cuda(hi, n2)
+    prec = _lib.PRECISIONS[precision]
+    D = hi.shape[1]
+    assert hi.shape == (nb_img * P, D) and hi.is_contiguous() and n2.shape == (nb_img * P,)
+    assert lo is None or (lo.shape == hi.shape and lo.is_contiguous())
+    q0 = n_old * P
+    Mq = nb_img * P - q0
+    dev = hi.device
+    rowmin = torch.empty(nb_img, Mq, dtype=torch.float32, device=dev)
+    rowarg = colmin = colkey = None
+    if arg:
+        rowarg = torch.zeros(nb_img, Mq, dtype=torch.int32, device=dev)
+        colkey = torch.empty(Mq // P, nb_img * P, dtype=torch.int64, device=dev)
+    else:
+        colmin = torch.empty(Mq // P, nb_img * P, dtype=torch.float32, device=dev)
+    ws_bytes = lib.ac_min_dist_workspace_bytes(Mq, nb_img, P, D, prec)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    rc = lib.ac_min_dist_sym_grow(_ptr(hi[q0:]), _ptr(None if lo is None else lo[q0:]), _ptr(n2[q0:]), Mq, n_old, _ptr(hi), _ptr(lo),
+                                  _ptr(n2), nb_img, P, D, prec, 0, nb_img, 1, _ptr(rowmin), _ptr(colmin), _ptr(rowarg), _ptr(colkey),
+                                  None, int(n_old), _ptr(ws), ws_bytes, _stream())
+    check(rc, "ac_min_dist_sym_grow")
+    return (rowmin, rowarg, colkey) if arg else (rowmin, colmin)
+
+
+def refine_min_dist_grow(Z: torch.Tensor, hi, lo, n2, n_old: int, nb_img: int, P: int, rowarg: torch.Tensor, colkey: torch.Tensor):
+    """ac_refine_min_dist_grow: exact fp32 distances of the new pairs of one growth launch, (drow [nb_img, M*P],
+    dcol [M, nb_img*P]) in the layouts of its minima.  Z [nb_img*P, D] fp32 of every image of the category."""
+    lib = _lib.load()
+    _need_cuda(Z, hi, rowarg, colkey)
+    D = hi.shape[1]
+    Mq = (nb_img - n_old) * P
+    assert Z.shape == (nb_img * P, D) and Z.dtype == torch.float32 and Z.is_contiguous()
+    assert hi.shape == (nb_img * P, D) and hi.is_contiguous()
+    assert rowarg.shape == (nb_img, Mq) and rowarg.dtype == torch.int32 and rowarg.is_contiguous()
+    assert colkey.shape == (nb_img - n_old, nb_img * P) and colkey.dtype == torch.int64 and colkey.is_contiguous()
+    drow = torch.empty(nb_img, Mq, dtype=torch.float32, device=hi.device)
+    dcol = torch.empty(nb_img - n_old, nb_img * P, dtype=torch.float32, device=hi.device)
+    rc = lib.ac_refine_min_dist_grow(_ptr(Z), _ptr(hi), _ptr(lo), _TORCH_TO_AC[hi.dtype], int(n_old), nb_img, P, D, _ptr(rowarg),
+                                     _ptr(colkey), _ptr(n2), _ptr(drow), _ptr(dcol), _stream())
+    check(rc, "ac_refine_min_dist_grow")
+    return drow, dcol
+
+
+def accumulate_weights_grow(rowv: torch.Tensor, colv: torch.Tensor, squared: bool, n_old: int, nb_img: int, P: int,
+                            S: torch.Tensor) -> torch.Tensor:
+    """ac_accumulate_weights_grow: adds the new pairs of one growth launch to the fp64 running sums S [>= nb_img*P] (in place)
+    and returns w [nb_img*P] fp32 for every row of the category."""
+    lib = _lib.load()
+    _need_cuda(rowv, colv, S)
+    Mq = (nb_img - n_old) * P
+    assert rowv.shape == (nb_img, Mq) and colv.shape == (nb_img - n_old, nb_img * P)
+    assert rowv.dtype == colv.dtype == torch.float32 and rowv.is_contiguous() and colv.is_contiguous()
+    assert S.dtype == torch.float64 and S.is_contiguous() and S.numel() >= nb_img * P
+    w = torch.empty(nb_img * P, dtype=torch.float32, device=rowv.device)
+    check(lib.ac_accumulate_weights_grow(_ptr(rowv), _ptr(colv), int(bool(squared)), int(n_old), nb_img, P, _ptr(S), _ptr(w), _stream()),
+          "ac_accumulate_weights_grow")
+    return w
+
+
 def refine_min_dist(Zq: Optional[torch.Tensor], Qhi, Qlo, Bhi, Blo, nb_img: int, P: int, rowarg: torch.Tensor,
                     colkey: Optional[torch.Tensor] = None, q_img0: int = 0, q_self: Optional[torch.Tensor] = None,
                     Pq: Optional[int] = None, groups: Optional[torch.Tensor] = None, Bn2: Optional[torch.Tensor] = None) -> torch.Tensor:

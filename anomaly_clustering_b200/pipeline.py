@@ -373,3 +373,122 @@ def run_categories(
                               taus=list(taus), grid=q.grid))
         start += n
     return out
+
+
+class GrowingCategory:
+    """One unsupervised category that gains images over time (an inspection line collecting defective images), clustered
+    after every addition without recomputing the image pairs it already has.
+
+    w[i, p] is a mean over the other images of one per-image minimum each (utils.py:222-227), so when M images join N_old
+    the old pairs keep their minima: `add` runs the distance pass over the M*N_old + M*(M-1)/2 new pairs only
+    (ac_min_dist_sym_grow), adds them to fp64 running sums kept per patch row (ac_accumulate_weights_grow) and runs stage 3 for
+    every image so far, which does change everywhere because every w does.  The result of each `add` is what `run_path`
+    returns for all images so far, up to the order of the sums (DESIGN.md section 5c).
+
+    Device state: the tensor-core operands and their norms, the running sums, and the source of X: the fp32 Z when keep_z or
+    a refined precision (whose exact re-evaluation reads it) is in use, else the hooked feature maps as they came in (fp32,
+    bf16 or fp16), from which ac_weighted_embed_from_features computes X exactly as `run_path` does.  Buffers hold `capacity`
+    images (default: the first addition) and double when full."""
+
+    def __init__(self, patchsize: int, stride: int, pretrain_dim: int, target_dim: int, taus: Sequence[float],
+                 precision: str = "auto", keep_z: bool = False, layernorm: bool = True, capacity: Optional[int] = None):
+        self.patchsize, self.stride, self.pretrain_dim, self.target_dim = patchsize, stride, pretrain_dim, target_dim
+        self.taus = [float(t) for t in taus]
+        self.precision = resolve_precision(precision, self.taus)
+        if self.precision not in _OPERAND_OF or self.precision == "f32":
+            raise ValueError("growth needs a tensor-core precision (f16, bf16, f16x3, bf16x3, f16r, bf16r), got %r" % self.precision)
+        self.refined = self.precision in REFINED
+        self.keep_z = keep_z or self.refined
+        self.layernorm = layernorm
+        self.capacity = int(capacity) if capacity else 0
+        self.n_img = 0
+        self._sig = None
+        self.P = 0
+        self.grid = (0, 0)
+        self._hi = self._lo = self._n2 = self._S = self._Z = None
+        self._feats: List[torch.Tensor] = []
+
+    def _signature(self, features) -> tuple:
+        return (len(features), tuple(tuple(f.shape[1:]) for f in features), features[0].dtype)
+
+    def _reserve(self, n: int, features) -> None:
+        """Room for n images in every device buffer: the capacity doubles (at least) and the rows of the images so far are
+        copied over on the current stream."""
+        if self._hi is not None and n <= self.capacity:
+            return
+        cap = max(n, 2 * self.capacity) if self._hi is not None else max(n, self.capacity)
+        P, D, n_old, dev = self.P, self.target_dim, self.n_img, features[0].device
+        operand, want_lo = _OPERAND_OF[self.precision]
+        tdt = torch.float16 if operand == "f16" else torch.bfloat16
+
+        def grown(old, per_img, shape, dtype):       # per_img: leading-axis entries per image
+            t = torch.empty((cap * per_img,) + tuple(shape), dtype=dtype, device=dev)
+            if old is not None and n_old:
+                t[:n_old * per_img].copy_(old[:n_old * per_img])
+            return t
+
+        self._hi = grown(self._hi, P, (D,), tdt)
+        self._lo = grown(self._lo, P, (D,), tdt) if want_lo else None
+        self._n2 = grown(self._n2, P, (), torch.float32)
+        self._S = grown(self._S, P, (), torch.float64)
+        if self.keep_z:
+            self._Z = grown(self._Z, P, (D,), torch.float32)
+        else:
+            olds = self._feats or [None] * len(features)
+            self._feats = [grown(old, 1, f.shape[1:], f.dtype) for old, f in zip(olds, features)]
+        self.capacity = cap
+
+    def add(self, features: Sequence[torch.Tensor]) -> PathResult:
+        """Embeds the new images (hooked features, device tensors of the layout run_path takes), multiplies only the pairs they
+        bring and returns the PathResult of all images so far."""
+        features = list(features)
+        sig = self._signature(features)
+        if self._sig is None:
+            if features[0].shape[0] < 2:
+                raise ValueError("the first add needs at least 2 images")
+            if not self.keep_z and not z_free_supported(features, self.patchsize, self.stride, self.pretrain_dim, self.target_dim,
+                                                        self.precision):
+                self.keep_z = True
+            v0 = ops.feature_view(features[0])
+            self.grid = ops.patch_grid(v0.shape[2], v0.shape[3], self.patchsize, self.stride)
+            self.P = self.grid[0] * self.grid[1]
+            if self.P < 32:
+                raise ValueError("growth runs the symmetric distance form, which needs at least 32 patches per image")
+            self._sig = sig
+        elif sig != self._sig:
+            raise ValueError("features of shape / dtype %s differ from the first add's %s" % (sig, self._sig))
+        M = features[0].shape[0]
+        if M < 1 or any(f.shape[0] != M for f in features):
+            raise ValueError("every layer must hold the same, non-zero number of images")
+        n_old, N, P, D = self.n_img, self.n_img + M, self.P, self.target_dim
+        self._reserve(N, features)
+        rows = slice(n_old * P, N * P)
+        operand, want_lo = _OPERAND_OF[self.precision]
+        need_z = self.keep_z or not _fusable(len(features), self.pretrain_dim, self.target_dim)
+        _mark("embed_begin")
+        ops.embed(features, self.patchsize, self.stride, self.pretrain_dim, self.target_dim, layernorm=self.layernorm, want_z=need_z,
+                  operand=operand, want_lo=want_lo, out_z=self._Z[rows] if self.keep_z else None, out_hi=self._hi[rows],
+                  out_lo=None if self._lo is None else self._lo[rows], out_n2=self._n2[rows])
+        if not self.keep_z:
+            for buf, f in zip(self._feats, features):
+                buf[n_old:N].copy_(f)
+        _mark("embed_end")
+        hi, lo, n2 = self._hi[:N * P], None if self._lo is None else self._lo[:N * P], self._n2[:N * P]
+        Z = self._Z[:N * P] if self.keep_z else None
+        _mark("mindist_begin")
+        if self.refined:
+            _, rowarg, colkey = ops.min_dist_sym_grow(hi, lo, n2, n_old, N, P, self.precision, arg=True)
+            _mark("mindist_end")
+            _mark("refine_begin")
+            rowv, colv = ops.refine_min_dist_grow(Z, hi, lo, n2, n_old, N, P, rowarg, colkey)
+            _mark("refine_end")
+        else:
+            rowv, colv = ops.min_dist_sym_grow(hi, lo, n2, n_old, N, P, self.precision)
+            _mark("mindist_end")
+        w = ops.accumulate_weights_grow(rowv, colv, not self.refined, n_old, N, P, self._S).reshape(N, P)
+        self.n_img = N
+        ps = PatchSet(n_img=N, P=P, D=D, grid=self.grid, Z=Z, hi=hi, lo=lo, n2=n2)
+        feats = None if self.keep_z else [buf[:N] for buf in self._feats]
+        a64, a32, X, Dm = alpha_X_dist(ps, w, self.taus, feats, (self.patchsize, self.stride, self.pretrain_dim, self.layernorm))
+        return PathResult(Z=None if Z is None else Z.reshape(N, P, D), w=w, alpha64=a64, alpha32=a32, X=X, Dmat=Dm,
+                          taus=list(self.taus), grid=self.grid)

@@ -246,6 +246,37 @@ int ac_min_dist_sym_ready(const void* Qhi, const void* Qlo, const float* Qn2, in
                           const int32_t* groups, const int32_t* bank_ready, void* ws, size_t ws_bytes, ac_stream_t stream);
 int ac_reduce_weights_sym_ex(const float* rowmin_d2, const float* colmin_d2, int64_t Mq, int nb_img, int Pq, int q_img0,
                              const int32_t* groups, float* w, ac_stream_t stream);
+
+/* ---- growing an unsupervised category ---------------------------------------------------------------
+ * w[r] of Weight_Distance_Unsupervised (utils.py:222-227) is a MEAN over the other images of one per-image minimum each, so when
+ * M images join N_old images only the M*N_old + M*(M-1)/2 new image pairs need the distance pass.  The bank is the
+ * nb_img = N_old + M images stored contiguously (new ones last), the query window is the new images (q_img0 = n_old,
+ * Mq = M*P), and ownership is
+ *   new image i, old image j:  i owns {i, j};
+ *   two new images:            pair_owned among the new images (the rule of ac_min_dist_sym with N = M);
+ *   two old images:            never visited.
+ * n_old = 0 is exactly ac_min_dist_sym_ex (the same units, the same bits).  Outputs and every other argument as
+ * ac_min_dist_sym_ex: rowmin_d2 [nb_img, Mq], colmin_d2 (or colkey) [M, nb_img*P], rowarg / colkey for the refined precisions.
+ * groups must be NULL (AC_ERR_UNSUPPORTED); q_img0 != n_old or Mq != (nb_img - n_old)*P: AC_ERR_INVALID. */
+int ac_min_dist_sym_grow(const void* Qhi, const void* Qlo, const float* Qn2, int64_t Mq, int q_img0, const void* Bhi,
+                         const void* Blo, const float* Bn2, int nb_img, int P, int D, int precision, int bank_begin,
+                         int bank_count, int init, float* rowmin_d2, float* colmin_d2, int32_t* rowarg, uint64_t* colkey,
+                         const int32_t* groups, int n_old, void* ws, size_t ws_bytes, ac_stream_t stream);
+/* Exact fp32 re-evaluation (as ac_refine_min_dist) of the NEW pairs of one growth launch only: the new rows against every other
+ * image, arg from rowarg where the new image owns the pair, else from colkey; the old rows against the new images, arg from
+ * colkey.  Z [nb_img*P, D] fp32 is the whole category (each row's own Z); Bhi / Blo / Bn2 its operands as for the launch.
+ * drow [nb_img, M*P] receives the distances of the pairs the new row's image owns, dcol [M, nb_img*P] those of the pairs a
+ * new image j owns (row R of the category at dcol[(j - n_old)*nb_img*P + R]); entries of other pairs are left untouched. */
+int ac_refine_min_dist_grow(const float* Z, const void* Bhi, const void* Blo, int op_dtype, int n_old, int nb_img, int P, int D,
+                            const int32_t* rowarg, const uint64_t* colkey, const float* Bn2, float* drow, float* dcol,
+                            ac_stream_t stream);
+/* Running sums of the category: S [nb_img*P] fp64, S[R] += d(R, j) over the new pairs of row R (old rows: the M new images;
+ * new rows: every other image), partner images in increasing order; then w[R] = float(S[R] / (nb_img - 1)) for every row.
+ * Rows of new images start from 0, rows of old ones from S as left by the previous update.  rowv / colv in the layouts of
+ * drow / dcol above: squared = 1 for the squared minima of ac_min_dist_sym_grow, 0 for the distances of
+ * ac_refine_min_dist_grow.  The order of addition is fixed by the data, so the result does not depend on the launch geometry. */
+int ac_accumulate_weights_grow(const float* rowv, const float* colv, int squared, int n_old, int nb_img, int P, double* S,
+                               float* w, ac_stream_t stream);
 int ac_reduce_weights_ex(const float* dmin, int64_t Mq, int nb_img, int Pq, const int32_t* q_self, const int32_t* groups,
                          int mode, float* w, ac_stream_t stream);
 
