@@ -18,7 +18,7 @@ AC_OK = 0
 AC_ERR_INVALID, AC_ERR_UNSUPPORTED, AC_ERR_DEVICE, AC_ERR_CUDA, AC_ERR_WORKSPACE = -1, -2, -3, -4, -5
 AC_DT_F32, AC_DT_F16, AC_DT_BF16 = 0, 1, 2
 AC_PREC_F16, AC_PREC_BF16, AC_PREC_F16X3, AC_PREC_BF16X3, AC_PREC_F32 = 0, 1, 2, 3, 4
-AC_REDUCE_MEAN, AC_REDUCE_MIN = 0, 1
+AC_REDUCE_MEAN, AC_REDUCE_MIN, AC_REDUCE_MIN_UPDATE = 0, 1, 2
 
 PRECISIONS = {"f16": AC_PREC_F16, "bf16": AC_PREC_BF16, "f16x3": AC_PREC_F16X3, "bf16x3": AC_PREC_BF16X3, "f32": AC_PREC_F32,
               # "r" modes: one tensor-core pass that also records the arg-min + exact fp32 re-evaluation (ac_refine_min_dist)

@@ -2,7 +2,7 @@
 // image-to-image Euclidean matrix.  All HBM-bound and tiny next to the distance GEMM.
 //
 // Reference lines replaced:
-//   ac_reduce_weights  models/patchcore/utils.py:227 (mean over j != i) / :236 (min over j)
+//   ac_reduce_weights  models/patchcore/utils.py:227 (mean over j != i) / :236 (min over j; MIN_UPDATE lowers a running min)
 //   ac_alpha           models/patchcore/utils.py:246-255, 266-275
 //   ac_weighted_embed  examples/main.py:294-296
 //   ac_pairwise_l2     examples/test.py:193-195 (Ward's internal pdist)
@@ -45,7 +45,8 @@ __global__ void __launch_bounds__(256) reduce_weights_kernel(const float* __rest
     }
     w[r] = cnt > 0 ? s / (float)cnt : nanf("");
   } else {
-    float m = INFINITY;
+    // AC_REDUCE_MIN_UPDATE lowers the running minimum w holds; a min of fp32 values does not depend on the order it is taken in
+    float m = mode == AC_REDUCE_MIN_UPDATE ? w[r] : INFINITY;
     for (int j = j0; j < j1; ++j) {
       if (j == self) continue;
       m = fminf(m, __ldg(dmin + (long long)j * Mq + r));
@@ -297,7 +298,7 @@ extern "C" int ac_device_ok(int dev) {
 extern "C" int ac_reduce_weights_ex(const float* dmin, int64_t Mq, int nb_img, int Pq, const int32_t* q_self, const int32_t* groups,
                                     int mode, float* w, ac_stream_t stream) {
   if (!dmin || !w || Mq < 0 || nb_img < 1 || Pq < 1) return AC_ERR_INVALID;
-  if (mode != AC_REDUCE_MEAN && mode != AC_REDUCE_MIN) return AC_ERR_INVALID;
+  if (mode != AC_REDUCE_MEAN && mode != AC_REDUCE_MIN && mode != AC_REDUCE_MIN_UPDATE) return AC_ERR_INVALID;
   if (groups && !q_self) return AC_ERR_INVALID;
   int rc = check_device();
   if (rc) return rc;

@@ -413,14 +413,24 @@ def reduce_weights_sym(rowmin: torch.Tensor, colfull: torch.Tensor, Pq: int, q_i
     return w
 
 
+_REDUCE_MODES = {"mean": _lib.AC_REDUCE_MEAN, "min": _lib.AC_REDUCE_MIN, "min_update": _lib.AC_REDUCE_MIN_UPDATE}
+
+
 def reduce_weights(dmin: torch.Tensor, Pq: int, q_self: Optional[torch.Tensor], mode: str,
-                   groups: Optional[torch.Tensor] = None) -> torch.Tensor:
+                   groups: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """ac_reduce_weights_ex: w [Mq] from dmin [nb_img, Mq].  mode 'mean' | 'min' | 'min_update'; 'min_update' lowers the running
+    minimum held in `out` in place.  `out` (contiguous fp32 [Mq] on dmin's device) receives w, else a new tensor does."""
+    if mode not in _REDUCE_MODES:
+        raise ValueError("reduce mode must be one of %s, got %r" % (sorted(_REDUCE_MODES), mode))
+    if out is None and mode == "min_update":
+        raise ValueError("mode 'min_update' updates the running minimum passed as out=")
     lib = _lib.load()
-    _need_cuda(dmin, q_self)
+    _need_cuda(dmin, q_self, out)
     nb_img, Mq = dmin.shape
     _groups_ok(groups, nb_img)
-    w = torch.empty(Mq, dtype=torch.float32, device=dmin.device)
-    m = _lib.AC_REDUCE_MEAN if mode == "mean" else _lib.AC_REDUCE_MIN
+    _out_ok(out, "out", (Mq,), torch.float32, dmin.device)
+    w = out if out is not None else torch.empty(Mq, dtype=torch.float32, device=dmin.device)
+    m = _REDUCE_MODES[mode]
     if q_self is not None:
         assert q_self.dtype == torch.int32 and q_self.numel() * Pq >= Mq
     check(lib.ac_reduce_weights_ex(_ptr(dmin), Mq, nb_img, Pq, _ptr(q_self), _ptr(groups), m, _ptr(w), _stream()), "ac_reduce_weights")

@@ -375,6 +375,90 @@ def run_categories(
     return out
 
 
+def _growth_precision(precision: str, taus: Sequence[float]) -> str:
+    """The precision of a growing category, resolved once from its taus; growth multiplies on the tensor cores only."""
+    precision = resolve_precision(precision, taus)
+    if precision not in _OPERAND_OF or precision == "f32":
+        raise ValueError("growth needs a tensor-core precision (f16, bf16, f16x3, bf16x3, f16r, bf16r), got %r" % precision)
+    return precision
+
+
+def _feature_signature(features, first: Optional[tuple]) -> tuple:
+    """(layer count, per-layer shape without the image axis, dtype) of one call's hooked features; every later call of a
+    growing category must repeat the first call's."""
+    sig = (len(features), tuple(tuple(f.shape[1:]) for f in features), features[0].dtype)
+    if first is not None and sig != first:
+        raise ValueError("features of shape / dtype %s differ from the first add's %s" % (sig, first))
+    return sig
+
+
+def _image_count(features) -> int:
+    M = features[0].shape[0]
+    if M < 1 or any(f.shape[0] != M for f in features):
+        raise ValueError("every layer must hold the same, non-zero number of images")
+    return M
+
+
+def _regrow(old: Optional[torch.Tensor], n_keep: int, shape, dtype, dev, dim: int = 0) -> torch.Tensor:
+    """A new buffer of `shape` holding the first n_keep entries of `old` along `dim`, copied on the current stream."""
+    t = torch.empty(tuple(shape), dtype=dtype, device=dev)
+    if old is not None and n_keep:
+        t.narrow(dim, 0, n_keep).copy_(old.narrow(dim, 0, n_keep))
+    return t
+
+
+class _GrowingImages:
+    """Embedded images that gain more over time: the tensor-core operands and their squared norms, plus the fp32 Z (keep_z)
+    or the hooked feature maps as they came in (keep_maps: the source of the Z-free X).  Buffers hold `capacity` images
+    (0: the first addition) and double when full; the rows of the images so far are copied over on the current stream."""
+
+    def __init__(self, precision: str, P: int, D: int, keep_z: bool, keep_maps: bool, capacity: int):
+        self.precision, self.P, self.D, self.keep_z, self.keep_maps = precision, P, D, keep_z, keep_maps
+        self.capacity = capacity
+        self.n_img = 0
+        self.hi = self.lo = self.n2 = self.Z = None
+        self.maps: List[torch.Tensor] = []
+
+    def _reserve(self, n: int, features) -> None:
+        if self.hi is not None and n <= self.capacity:
+            return
+        cap = max(n, 2 * self.capacity) if self.hi is not None else max(n, self.capacity)
+        P, D, rows, dev = self.P, self.D, self.n_img * self.P, features[0].device
+        operand, want_lo = _OPERAND_OF[self.precision]
+        tdt = torch.float16 if operand == "f16" else torch.bfloat16
+        self.hi = _regrow(self.hi, rows, (cap * P, D), tdt, dev)
+        self.lo = _regrow(self.lo, rows, (cap * P, D), tdt, dev) if want_lo else None
+        self.n2 = _regrow(self.n2, rows, (cap * P,), torch.float32, dev)
+        if self.keep_z:
+            self.Z = _regrow(self.Z, rows, (cap * P, D), torch.float32, dev)
+        if self.keep_maps:
+            olds = self.maps or [None] * len(features)
+            self.maps = [_regrow(old, self.n_img, (cap,) + tuple(f.shape[1:]), f.dtype, dev) for old, f in zip(olds, features)]
+        self.capacity = cap
+
+    def append(self, features, patchsize: int, stride: int, pretrain_dim: int, layernorm: bool) -> None:
+        """Embeds the new images (one ac_embed_dt call) into the rows after the images so far."""
+        n_old, N, P = self.n_img, self.n_img + features[0].shape[0], self.P
+        self._reserve(N, features)
+        rows = slice(n_old * P, N * P)
+        operand, want_lo = _OPERAND_OF[self.precision]
+        need_z = self.keep_z or not _fusable(len(features), pretrain_dim, self.D)
+        _mark("embed_begin")
+        ops.embed(features, patchsize, stride, pretrain_dim, self.D, layernorm=layernorm, want_z=need_z, operand=operand,
+                  want_lo=want_lo, out_z=self.Z[rows] if self.keep_z else None, out_hi=self.hi[rows],
+                  out_lo=None if self.lo is None else self.lo[rows], out_n2=self.n2[rows])
+        for buf, f in zip(self.maps, features):
+            buf[n_old:N].copy_(f)
+        _mark("embed_end")
+        self.n_img = N
+
+    def patchset(self, i0: int, i1: int, grid) -> PatchSet:
+        """Images [i0, i1) as views into the buffers."""
+        rows = slice(i0 * self.P, i1 * self.P)
+        return PatchSet(n_img=i1 - i0, P=self.P, D=self.D, grid=grid, Z=self.Z[rows] if self.keep_z else None, hi=self.hi[rows],
+                        lo=None if self.lo is None else self.lo[rows], n2=self.n2[rows])
+
+
 class GrowingCategory:
     """One unsupervised category that gains images over time (an inspection line collecting defective images), clustered
     after every addition without recomputing the image pairs it already has.
@@ -394,55 +478,30 @@ class GrowingCategory:
                  precision: str = "auto", keep_z: bool = False, layernorm: bool = True, capacity: Optional[int] = None):
         self.patchsize, self.stride, self.pretrain_dim, self.target_dim = patchsize, stride, pretrain_dim, target_dim
         self.taus = [float(t) for t in taus]
-        self.precision = resolve_precision(precision, self.taus)
-        if self.precision not in _OPERAND_OF or self.precision == "f32":
-            raise ValueError("growth needs a tensor-core precision (f16, bf16, f16x3, bf16x3, f16r, bf16r), got %r" % self.precision)
+        self.precision = _growth_precision(precision, self.taus)
         self.refined = self.precision in REFINED
         self.keep_z = keep_z or self.refined
         self.layernorm = layernorm
-        self.capacity = int(capacity) if capacity else 0
-        self.n_img = 0
+        self._capacity = int(capacity) if capacity else 0
         self._sig = None
         self.P = 0
         self.grid = (0, 0)
-        self._hi = self._lo = self._n2 = self._S = self._Z = None
-        self._feats: List[torch.Tensor] = []
+        self._images: Optional[_GrowingImages] = None
+        self._S = None
 
-    def _signature(self, features) -> tuple:
-        return (len(features), tuple(tuple(f.shape[1:]) for f in features), features[0].dtype)
+    @property
+    def n_img(self) -> int:
+        return self._images.n_img if self._images is not None else 0
 
-    def _reserve(self, n: int, features) -> None:
-        """Room for n images in every device buffer: the capacity doubles (at least) and the rows of the images so far are
-        copied over on the current stream."""
-        if self._hi is not None and n <= self.capacity:
-            return
-        cap = max(n, 2 * self.capacity) if self._hi is not None else max(n, self.capacity)
-        P, D, n_old, dev = self.P, self.target_dim, self.n_img, features[0].device
-        operand, want_lo = _OPERAND_OF[self.precision]
-        tdt = torch.float16 if operand == "f16" else torch.bfloat16
-
-        def grown(old, per_img, shape, dtype):       # per_img: leading-axis entries per image
-            t = torch.empty((cap * per_img,) + tuple(shape), dtype=dtype, device=dev)
-            if old is not None and n_old:
-                t[:n_old * per_img].copy_(old[:n_old * per_img])
-            return t
-
-        self._hi = grown(self._hi, P, (D,), tdt)
-        self._lo = grown(self._lo, P, (D,), tdt) if want_lo else None
-        self._n2 = grown(self._n2, P, (), torch.float32)
-        self._S = grown(self._S, P, (), torch.float64)
-        if self.keep_z:
-            self._Z = grown(self._Z, P, (D,), torch.float32)
-        else:
-            olds = self._feats or [None] * len(features)
-            self._feats = [grown(old, 1, f.shape[1:], f.dtype) for old, f in zip(olds, features)]
-        self.capacity = cap
+    @property
+    def capacity(self) -> int:
+        return self._images.capacity if self._images is not None else self._capacity
 
     def add(self, features: Sequence[torch.Tensor]) -> PathResult:
         """Embeds the new images (hooked features, device tensors of the layout run_path takes), multiplies only the pairs they
         bring and returns the PathResult of all images so far."""
         features = list(features)
-        sig = self._signature(features)
+        sig = _feature_signature(features, self._sig)
         if self._sig is None:
             if features[0].shape[0] < 2:
                 raise ValueError("the first add needs at least 2 images")
@@ -455,26 +514,16 @@ class GrowingCategory:
             if self.P < 32:
                 raise ValueError("growth runs the symmetric distance form, which needs at least 32 patches per image")
             self._sig = sig
-        elif sig != self._sig:
-            raise ValueError("features of shape / dtype %s differ from the first add's %s" % (sig, self._sig))
-        M = features[0].shape[0]
-        if M < 1 or any(f.shape[0] != M for f in features):
-            raise ValueError("every layer must hold the same, non-zero number of images")
+        M = _image_count(features)
         n_old, N, P, D = self.n_img, self.n_img + M, self.P, self.target_dim
-        self._reserve(N, features)
-        rows = slice(n_old * P, N * P)
-        operand, want_lo = _OPERAND_OF[self.precision]
-        need_z = self.keep_z or not _fusable(len(features), self.pretrain_dim, self.target_dim)
-        _mark("embed_begin")
-        ops.embed(features, self.patchsize, self.stride, self.pretrain_dim, self.target_dim, layernorm=self.layernorm, want_z=need_z,
-                  operand=operand, want_lo=want_lo, out_z=self._Z[rows] if self.keep_z else None, out_hi=self._hi[rows],
-                  out_lo=None if self._lo is None else self._lo[rows], out_n2=self._n2[rows])
-        if not self.keep_z:
-            for buf, f in zip(self._feats, features):
-                buf[n_old:N].copy_(f)
-        _mark("embed_end")
-        hi, lo, n2 = self._hi[:N * P], None if self._lo is None else self._lo[:N * P], self._n2[:N * P]
-        Z = self._Z[:N * P] if self.keep_z else None
+        if self._images is None:
+            self._images = _GrowingImages(self.precision, P, D, self.keep_z, not self.keep_z, self._capacity)
+        images = self._images
+        images.append(features, self.patchsize, self.stride, self.pretrain_dim, self.layernorm)
+        if self._S is None or self._S.numel() < images.capacity * P:
+            self._S = _regrow(self._S, n_old * P, (images.capacity * P,), torch.float64, features[0].device)
+        ps = images.patchset(0, N, self.grid)
+        hi, lo, n2, Z = ps.hi, ps.lo, ps.n2, ps.Z
         _mark("mindist_begin")
         if self.refined:
             _, rowarg, colkey = ops.min_dist_sym_grow(hi, lo, n2, n_old, N, P, self.precision, arg=True)
@@ -486,9 +535,152 @@ class GrowingCategory:
             rowv, colv = ops.min_dist_sym_grow(hi, lo, n2, n_old, N, P, self.precision)
             _mark("mindist_end")
         w = ops.accumulate_weights_grow(rowv, colv, not self.refined, n_old, N, P, self._S).reshape(N, P)
-        self.n_img = N
-        ps = PatchSet(n_img=N, P=P, D=D, grid=self.grid, Z=Z, hi=hi, lo=lo, n2=n2)
-        feats = None if self.keep_z else [buf[:N] for buf in self._feats]
+        feats = None if self.keep_z else [buf[:N] for buf in images.maps]
         a64, a32, X, Dm = alpha_X_dist(ps, w, self.taus, feats, (self.patchsize, self.stride, self.pretrain_dim, self.layernorm))
         return PathResult(Z=None if Z is None else Z.reshape(N, P, D), w=w, alpha64=a64, alpha32=a32, X=X, Dmat=Dm,
                           taus=list(self.taus), grid=self.grid)
+
+
+# query rows per block of the refine kernel (kRQ in csrc/refine.cu).  Unless D is a multiple of 256, the lanes that sum a query
+# row's |q|^2 there depend on the row's place in its block, so a refine launch over new query rows starts on a multiple of it,
+# as run_path's launch from row 0 does.
+_REFINE_QUERY_ROWS = 4
+
+
+class GrowingSupervisedCategory:
+    """One supervised category whose query images and normal bank both grow over time (an inspection line clustering its
+    defects against known-good images), clustered after every call without recomputing the image pairs it already has.
+
+    w[r] of Weight_Distance_Supervised (utils.py:230-237) is a minimum over bank images of one per-(row, bank image) minimum
+    each, and a min of fp32 values does not depend on the order it is taken in.  So `add` runs the new query rows against the
+    whole bank and leaves the old queries' w, alpha and X alone; `add_normal` runs every query row against the new bank images
+    only and lowers w in place (ac_reduce_weights, AC_REDUCE_MIN_UPDATE), then runs stage 3 for every query.  Each result is
+    bit-identical to `run_path(queries so far, mode="supervised", bank_features=normals so far)` (DESIGN.md section 5d).
+
+    Device state: for the queries the tensor-core operands and their norms, w, alpha64 / alpha32 / X per tau and the source of X
+    (the fp32 Z when keep_z or a refined precision is in use, else the hooked feature maps as they came in); for the bank the
+    operands and norms only.  Buffers hold `capacity` query / `bank_capacity` bank images (default: the first addition) and
+    double when full.  Both sides must give the features of the first call's layer count, shapes and dtype."""
+
+    def __init__(self, patchsize: int, stride: int, pretrain_dim: int, target_dim: int, taus: Sequence[float],
+                 precision: str = "auto", keep_z: bool = False, layernorm: bool = True, capacity: Optional[int] = None,
+                 bank_capacity: Optional[int] = None):
+        self.patchsize, self.stride, self.pretrain_dim, self.target_dim = patchsize, stride, pretrain_dim, target_dim
+        self.taus = [float(t) for t in taus]
+        self.precision = _growth_precision(precision, self.taus)
+        self.refined = self.precision in REFINED
+        self.keep_z = keep_z or self.refined
+        self.layernorm = layernorm
+        self._capacity = (int(capacity) if capacity else 0, int(bank_capacity) if bank_capacity else 0)
+        self._sig = None
+        self.P = 0
+        self.grid = (0, 0)
+        self._q: Optional[_GrowingImages] = None
+        self._bank: Optional[_GrowingImages] = None
+        self._w = self._a64 = self._a32 = self._X = None
+
+    @property
+    def n_img(self) -> int:
+        """Query images so far."""
+        return self._q.n_img if self._q is not None else 0
+
+    @property
+    def n_normal(self) -> int:
+        """Normal (bank) images so far."""
+        return self._bank.n_img if self._bank is not None else 0
+
+    def _check(self, features) -> int:
+        """Refuses features unlike the first call's (on either side); the first call fixes the patch grid and whether Z is
+        kept, as run_path would decide them.  Returns the image count."""
+        sig = _feature_signature(features, self._sig)
+        M = _image_count(features)
+        if self._sig is None:
+            if not self.keep_z and not z_free_supported(features, self.patchsize, self.stride, self.pretrain_dim, self.target_dim,
+                                                        self.precision):
+                self.keep_z = True
+            v0 = ops.feature_view(features[0])
+            self.grid = ops.patch_grid(v0.shape[2], v0.shape[3], self.patchsize, self.stride)
+            self.P = self.grid[0] * self.grid[1]
+            self._q = _GrowingImages(self.precision, self.P, self.target_dim, self.keep_z, not self.keep_z, self._capacity[0])
+            self._bank = _GrowingImages(self.precision, self.P, self.target_dim, False, False, self._capacity[1])
+            self._sig = sig
+        return M
+
+    def _nearest(self, r0: int, r1: int, b0: int, b1: int) -> torch.Tensor:
+        """dmin [b1 - b0, r1 - r0]: distance of query rows [r0, r1) to their nearest row of each bank image [b0, b1), from one
+        all-pairs tensor-core launch and, in f16r / bf16r, the exact fp32 re-evaluation of the selected pairs."""
+        q, bank, P = self._q, self._bank, self.P
+        rows, brows = slice(r0, r1), slice(b0 * P, b1 * P)
+        qhi, qlo, qn2 = q.hi[rows], None if q.lo is None else q.lo[rows], q.n2[rows]
+        bhi, blo, bn2 = bank.hi[brows], None if bank.lo is None else bank.lo[brows], bank.n2[brows]
+        _mark("mindist_begin")
+        if not self.refined:
+            dmin = ops.min_dist(qhi, qlo, qn2, bhi, blo, bn2, b1 - b0, P, self.precision)
+            _mark("mindist_end")
+            return dmin
+        dmin, arg = ops.min_dist_arg(qhi, qlo, qn2, bhi, blo, bn2, b1 - b0, P, self.precision)
+        _mark("mindist_end")
+        _mark("refine_begin")
+        dmin = ops.refine_min_dist(q.Z[rows], qhi, qlo, bhi, blo, b1 - b0, P, arg, Pq=P, Bn2=bn2)
+        _mark("refine_end")
+        return dmin
+
+    def _stage3(self, i0: int, i1: int, features) -> None:
+        """alpha and X of query images [i0, i1) from their w, into the state buffers."""
+        P = self.P
+        w = self._w[i0 * P:i1 * P].reshape(i1 - i0, P)
+        a64, a32, X, _ = alpha_X_dist(self._q.patchset(i0, i1, self.grid), w, self.taus, features,
+                                      (self.patchsize, self.stride, self.pretrain_dim, self.layernorm), want_dmat=False)
+        self._a64[:, i0:i1].copy_(a64)
+        self._a32[:, i0:i1].copy_(a32)
+        self._X[:, i0:i1].copy_(X)
+
+    def _result(self) -> PathResult:
+        """The PathResult of all queries so far, in tensors of its own (later calls do not change it)."""
+        N, P, D = self.n_img, self.P, self.target_dim
+        own = lambda t: t.clone(memory_format=torch.contiguous_format)
+        X = own(self._X[:, :N])
+        Dm = torch.stack([ops.pairwise_l2(X[t]) for t in range(len(self.taus))])
+        return PathResult(Z=self._q.Z[:N * P].reshape(N, P, D) if self.keep_z else None, w=own(self._w[:N * P]).reshape(N, P),
+                          alpha64=own(self._a64[:, :N]), alpha32=own(self._a32[:, :N]), X=X, Dmat=Dm, taus=list(self.taus),
+                          grid=self.grid)
+
+    def add_normal(self, features: Sequence[torch.Tensor]) -> Optional[PathResult]:
+        """Normal images join the bank: every query row runs against the new bank images only, w is lowered in place and stage 3
+        runs for every query.  Returns the PathResult of all queries so far (None while there are none)."""
+        features = list(features)
+        K = self._check(features)
+        k_old, N, P = self.n_normal, self.n_img, self.P
+        self._bank.append(features, self.patchsize, self.stride, self.pretrain_dim, self.layernorm)
+        if N == 0:
+            return None
+        dmin = self._nearest(0, N * P, k_old, k_old + K)
+        ops.reduce_weights(dmin, P, None, "min_update", out=self._w[:N * P])
+        self._stage3(0, N, None if self.keep_z else [buf[:N] for buf in self._q.maps])
+        return self._result()
+
+    def add(self, features: Sequence[torch.Tensor]) -> PathResult:
+        """Query images join: only their rows run against the bank, and only their alpha and X are computed.  Returns the
+        PathResult of all queries so far."""
+        features = list(features)
+        if self.n_normal == 0:
+            raise ValueError("add needs a normal bank: call add_normal first")
+        M = self._check(features)
+        n_old, N, P, T, D = self.n_img, self.n_img + M, self.P, len(self.taus), self.target_dim
+        q = self._q
+        q.append(features, self.patchsize, self.stride, self.pretrain_dim, self.layernorm)
+        if self._w is None or self._w.numel() < q.capacity * P:
+            dev, cap = q.hi.device, q.capacity
+            self._w = _regrow(self._w, n_old * P, (cap * P,), torch.float32, dev)
+            self._a64 = _regrow(self._a64, n_old, (T, cap, P), torch.float64, dev, dim=1)
+            self._a32 = _regrow(self._a32, n_old, (T, cap, P), torch.float32, dev, dim=1)
+            self._X = _regrow(self._X, n_old, (T, cap, D), torch.float32, dev, dim=1)
+        r0 = n_old * P
+        if self.refined:
+            r0 -= r0 % _REFINE_QUERY_ROWS     # the rows before n_old * P get the w they already hold
+        dmin = self._nearest(r0, N * P, 0, self.n_normal)
+        ops.reduce_weights(dmin, P, None, "min", out=self._w[r0:N * P])
+        self._stage3(n_old, N, features)
+        return self._result()
+
+

@@ -48,6 +48,7 @@ extern "C" {
 /* reduce modes of ac_reduce_weights */
 #define AC_REDUCE_MEAN 0 /* unsupervised: mean over bank images (self excluded)  utils.py:227 */
 #define AC_REDUCE_MIN 1  /* supervised:   min over bank images                   utils.py:236 */
+#define AC_REDUCE_MIN_UPDATE 2 /* supervised, grown bank: min of w (read) and of the given bank images */
 
 typedef void* ac_stream_t; /* cudaStream_t */
 
@@ -156,7 +157,12 @@ int ac_min_dist(const void* Qhi, const void* Qlo, const float* Qn2, int64_t Mq, 
 
 /* w[r] = mean_j dmin[j, r] over bank images j != q_self[r / Pq]   (AC_REDUCE_MEAN, utils.py:227)
  *      = min_j  dmin[j, r]                                           (AC_REDUCE_MIN,  utils.py:236)
- * q_self: [ceil(Mq/Pq)] int32 bank-image index of each query image, -1 or NULL = none. */
+ *      = min(w[r], min_j dmin[j, r])                                 (AC_REDUCE_MIN_UPDATE)
+ * q_self: [ceil(Mq/Pq)] int32 bank-image index of each query image, -1 or NULL = none.
+ * AC_REDUCE_MIN_UPDATE reads w as a running minimum: a supervised bank that gains images passes the distances to the new
+ * images only (dmin [K, Mq]) and gets the minimum over the whole bank, bit-identical to AC_REDUCE_MIN over all of it
+ * because a min of fp32 values does not depend on the order it is taken in.  q_self and groups mean what they mean for
+ * AC_REDUCE_MIN.  Any other mode is AC_ERR_INVALID. */
 int ac_reduce_weights(const float* dmin, int64_t Mq, int nb_img, int Pq, const int32_t* q_self,
                       int mode, float* w, ac_stream_t stream);
 
