@@ -280,7 +280,9 @@ int ac_refine_min_dist_grow(const float* Z, const void* Bhi, const void* Blo, in
  * new rows: every other image), partner images in increasing order; then w[R] = float(S[R] / (nb_img - 1)) for every row.
  * Rows of new images start from 0, rows of old ones from S as left by the previous update.  rowv / colv in the layouts of
  * drow / dcol above: squared = 1 for the squared minima of ac_min_dist_sym_grow, 0 for the distances of
- * ac_refine_min_dist_grow.  The order of addition is fixed by the data, so the result does not depend on the launch geometry. */
+ * ac_refine_min_dist_grow.  The order of addition is fixed by the data, so the result does not depend on the launch geometry.
+ * Only the entries of the rule's table are read for each pair (the other one may hold anything, NaN included).  A category of
+ * one image (nb_img = 1, n_old = 0) has no partner: S = 0 and w = NaN. */
 int ac_accumulate_weights_grow(const float* rowv, const float* colv, int squared, int n_old, int nb_img, int P, double* S,
                                float* w, ac_stream_t stream);
 int ac_reduce_weights_ex(const float* dmin, int64_t Mq, int nb_img, int Pq, const int32_t* q_self, const int32_t* groups,
